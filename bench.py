@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched under torchrun, one rank per GPU)
   python bench.py --impl reference ...                     (the reference arm: CPU restatement on the host cores)
+  python bench.py ... --dump-outputs DIR                   (also writes the last timed step's outputs to DIR/*.npy)
 
 Workload = BASELINE.json configs[2] ("65536 random paths, full nonlinear time allocation and feasibility subdivision"),
 the configuration the metric "optimized+sampled trajectories/sec (10-seg, N=10, fp64) at 1/2/4/8 B200" is quoted on.
@@ -152,6 +153,41 @@ def single_path_latency(ctx, P, n=101):
             "what": "single 11-waypoint random-flier path per call, host waypoints in -> samples + result record on the host (configs[0]-style single problem)"}
 
 
+DUMP_PATHS = 4096            # paths whose full outputs are written
+DUMP_LIMIT = 64 << 20        # bytes, all files together
+
+
+def dump_outputs(out_dir, ctx, res):
+    """Writes what a caller of the timed call receives for the last timed step, as float64 .npy files that two builds can be
+    compared with file by file.  For a fixed seeded sample of paths (path_index.npy, ascending): their final waypoints, segment
+    times, coefficients and samples, concatenated in path order (path p contributes n_waypoints[p] waypoints, n_waypoints[p] - 1
+    segments and n_samples[p] samples).  The result records (result_<field>.npy, one value per path) cover every path while they
+    take at most half of DUMP_LIMIT (batches up to 262144 paths), the sampled paths only beyond that.  The sample is halved until
+    all files fit DUMP_LIMIT; one path always fits."""
+    out = ctx.fetch_outputs()
+    B = len(res)
+    all_records = B * len(res.dtype.names) * 8 <= DUMP_LIMIT // 2
+
+    def gather(idx):
+        s0, s1 = out["seg_off"][idx], out["seg_off"][idx + 1]
+        m0, m1 = out["smp_off"][idx], out["smp_off"][idx + 1]
+        cat = lambda a, lo, hi: np.concatenate([a[l:h] for l, h in zip(lo, hi)]).astype(np.float64)
+        rec = res if all_records else res[idx]
+        arrays = {"result_" + k: rec[k].astype(np.float64) for k in res.dtype.names}
+        arrays.update({"path_index": idx.astype(np.float64), "wp": cat(out["wp"], s0 + idx, s1 + idx + 1), "times": cat(out["times"], s0, s1),
+                       "coef": cat(out["coef"], s0, s1), "samples": cat(out["samples"], m0, m1)})
+        return arrays
+
+    idx = np.sort(np.random.default_rng(20261020).permutation(B)[:DUMP_PATHS])
+    arrays = gather(idx)
+    while len(idx) > 1 and sum(a.nbytes for a in arrays.values()) > DUMP_LIMIT:
+        idx = idx[::2]
+        arrays = gather(idx)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return
@@ -194,7 +230,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--same-batch", action="store_true", help="diagnostic: every rank gets rank 0's batch (separates batch-to-batch work variance from the box)")
     ap.add_argument("--no-profile", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -252,6 +291,8 @@ def main():
     clocks = sampler.stop()
     barrier()
     c1 = ctx.counters()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, res)
     tmax = torch.tensor([dev_ms, wall_ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)

@@ -10,7 +10,8 @@
  *
  * PARITY STATUS: pinned to the reference's own SOURCES, bit for bit, for everything the reference's repository contains; unpinned
  * only where the reference calls third-party BINARIES that are not in its tree.
- *   - oracle/Makefile target _ref/libref_eth.so compiles, unmodified and from where they lie under /root/reference,
+ *   - oracle/Makefile target _ref/libref_eth.so compiles, unmodified and from where they lie in a checkout of the reference
+ *     ($TG_REFERENCE_DIR, else BASELINE.json's reference_path, /root/reference),
  *     src/eth_trajectory_generation/{motion_defines,polynomial,segment,trajectory,trajectory_sampling,vertex,timing,
  *     rpoly/rpoly_ak1}.cpp and the templates impl/polynomial_optimization_{linear,nonlinear}_impl.h, against stand-in headers for
  *     Eigen (oracle/ref_shim/Eigen: eager dense/sparse subset with the summation orders written down), NLopt (ref_shim/nlopt.hpp),
@@ -19,7 +20,8 @@
  *     maxima through Jenkins-Traub, computeMaximumOfMagnitude, scaleSegmentTimesToMeetConstraints, sampleWholeTrajectory,
  *     Trajectory::evaluate, the Mellinger time allocation end to end (optimize -> scaleSegmentTimesWithViolation) and the objective
  *     functions of methods 0/1/3/4.  tests/golden/ref_eth.npz holds outputs of that build (generator: tests/golden/gen_golden.py)
- *     so that the pin travels to machines without /root/reference.
+ *     for eight problems, so that the time estimates, coefficients and cost, maxima, time scaling, sampling and time allocation
+ *     stay pinned on machines without the checkout.
  *   - What the stand-ins stand in for is NOT in the reference tree and cannot be pinned: (i) Eigen::SparseQR<COLAMD> on Rpp
  *     (lin_impl.h:362-369) -- the stand-in's solve is LU without pivoting on the full band (the contract the GPU follows); a
  *     Householder-QR variant of the stand-in (_ref/libref_eth_qr.so) and a 50-digit mpmath solve bound the difference

@@ -1,7 +1,7 @@
 // tests/cpp/test_shim_eigen.cpp -- the drop-in header with REFERENCE-TYPED call sites: Eigen::Vector4d / Eigen::VectorXd
 // arguments and results and an EigenTrajectoryPoint result type, written the way MrsTrajectoryGeneration::findTrajectory
 // writes them (src/mrs_trajectory_generation.cpp:923-977, 1063-1169).  Eigen itself is absent from this image: the test
-// compiles against the stand-in of oracle/ref_shim/ (TEST INFRASTRUCTURE), and -- where /root/reference exists -- against
+// compiles against the stand-in of oracle/ref_shim/ (TEST INFRASTRUCTURE), and -- where a checkout of the reference is present -- against
 // the reference's own eth_mav_msgs/eigen_mav_msgs.h for the point type.  Also: optimize() for a derivative-free time
 // allocation method and the multi-context TrajectoryGeneratorBatch.  Dumps hex floats for tests/test_cpp_shim.py.
 #include <Eigen/Core>

@@ -1,8 +1,9 @@
 #!/usr/bin/env python3
-"""Generates the committed golden fixtures of tests/golden/ (run in the build container, where /root/reference exists).
+"""Generates the committed golden fixtures of tests/golden/ (run where a checkout of the reference is present:
+$TG_REFERENCE_DIR, else BASELINE.json's reference_path).
 
   rpoly_reference.npz   zeros returned by the REFERENCE's own Jenkins-Traub file
-                        (/root/reference/src/eth_trajectory_generation/rpoly/rpoly_ak1.cpp, compiled unmodified by
+                        (src/eth_trajectory_generation/rpoly/rpoly_ak1.cpp of that checkout, compiled unmodified by
                         oracle/Makefile into oracle/_ref/libref_rpoly.so) for 600 polynomials of the kinds the path meets:
                         extremum polynomials of real trajectory segments (degrees 15/13/11/7/6/5), random polynomials
                         with exact zeros at the origin, vanishing leading coefficients, clustered zeros.
@@ -98,7 +99,7 @@ def ref_eth_fixtures():
 
 def main():
     O.build_oracle(ref=True)
-    assert O.ref_lib() is not None, "needs /root/reference (build container)"
+    assert O.ref_lib() is not None, "needs a checkout of ctu-mrs/mrs_uav_trajectory_generation (TG_REFERENCE_DIR or BASELINE.json reference_path)"
     O.set_math_mode(O.MATH_DET)
     rng = np.random.default_rng(20261017)
     polys = []

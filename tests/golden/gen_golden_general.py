@@ -1,6 +1,6 @@
 """Writes tests/golden/ref_eth_general.npz: outputs of the REFERENCE's PolynomialOptimization<N> templates for N = 6, 8, 12
-(oracle/_ref/libref_eth_n{N}.so, compiled from /root/reference by oracle/Makefile) on the inputs of
-tests/test_general_shape.py::reference_cases.  Run in the build container: python tests/golden/gen_golden_general.py"""
+(oracle/_ref/libref_eth_n{N}.so, compiled by oracle/Makefile from a checkout of the reference) on the inputs of
+tests/test_general_shape.py::reference_cases.  Run: TG_REFERENCE_DIR=<checkout> python tests/golden/gen_golden_general.py"""
 import ctypes as C
 import os
 import sys

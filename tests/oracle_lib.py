@@ -3,6 +3,7 @@
 The oracle is the CPU restatement of the reference; the product package never imports this module.
 """
 import ctypes as C
+import json
 import os
 import subprocess
 
@@ -86,10 +87,25 @@ class Result(C.Structure):
     ]
 
 
+def reference_dir():
+    """The checkout of the original ctu-mrs/mrs_uav_trajectory_generation that oracle/Makefile compiles into oracle/_ref/:
+    $TG_REFERENCE_DIR, else the reference_path BASELINE.json records (the same rule as oracle/Makefile); None where it is
+    absent.  The repository does not contain it: without it the live comparisons with the reference's own code skip, and only
+    the reference outputs stored under tests/golden/ are compared with."""
+    d = os.environ.get("TG_REFERENCE_DIR")
+    if not d:
+        with open(os.path.join(ROOT, "BASELINE.json")) as f:
+            d = json.load(f).get("reference_path")
+    return os.path.abspath(d) if d and os.path.isdir(d) else None
+
+
+REFERENCE = reference_dir()
+
+
 def build_oracle(ref=True):
     subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "liboracle.so"])
-    if ref and os.path.isdir("/root/reference"):
-        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "ref"])
+    if ref and REFERENCE:
+        subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "ref", "REFERENCE=" + REFERENCE])
 
 
 _lib = None
@@ -122,7 +138,7 @@ def ref_lib():
     if _ref is None:
         path = os.path.join(ORACLE_DIR, "_ref", "libref_rpoly.so")
         if not os.path.exists(path):
-            if not os.path.isdir("/root/reference"):
+            if not REFERENCE:
                 return None
             build_oracle(ref=True)
         _ref = C.CDLL(path)

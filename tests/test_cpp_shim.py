@@ -114,11 +114,11 @@ def _check_side_steps(res):
 
 
 def _eigen_flags():
-    # the Eigen stand-in (test infrastructure; Eigen is absent from this image) and, in the build container, the reference's own
-    # eth_mav_msgs/eigen_mav_msgs.h for the EigenTrajectoryPoint type
+    # the Eigen stand-in (test infrastructure: the tests do not need Eigen) and, where a checkout of the reference is present
+    # (oracle_lib.reference_dir()), its own eth_mav_msgs/eigen_mav_msgs.h for the EigenTrajectoryPoint type
     flags = ["-I" + os.path.join(ROOT, "oracle", "ref_shim")]
-    if os.path.isdir("/root/reference/include"):
-        flags.append("-I/root/reference/include")
+    if O.REFERENCE and os.path.isdir(os.path.join(O.REFERENCE, "include")):
+        flags.append("-I" + os.path.join(O.REFERENCE, "include"))
     return flags
 
 

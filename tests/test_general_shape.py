@@ -7,8 +7,8 @@ tg_evaluate_batch_nd / tg_sample_batch_nd (csrc/tg_generic.cuh).  Checked here, 
     emulation of the device code (CPU) and on the GPU;
   * N = 10, D = 4: the general-shape kernels against the tuned kernels of the benchmarked path;
   * the restatement for N = 6, 8, 12 against the REFERENCE's own templates instantiated for that N
-    (oracle/_ref/libref_eth_n{6,8,12}.so, built from /root/reference against the stand-in headers), and against the vectors that
-    build left in tests/golden/ref_eth_general.npz for machines without /root/reference.
+    (oracle/_ref/libref_eth_n{6,8,12}.so, built from a checkout of the reference against the stand-in headers), and against
+    the vectors that build left in tests/golden/ref_eth_general.npz (the same inputs) for machines without that checkout.
 """
 import ctypes as C
 import os
@@ -274,8 +274,8 @@ def ref_outputs(lib, n_coef, case):
 @pytest.mark.parametrize("n_coef", [6, 8, 12])
 def test_restatement_equals_reference_templates(n_coef):
     """PolynomialOptimization<N>::setupFromVertices / solveLinear / computeCost of the reference, instantiated for N, vs oracle/."""
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("/root/reference is only present in the build container")
+    if not O.REFERENCE:
+        pytest.skip("needs a checkout of the original ctu-mrs/mrs_uav_trajectory_generation (TG_REFERENCE_DIR or BASELINE.json reference_path)")
     O.build_oracle(ref=True)
     lib = C.CDLL(os.path.join(ROOT, "oracle", "_ref", f"libref_eth_n{n_coef}.so"))
     orc = O.OracleN(n_coef, mode=O.MATH_LIBM)

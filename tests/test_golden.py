@@ -40,9 +40,10 @@ def test_oracle_rpoly_matches_reference_vectors(oracle):
 
 
 def test_oracle_rpoly_matches_live_reference_build(oracle):
-    """Where /root/reference exists (the build container) the comparison also runs live against oracle/_ref."""
+    """Where a checkout of the reference is present, the comparison also runs live against oracle/_ref on 300 more polynomials."""
     if O.ref_lib() is None:
-        pytest.skip("reference sources not present on this machine; the committed vectors cover it")
+        pytest.skip("needs a checkout of the original project (TG_REFERENCE_DIR or BASELINE.json reference_path); "
+                    "the 600 stored cases of rpoly_reference.npz are compared instead")
     rng = np.random.default_rng(5)
     O.set_math_mode(O.MATH_LIBM)
     try:

@@ -95,9 +95,8 @@ def _mp_solve(m, v, t):
 
 
 def test_band_lu_vs_qr_vs_exact(oracle, record_property):
-    have_ref = os.path.isdir("/root/reference")
     qr = None
-    if have_ref:
+    if O.REFERENCE:
         O.build_oracle(ref=True)
         qr = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_eth_qr.so"))
     O.set_math_mode(O.MATH_LIBM)

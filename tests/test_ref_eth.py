@@ -1,6 +1,7 @@
 """Oracle pinned to the REFERENCE's own source.
 
-oracle/Makefile compiles the reference's eth_trajectory_generation library UNMODIFIED from /root/reference (polynomial.cpp,
+oracle/Makefile compiles the reference's eth_trajectory_generation library UNMODIFIED from a checkout of the reference
+($TG_REFERENCE_DIR, else the reference_path BASELINE.json records) (polynomial.cpp,
 segment.cpp, trajectory.cpp, trajectory_sampling.cpp, vertex.cpp, motion_defines.cpp, timing.cpp, rpoly/rpoly_ak1.cpp and the
 header templates PolynomialOptimization<10> / PolynomialOptimizationNonLinear<10>) against the stand-ins of oracle/ref_shim/
 (Eigen, NLopt, mrs_lib, ROS messages, boost are absent from this image) into oracle/_ref/libref_eth.so.  These tests run the
@@ -10,8 +11,11 @@ thereby checked against the reference's own code for SURVEY rows a3-a13, a14-a21
 rounding of real Eigen's products / SparseQR and of a real NLopt build -- the stand-ins implement this project's numeric
 contract for those (oracle/ref_shim/Eigen/shim_impl.h, oracle/plis.cpp).
 
-/root/reference exists only in the build container: the tests skip elsewhere, and the vectors they produce are committed under
-tests/golden/ref_eth.npz (tests/golden/gen_golden.py) so that the same comparison runs on the GPU box against the fixtures.
+The reference's sources are not part of this repository: these tests run where that checkout is present and skip elsewhere.
+Without it only part of what they check is compared with stored reference outputs (tests/golden/ref_eth.npz, eight problems,
+tests/test_golden.py): segment-time estimates, linear-solve coefficients and cost (r = 2, 4), per-segment maxima, time
+scaling, sampling and the Mellinger time allocation.  The mapping / inverse / cost matrices, the dense R, the free derivatives,
+r = 3, computeMaximumOfMagnitude, Trajectory::evaluate and the soft-constraint objectives have no stored counterpart.
 """
 import ctypes as C
 import os
@@ -36,8 +40,8 @@ def _p(a, t=dp):
 
 @pytest.fixture(scope="module")
 def ref():
-    if not os.path.isdir("/root/reference"):
-        pytest.skip("/root/reference is only present in the build container")
+    if not O.REFERENCE:
+        pytest.skip("needs a checkout of the original ctu-mrs/mrs_uav_trajectory_generation (TG_REFERENCE_DIR or BASELINE.json reference_path)")
     O.build_oracle(ref=True)
     lib = C.CDLL(os.path.join(ROOT, "oracle", "_ref", "libref_eth.so"))
     O.set_math_mode(O.MATH_LIBM)
