@@ -177,6 +177,25 @@ int tg_evaluate_batch_nd(tg_ctx* ctx, int N, int D, int S, const double* coef, c
                          double* out, uint8_t* ok);
 int tg_sample_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times, double dt, int* counts,
                        double* samples, double* full);
+/* The nonlinear half on the same shapes, with the contracts of the N = 10 entry points above (coef[totS][D][N] everywhere):
+ *   tg_extrema_batch_nd        = tg_extrema_batch: Trajectory::computeMaxDerivatives{Horizontal,Vertical,Heading}
+ *                                (eth/trajectory.cpp:422-565) -> maxima[totS][9]; a missing dimension has zero maxima.
+ *   tg_max_magnitude_batch_nd  = tg_max_magnitude_batch: PolynomialOptimization<N>::computeMaximumOfMagnitude (lin_impl.h:477-508)
+ *                                over the D dimensions; derivative in 1..4.
+ *   tg_scale_times_batch_nd    = tg_scale_times_batch: Trajectory::scaleSegmentTimesToMeetConstraints (eth/trajectory.cpp:598-692)
+ *                                in place on coef / times.
+ *   tg_time_alloc_batch_nd     = tg_time_alloc_batch: PolynomialOptimizationNonLinear<N>::setupFromVertices + optimize() with the
+ *                                Mellinger outer loop (nl_impl.h:159-234, 256-333) + scaleSegmentTimesWithViolation (335-427) +
+ *                                getTrajectory; vval[totV][N/2][D]; derivative_to_optimize in 0 .. N/2-1.
+ *   Every (segment, quantity) maximum is found by exact root finding (no Bernstein pruning: that is built for N = 10), and a
+ *   Mellinger evaluation is S+1 dense solves per running problem; both give the tuned kernels' bits at N = 10, D = 4. */
+int tg_extrema_batch_nd(tg_ctx* ctx, int N, int D, int totS, const double* coef, const double* times, double* maxima);
+int tg_max_magnitude_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times, int derivative,
+                              double* value, double* time, int* segment_idx);
+int tg_scale_times_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, double* coef, double* times, const double* limits9,
+                            int* passes, uint8_t* within);
+int tg_time_alloc_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                           const tg_params* params, double* coef, int* nlopt_code, int* n_evals, int* n_scale_passes, double* final_cost);
 /* tg_sweep_costs (BASELINE config 5) = updateSegmentTimes + solveLinear + computeCost for K candidate time vectors
  *   of ONE problem (lin_impl.h:288-304, 340-373, 127-141).  cand[K][S] host (or device when cand_on_device).
  *   costs (optional) [K] host; best_index / best_cost = argmin (first minimum). */

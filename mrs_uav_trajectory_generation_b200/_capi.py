@@ -125,6 +125,10 @@ class Library:
         L.tg_solve_linear_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.c_int, _dp, _dp]
         L.tg_evaluate_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, C.c_int, _dp, _u8p]
         L.tg_sample_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_double, _ip, _dp, _dp]
+        L.tg_extrema_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp]
+        L.tg_max_magnitude_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
+        L.tg_scale_times_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _ip, _u8p]
+        L.tg_time_alloc_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.POINTER(Params), _dp, _ip, _ip, _ip, _dp]
         L.tg_objective_batch.argtypes = [C.c_void_p, C.c_int, _u8p, _dp, C.c_int, C.c_int, C.c_longlong, _dp, C.c_int, C.c_double, C.c_int, C.c_double,
                                          C.c_int, _ip, _dp, _dp, _dp, _dp]
         L.tg_max_magnitude_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
@@ -448,6 +452,61 @@ class Context:
         self._check(lib.tg_sample_batch_nd(self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), float(dt), _p(counts, _ip),
                                            _p(samples), _p(fullv)))
         return counts, samples, fullv
+
+    def extrema_nd(self, n_coef, dim, coef, times):
+        """Nine maxima per segment of N-coefficient, D-dimensional segments: coef [totS][dim][n_coef] -> maxima [totS][9]."""
+        coef = np.ascontiguousarray(coef, dtype=np.float64)
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        assert coef.size == len(times) * dim * n_coef
+        m = np.empty((len(times), 9))
+        self._check(self.L.lib.tg_extrema_batch_nd(self.h, int(n_coef), int(dim), len(times), _p(coef), _p(times), _p(m)))
+        return m
+
+    def max_magnitude_nd(self, n_coef, dim, seg_off, coef, times, derivative):
+        """computeMaximumOfMagnitude(derivative) of PolynomialOptimization<n_coef>(dim) per trajectory -> time[B], value[B], segment_idx[B]."""
+        seg_off = np.ascontiguousarray(seg_off, dtype=np.int32)
+        coef = np.ascontiguousarray(coef, dtype=np.float64)
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        B = len(seg_off) - 1
+        assert coef.size == int(seg_off[-1]) * dim * n_coef and times.size == int(seg_off[-1])
+        v, t, i = np.empty(B), np.empty(B), np.empty(B, dtype=np.int32)
+        self._check(self.L.lib.tg_max_magnitude_batch_nd(self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), int(derivative),
+                                                         _p(v), _p(t), _p(i, _ip)))
+        return t, v, i
+
+    def scale_times_nd(self, n_coef, dim, seg_off, coef, times, limits):
+        """scaleSegmentTimesToMeetConstraints on copies of coef [totS][dim][n_coef] / times -> coef, times, passes[B], within[B]."""
+        seg_off = np.ascontiguousarray(seg_off, dtype=np.int32)
+        coef = np.array(coef, dtype=np.float64, order="C")
+        times = np.array(times, dtype=np.float64)
+        lim = np.ascontiguousarray(limits, dtype=np.float64)
+        B = len(seg_off) - 1
+        assert coef.size == int(seg_off[-1]) * dim * n_coef and times.size == int(seg_off[-1]) and lim.size == 9
+        passes = np.zeros(B, dtype=np.int32)
+        within = np.zeros(B, dtype=np.uint8)
+        self._check(self.L.lib.tg_scale_times_batch_nd(self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), _p(lim), _p(passes, _ip),
+                                                       _p(within, _u8p)))
+        return coef, times, passes, within.astype(bool)
+
+    def time_alloc_batch_nd(self, n_coef, dim, vtx_off, vmask, vval, times, params=None):
+        """PolynomialOptimizationNonLinear<n_coef>(dim)::optimize() (Mellinger) for B problems given as vertices: vval [totV][n_coef/2][dim].
+        Returns the dict of time_alloc_batch with coef [totS][dim][n_coef]."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        vmask = np.ascontiguousarray(vmask, dtype=np.uint8)
+        vval = np.ascontiguousarray(vval, dtype=np.float64)
+        times = np.array(times, dtype=np.float64, copy=True)
+        B = len(vtx_off) - 1
+        totS = int(vtx_off[-1]) - B
+        assert vval.size == int(vtx_off[-1]) * (n_coef // 2) * dim and times.size == totS
+        P = params or self.L.default_params()
+        coef = np.empty((totS, dim, n_coef))
+        code = np.zeros(B, dtype=np.int32)
+        evals = np.zeros(B, dtype=np.int32)
+        passes = np.zeros(B, dtype=np.int32)
+        cost = np.zeros(B)
+        self._check(self.L.lib.tg_time_alloc_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times), C.byref(P),
+                                                      _p(coef), _p(code, _ip), _p(evals, _ip), _p(passes, _ip), _p(cost)))
+        return {"times": times, "coef": coef, "nlopt_code": code, "n_evals": evals, "n_scale_passes": passes, "final_cost": cost}
 
     def extrema(self, coef, times):
         coef = np.ascontiguousarray(coef, dtype=np.float64)

@@ -313,6 +313,16 @@ inline std::vector<double> tg_pad_coef(const double* coef, size_t S, int N, int 
     for (int d = 0; d < D; ++d) std::memcpy(&out[(s * TG_D + d) * N], coef + (s * D + d) * N, sizeof(double) * N);
   return out;
 }
+// [S][4][N] -> [S][D][N]
+inline void tg_strip_coef(const double* c4, size_t S, int N, int D, double* coef) {
+  for (size_t s = 0; s < S; ++s)
+    for (int d = 0; d < D; ++d) std::memcpy(coef + (s * D + d) * N, c4 + (s * TG_D + d) * N, sizeof(double) * N);
+}
+inline bool tg_segments_ok(int B, const int* seg_off) {
+  for (int p = 0; p < B; ++p)
+    if (seg_off[p + 1] - seg_off[p] < 1) return false;
+  return true;
+}
 template <class F>
 inline void tg_dispatch_n(int N, F&& f) {
   switch (N) {
@@ -370,6 +380,78 @@ int tg_sample_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, con
     ctx->be.timer_start();
     tg_dispatch_n(N, [&](auto nn) { ctx->pipe.template sample_batch_n<decltype(nn)::value>(B, seg_off, c4.data(), times, dt, counts, samples, full); });
     ctx->last_ms = ctx->be.timer_stop();
+    return TG_OK;
+  });
+}
+
+int tg_extrema_batch_nd(tg_ctx* ctx, int N, int D, int totS, const double* coef, const double* times, double* maxima) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (totS < 1 || !coef || !times || !maxima) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    const std::vector<double> c4 = tg_pad_coef(coef, (size_t)totS, N, D);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) { ctx->pipe.template extrema_batch_n<decltype(nn)::value>(totS, c4.data(), times, maxima); });
+    ctx->last_ms = ctx->be.timer_stop();
+    return TG_OK;
+  });
+}
+
+int tg_max_magnitude_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times, int derivative,
+                              double* value, double* time, int* segment_idx) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !seg_off || !coef || !times || !value || !time || !segment_idx) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    if (derivative < 1 || derivative > 4) { ctx->err = "derivative must be 1..4"; return TG_ERR_INVALID; }
+    if (!tg_segments_ok(B, seg_off)) { ctx->err = "every trajectory needs at least one segment"; return TG_ERR_INVALID; }
+    const std::vector<double> c4 = tg_pad_coef(coef, (size_t)seg_off[B], N, D);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) {
+      ctx->pipe.template max_magnitude_batch_n<decltype(nn)::value>(B, seg_off, c4.data(), times, derivative, value, time, segment_idx);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    return TG_OK;
+  });
+}
+
+int tg_scale_times_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, double* coef, double* times, const double* limits9,
+                            int* passes, uint8_t* within) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !seg_off || !coef || !times || !limits9) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    if (!tg_segments_ok(B, seg_off)) { ctx->err = "every trajectory needs at least one segment"; return TG_ERR_INVALID; }
+    const size_t totS = (size_t)seg_off[B];
+    std::vector<double> c4 = tg_pad_coef(coef, totS, N, D);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) { ctx->pipe.template scale_times_batch_n<decltype(nn)::value>(B, seg_off, c4.data(), times, limits9, passes, within); });
+    ctx->last_ms = ctx->be.timer_stop();
+    tg_strip_coef(c4.data(), totS, N, D, coef);
+    return TG_OK;
+  });
+}
+
+int tg_time_alloc_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                           const tg_params* params, double* coef, int* nlopt_code, int* n_evals, int* n_scale_passes, double* final_cost) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !vtx_off || !vmask || !vval || !times || !params || params->derivative_to_optimize < 0 ||
+        params->derivative_to_optimize > N / 2 - 1 || params->max_evals < 1) {
+      ctx->err = "invalid argument";
+      return TG_ERR_INVALID;
+    }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) { ctx->err = "every problem needs at least two vertices"; return TG_ERR_INVALID; }
+    tg::Params P;
+    std::memcpy(&P, params, sizeof(P));
+    const size_t totV = (size_t)vtx_off[B], totS = totV - (size_t)B;
+    const std::vector<double> vv = tg_pad_dims(vval, totV * (size_t)(N / 2), D);
+    std::vector<double> c4(coef ? totS * TG_D * N : 0);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) {
+      ctx->pipe.template time_alloc_batch_n<decltype(nn)::value>(B, vtx_off, vmask, vv.data(), times, P, coef ? c4.data() : nullptr, nlopt_code,
+                                                                 n_evals, n_scale_passes, final_cost);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (coef) tg_strip_coef(c4.data(), totS, N, D, coef);
     return TG_OK;
   });
 }

@@ -13,6 +13,10 @@
 //                                                      (lin_impl.h:310-373, 263-282, 127-141) -- the phases of tg_solve.cuh
 //   poly_eval_n<N>, sample_eval_n<N>                   Trajectory::evaluate / sampleWholeTrajectory (eth/trajectory.cpp:55-151,
 //                                                      eth/trajectory_sampling.cpp:49-124)
+//   ExtremaFn<N, Q>, MaxMagnitudeSegFn<N, K>           per-segment maxima (tg_poly.cuh over N), one thread per segment
+//   ScaleFn<N>                                         scaleSegmentTimesToMeetConstraints' stretch (eth/trajectory.cpp:610-658)
+//   MellingerHeadFn / HrowFn / SolveFn<N>              one Mellinger evaluation: S+1 solves per running problem (nl_impl.h:282-323);
+//                                                      the optimiser state machine (tg_plis.cuh) does not depend on N
 // Every sum is the DENSE sum over ascending index, exactly as the reference-order restatement writes it (the tuned path skips structural
 // zeros, which is the same IEEE result); for N = 10 this path and the tuned one are compared bit for bit in the tests.
 // D: the device works on 4 right-hand sides; tg_*_nd pad D < 4 with zero dimensions (a zero dimension adds exact zeros to the
@@ -21,8 +25,10 @@
 #define TG_GENERIC_CUH_
 
 #include "tg_common.cuh"
-#include "tg_node.cuh"   // sample_cap, sample_walk
-#include "tg_solve.cuh"  // TG_PHASE
+#include "tg_kernels.cuh"  // BatchPtrs, the PLIS and scaling functors that do not depend on N
+#include "tg_node.cuh"     // sample_cap, sample_walk
+#include "tg_poly.cuh"     // segment maxima and Jenkins-Traub over N coefficients
+#include "tg_solve.cuh"    // TG_PHASE
 
 namespace tg {
 namespace gen {
@@ -156,14 +162,23 @@ TG_HD void record_hrow(double* __restrict__ rec, int a) {
 // ---- one problem per warp ---------------------------------------------------------------------------------------------
 struct Problem {
   int S, np, hbw, r;
+  int rec_stride;        // records per segment: 1 (one time per segment) or 3 (the time variants of a Mellinger evaluation)
+  int variant;           // with 3 records: 0 the point itself, n >= 1 the point perturbed along segment n-1
   const uint8_t* vmask;  // [V]
   const int* vfree;      // [V+1]
   const double* vval;    // [V][N/2][4]
-  const double* recs;    // [S][Rec<N>::kSize]
-  double* coef;          // [S][4][N]
+  const double* recs;    // [S][rec_stride][Rec<N>::kSize]
+  double* coef;          // [S][4][N], or null
   double* cost;          // scalar
   double* ws;            // solve_ws_doubles<N>(S, np, hbw) doubles
 };
+// the record segment s is solved with: variant 0 for every segment of the point itself; for the point perturbed along segment
+// n-1, variant 1 (T + 0.1) on that segment and variant 2 (T - 0.1/(S-1)) on the others (nl_impl.h:282-323)
+template <int N>
+TG_HD const double* problem_rec(const Problem& P, int s) {
+  const int which = (P.rec_stride == 1 || P.variant == 0) ? 0 : (s == P.variant - 1 ? 1 : 2);
+  return P.recs + ((size_t)s * P.rec_stride + which) * Rec<N>::kSize;
+}
 TG_HD int row_stride(int hbw) { return 2 * hbw + 1 + TG_D + 1; }  // band, 4 right-hand sides, reciprocal pivot
 template <int N>
 TG_HD size_t ws_doubles(int S, int np, int hbw) {
@@ -201,8 +216,8 @@ TG_HD void solve_warp(const Problem& P, int lane) {
         if (i < 0) continue;
         const int v = it / H, a = it - v * H;
         const bool has_p = v > 0, has_c = v < S;
-        const double* hp = has_p ? P.recs + (size_t)(v - 1) * Rec<N>::kSize + Rec<N>::kH + (H + a) * N : nullptr;
-        const double* hc = has_c ? P.recs + (size_t)v * Rec<N>::kSize + Rec<N>::kH + a * N : nullptr;
+        const double* hp = has_p ? problem_rec<N>(P, v - 1) + Rec<N>::kH + (H + a) * N : nullptr;
+        const double* hc = has_c ? problem_rec<N>(P, v) + Rec<N>::kH + a * N : nullptr;
         double* row = rows + (size_t)i * W;
         double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
         for (int g = 0; g < 3; ++g) {
@@ -272,7 +287,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
   TG_PHASE(lane) {
     for (int it = lane; it < S * TG_D * N; it += 32) {
       const int s = it / (TG_D * N), rem = it - s * (TG_D * N), d = rem / N, a = rem - d * N;
-      const double* Ai = P.recs + (size_t)s * Rec<N>::kSize + Rec<N>::kAinv + a * N;
+      const double* Ai = problem_rec<N>(P, s) + Rec<N>::kAinv + a * N;
       double c = 0.0;
       for (int k = 0; k < N; ++k) {
         const int j = slot[s * H + k];  // the slots of vertex s and of vertex s+1 are contiguous in the table
@@ -281,14 +296,14 @@ TG_HD void solve_warp(const Problem& P, int lane) {
         c = (k == 0) ? t : c + t;
       }
       cf[it] = c;
-      P.coef[it] = c;
+      if (P.coef) P.coef[it] = c;
     }
   }
   // ---- phase 5: (c^T Q) c per (segment, dimension), dense (lin_impl.h:135-137)
   TG_PHASE(lane) {
     for (int it = lane; it < S * TG_D; it += 32) {
       const int s = it / TG_D;
-      const double* Q = P.recs + (size_t)s * Rec<N>::kSize + Rec<N>::kQ;
+      const double* Q = problem_rec<N>(P, s) + Rec<N>::kQ;
       const double* c = cf + (size_t)it * N;
       double partial = 0.0;
       for (int b = 0; b < N; ++b) {
@@ -386,6 +401,8 @@ struct SolveFn {  // one warp per problem
     P.np = np[p];
     P.hbw = hbw[p];
     P.r = r;
+    P.rec_stride = 1;
+    P.variant = 0;
     P.vmask = vmask + v0;
     P.vfree = vfree + v0 + p;
     P.vval = vval + (size_t)v0 * (N / 2) * TG_D;
@@ -440,6 +457,120 @@ struct SampleEvalFn {  // one thread per sample slot; slots beyond a trajectory'
     if ((int)slot - smp_off[p] >= count[p]) return;
     const int gs = seg_off[p] + seg_idx[slot];
     sample_eval_n<N>(coef + (size_t)gs * TG_D * N, t_in[slot], xyzh ? xyzh + 4 * slot : nullptr, full ? full + 19 * slot : nullptr);
+  }
+};
+
+// ---- maxima, time scaling and the Mellinger evaluation ----------------------------------------------------------------------
+// Per-segment maximum of quantity Q (tg_poly.cuh over N coefficients): one thread per work item (every segment, or the entries of a
+// device work list), one launch per quantity so that a kernel has one polynomial degree.  Every (segment, quantity) goes through
+// exact root finding: the Bernstein certificates of tg_bound.cuh are built for N = 10, and since they never change a result,
+// leaving them out only costs time.
+template <int N, int Q>
+struct ExtremaFn {
+  const double* coef;  // [totS][4][N]
+  const double* times;
+  double* maxima;      // [totS][9]
+  const int* work;     // optional work list
+  const int* n_dev;    // optional length of the work list (device memory)
+  static constexpr int kScratch = JtScratch<QuantityDegree<Q, N>::value>::kShared;
+  TG_HD void operator()(size_t item, double* scratch, int stride) const {
+    if (n_dev && item >= (size_t)*n_dev) return;
+    const size_t gs = work ? (size_t)work[item] : item;
+    maxima[gs * 9 + Q] = segment_max_impl<Q, N>(coef + gs * TG_D * N, times[gs], scratch, stride, nullptr);
+  }
+};
+// computeMaximumOfMagnitude (lin_impl.h:477-508), step 1 over N coefficients; step 2 is MaxMagnitudeReduceFn
+template <int N, int K>
+struct MaxMagnitudeSegFn {
+  const double* coef;
+  const double* times;
+  double* seg_value;
+  double* seg_time;
+  static constexpr int kScratch = JtScratch<MaxAllDegree<K, N>::value>::kShared;
+  TG_HD void operator()(size_t gs, double* scratch, int stride) const {
+    segment_max_all_dims<K, N>(coef + gs * TG_D * N, times[gs], scratch, stride, seg_value + gs, seg_time + gs);
+  }
+};
+template <int N>
+struct ScaleFn {  // one thread per segment (eth/trajectory.cpp:610-658); b.coef is [totS][4][N]
+  BatchPtrs b;
+  double L[9];
+  uint8_t* changed;  // [totS]: 1 when the segment was stretched by a factor other than exactly 1
+  TG_HD void operator()(size_t gs) const {
+    const int p = b.prob_of_seg[gs];
+    if (b.ps[p].scale_done) return;
+    const double s = violation_scaling(b.maxima + gs * 9, L);
+    scale_segment<N>(b.coef + gs * TG_D * N, b.times + gs, s);
+    changed[gs] = (s != 1.0) ? 1 : 0;
+  }
+};
+
+// One Mellinger evaluation (nl_impl.h:282-323): records of every segment at three times, item = 3 * segment + variant, the times
+// computed exactly as SetupMellingerFn computes them; nothing for a problem whose optimiser has finished, nor for the perturbed
+// variants of a one-segment problem (its gradient needs the point only).  b.recs: [totS][3][Rec<N>::kSize].
+TG_HD bool mellinger_item_live(const BatchPtrs& b, size_t gs, int which, int* S) {
+  const int p = b.prob_of_seg[gs];
+  if (b.opt[p].done) return false;
+  *S = b.seg_off[p + 1] - b.seg_off[p];
+  return !(*S == 1 && which != 0);
+}
+template <int N>
+struct MellingerHeadFn {  // one thread per (segment, variant)
+  BatchPtrs b;
+  TG_HD void operator()(size_t item) const {
+    const size_t gs = item / 3;
+    const int which = (int)(item - gs * 3);
+    int S;
+    if (!mellinger_item_live(b, gs, which, &S)) return;
+    double T = b.xeval[gs];
+    if (which == 1) {
+      T = T + 0.1;
+      T = dmax(kTimeLowerBound, T);
+    } else if (which == 2) {
+      const double corr = 0.1 / ((double)S - 1.0);  // nl_impl.h:288
+      T = T - corr;
+      T = dmax(kTimeLowerBound, T);
+    }
+    record_head<N>(T, b.r, b.recs + item * Rec<N>::kSize);
+  }
+};
+template <int N>
+struct MellingerHrowFn {  // one thread per (segment, variant, row)
+  BatchPtrs b;
+  TG_HD void operator()(size_t it) const {
+    const size_t item = it / N, gs = item / 3;
+    int S;
+    if (!mellinger_item_live(b, gs, (int)(item - gs * 3), &S)) return;
+    record_hrow<N>(b.recs + item * Rec<N>::kSize, (int)(it - item * N));
+  }
+};
+// one warp per solve instance = vertex index: instance (p, n) is vertex n of problem p, n = 0 the point, n >= 1 the point perturbed
+// along segment n-1 (the numbering of SolveProblemDesc mode 1).  Cost to b.costs[first vertex of p + n]; coefficients for n = 0 only.
+template <int N>
+struct MellingerSolveFn {
+  BatchPtrs b;
+  const long long* ws_off;  // [totV] workspace offset of every instance (doubles)
+  double* ws;
+  TG_HD void operator()(size_t inst, int lane) const {
+    const int p = b.prob_of_vtx[inst], v0 = vtx_off(b, p), n = (int)inst - v0;
+    if (b.opt[p].done) return;
+    const int s0 = b.seg_off[p], S = b.seg_off[p + 1] - s0;
+    if (S == 1 && n > 0) return;
+    Problem P;
+    P.S = S;
+    P.np = b.np[p];
+    P.hbw = b.hbw[p];
+    P.r = b.r;
+    P.rec_stride = 3;
+    P.variant = n;
+    P.vmask = b.vmask + v0;
+    P.vfree = b.vfree + v0 + p;
+    P.vval = b.vval + (size_t)v0 * (N / 2) * TG_D;
+    P.recs = b.recs + (size_t)s0 * 3 * Rec<N>::kSize;
+    P.coef = (n == 0) ? b.coef + (size_t)s0 * TG_D * N : nullptr;
+    P.cost = b.costs + v0 + n;
+    P.ws = ws + ws_off[inst];
+    solve_warp<N>(P, lane);
   }
 };
 

@@ -1303,19 +1303,19 @@ class Pipeline {
   // setupFromVertices + solveLinear + getSegments + computeCost for B problems.  The vertex bookkeeping (first free unknown per
   // vertex, half bandwidth, workspace offsets) is host logic here: the inputs arrive from the host and this path is not the
   // benchmarked one.  vval: [totV][N/2][4]; coef out: [totS][4][N].
+  struct GenVertices {
+    std::vector<int> vfree, np, hbw;  // first free unknown per vertex (V + 1 entries per problem, at vtx_off[p] + p); per problem
+  };
   template <int N>
-  bool linear_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, const double* times, int r, double* coef, double* cost) {
+  static GenVertices gen_vertices(int B, const int* vtx_off, const uint8_t* vmask) {
     constexpr int H = N / 2;
-    scratch_.reset();
-    const int totV = vtx_off[B], totS = totV - B;
-    for (int p = 0; p < B; ++p)
-      if (vtx_off[p + 1] - vtx_off[p] < 2) return false;
-    std::vector<int> vfree((size_t)totV + B), np(B), hbw(B);
-    std::vector<long long> ws_off(B);
-    long long ws_tot = 0;
+    GenVertices g;
+    g.vfree.resize((size_t)vtx_off[B] + B);
+    g.np.resize(B);
+    g.hbw.resize(B);
     for (int p = 0; p < B; ++p) {
       const int v0 = vtx_off[p], V = vtx_off[p + 1] - v0;
-      int* ff = vfree.data() + v0 + p;  // V + 1 entries
+      int* ff = g.vfree.data() + v0 + p;
       ff[0] = 0;
       for (int v = 0; v < V; ++v) {
         int cnt = 0;
@@ -1325,10 +1325,25 @@ class Pipeline {
       int hb = 0;  // a free slot of vertex v couples to the free slots of v-1 .. v+1 (lin_impl.h:317-333)
       for (int v = 0; v < V; ++v)
         if (ff[v + 1] > ff[v]) hb = std::max(hb, ff[std::min(v + 2, V)] - 1 - ff[v]);
-      np[p] = ff[V];
-      hbw[p] = hb;
+      g.np[p] = ff[V];
+      g.hbw[p] = hb;
+    }
+    return g;
+  }
+  template <int N>
+  bool linear_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, const double* times, int r, double* coef, double* cost) {
+    constexpr int H = N / 2;
+    scratch_.reset();
+    const int totV = vtx_off[B], totS = totV - B;
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) return false;
+    const GenVertices gv = gen_vertices<N>(B, vtx_off, vmask);
+    const std::vector<int>&vfree = gv.vfree, &np = gv.np, &hbw = gv.hbw;
+    std::vector<long long> ws_off(B);
+    long long ws_tot = 0;
+    for (int p = 0; p < B; ++p) {
       ws_off[p] = ws_tot;
-      ws_tot += (long long)gen::ws_doubles<N>(V - 1, np[p], hb);
+      ws_tot += (long long)gen::ws_doubles<N>(vtx_off[p + 1] - vtx_off[p] - 1, np[p], hbw[p]);
     }
     int* d_vtx_off = scratch_.template alloc<int>((size_t)B + 1);
     uint8_t* d_vmask = scratch_.template alloc<uint8_t>(totV);
@@ -1418,6 +1433,179 @@ class Pipeline {
       if (full) be_.d2h(full + 19 * (size_t)dst[p], d_full + 19 * (size_t)smp_off[p], sizeof(double) * 19 * (size_t)counts[p]);
     }
   }
+  // per-segment maxima of |v|,|a|,|j| for the three dimension groups, N-coefficient segments
+  template <int N>
+  void extrema_batch_n(int totS, const double* coef, const double* times, double* maxima) {
+    scratch_.reset();
+    double* d_coef = scratch_.template alloc<double>((size_t)totS * TG_D * N);
+    double* d_T = scratch_.template alloc<double>(totS);
+    double* d_m = scratch_.template alloc<double>((size_t)totS * 9);
+    be_.h2d(d_coef, coef, sizeof(double) * (size_t)totS * TG_D * N);
+    be_.h2d(d_T, times, sizeof(double) * totS);
+    extrema_segments_n<N>(d_coef, d_T, d_m, (size_t)totS, nullptr, nullptr);
+    counters.root_finds += (long long)totS * 9;
+    counters.root_finds_executed += (long long)totS * 9;
+    be_.d2h(maxima, d_m, sizeof(double) * (size_t)totS * 9);
+  }
+  // PolynomialOptimization<N>::computeMaximumOfMagnitude(derivative) for B trajectories (lin_impl.h:477-508)
+  template <int N>
+  void max_magnitude_batch_n(int B, const int* seg_off, const double* coef, const double* times, int derivative, double* value, double* time,
+                             int* segment_idx) {
+    scratch_.reset();
+    const int totS = seg_off[B];
+    int* d_off = scratch_.template alloc<int>((size_t)B + 1);
+    double* d_coef = scratch_.template alloc<double>((size_t)totS * TG_D * N);
+    double* d_T = scratch_.template alloc<double>(totS);
+    double* d_sv = scratch_.template alloc<double>(totS);
+    double* d_st = scratch_.template alloc<double>(totS);
+    double* d_v = scratch_.template alloc<double>(B);
+    double* d_t = scratch_.template alloc<double>(B);
+    int* d_i = scratch_.template alloc<int>(B);
+    be_.h2d(d_off, seg_off, sizeof(int) * ((size_t)B + 1));
+    be_.h2d(d_coef, coef, sizeof(double) * (size_t)totS * TG_D * N);
+    be_.h2d(d_T, times, sizeof(double) * totS);
+    switch (derivative) {
+      case 1: be_.for_each_scratch((size_t)totS, gen::MaxMagnitudeSegFn<N, 1>{d_coef, d_T, d_sv, d_st}); break;
+      case 2: be_.for_each_scratch((size_t)totS, gen::MaxMagnitudeSegFn<N, 2>{d_coef, d_T, d_sv, d_st}); break;
+      case 3: be_.for_each_scratch((size_t)totS, gen::MaxMagnitudeSegFn<N, 3>{d_coef, d_T, d_sv, d_st}); break;
+      default: be_.for_each_scratch((size_t)totS, gen::MaxMagnitudeSegFn<N, 4>{d_coef, d_T, d_sv, d_st}); break;
+    }
+    be_.for_each((size_t)B, MaxMagnitudeReduceFn{d_off, d_sv, d_st, d_v, d_t, d_i});
+    launches(2);
+    counters.root_finds += totS;
+    counters.root_finds_executed += totS;
+    be_.d2h(value, d_v, sizeof(double) * B);
+    be_.d2h(time, d_t, sizeof(double) * B);
+    be_.d2h(segment_idx, d_i, sizeof(int) * B);
+  }
+  // Trajectory::scaleSegmentTimesToMeetConstraints in place, N-coefficient segments
+  template <int N>
+  void scale_times_batch_n(int B, const int* seg_off, double* coef, double* times, const double* L9, int* passes, uint8_t* within) {
+    scratch_.reset();
+    Bare bb = bare_batch(B, seg_off, 2);
+    BatchPtrs& b = bb.b;
+    b.times = scratch_.template alloc<double>(b.totS);
+    b.coef = scratch_.template alloc<double>((size_t)b.totS * TG_D * N);
+    b.maxima = scratch_.template alloc<double>((size_t)b.totS * 9);
+    be_.h2d(b.times, times, sizeof(double) * b.totS);
+    be_.h2d(b.coef, coef, sizeof(double) * (size_t)b.totS * TG_D * N);
+    scale_loop_n<N>(b, L9);
+    ScaleOutFn of{b.ps, b.maxima, bb.d_seg_off, {}, nullptr, nullptr, scale_tolerance};
+    for (int i = 0; i < 9; ++i) of.L[i] = L9[i];
+    of.passes = scratch_.template alloc<int>(B);
+    of.within = scratch_.template alloc<uint8_t>(B);
+    be_.for_each(B, of); launches(1);
+    be_.d2h(coef, b.coef, sizeof(double) * (size_t)b.totS * TG_D * N);
+    be_.d2h(times, b.times, sizeof(double) * b.totS);
+    if (passes) be_.d2h(passes, of.passes, sizeof(int) * B);
+    if (within) be_.d2h(within, of.within, B);
+  }
+  // PolynomialOptimizationNonLinear<N>::setupFromVertices + optimize() (Mellinger outer loop, nl_impl.h:159-234, then the time
+  // scaling of scaleSegmentTimesWithViolation, 335-427) + getTrajectory for B problems given as vertices.  The evaluation runs S+1
+  // solves per running problem with dense launches (a finished problem costs an early exit); the optimiser state machine is the one
+  // of time_alloc_core.  vval: [totV][N/2][4]; coef out: [totS][4][N].
+  template <int N>
+  bool time_alloc_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const Params& P, double* coef,
+                          int* nlopt_code, int* n_evals, int* n_scale_passes, double* final_cost) {
+    constexpr int H = N / 2;
+    scratch_.reset();
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) return false;
+    const GenVertices gv = gen_vertices<N>(B, vtx_off, vmask);
+    std::vector<int> so(B + 1);
+    for (int p = 0; p <= B; ++p) so[p] = vtx_off[p] - p;
+    Bare bb = bare_batch(B, so.data(), P.derivative_to_optimize);
+    BatchPtrs& b = bb.b;
+    const int totS = b.totS, totV = b.totV;
+    // a workspace per solve instance (p, n) = vertex v0 + n; the final solve of problem p reuses that of instance (p, 0)
+    std::vector<long long> ws_inst(totV), ws_prob(B);
+    long long ws_tot = 0;
+    for (int p = 0; p < B; ++p) {
+      const int S = so[p + 1] - so[p];
+      const long long w = (long long)gen::ws_doubles<N>(S, gv.np[p], gv.hbw[p]);
+      ws_prob[p] = ws_tot;
+      for (int n = 0; n <= S; ++n, ws_tot += w) ws_inst[(size_t)vtx_off[p] + n] = ws_tot;
+    }
+    const int mf = (P.max_evals > 0) ? std::min(std::max(P.max_evals, 1), kPlisMfMax) : kPlisMfMax;
+    int* d_vtx_off = scratch_.template alloc<int>((size_t)B + 1);
+    long long* d_ws_inst = scratch_.template alloc<long long>(totV);
+    long long* d_ws_prob = scratch_.template alloc<long long>(B);
+    double* d_ws = scratch_.template alloc<double>((size_t)std::max<long long>(ws_tot, 1));
+    double* d_cost = scratch_.template alloc<double>(B);
+    b.vmask = scratch_.template alloc<uint8_t>(totV);
+    b.vval = scratch_.template alloc<double>((size_t)totV * H * TG_D);
+    b.vfree = scratch_.template alloc<int>(gv.vfree.size());
+    b.np = scratch_.template alloc<int>(B);
+    b.hbw = scratch_.template alloc<int>(B);
+    b.times = scratch_.template alloc<double>(totS);
+    b.coef = scratch_.template alloc<double>((size_t)totS * TG_D * N);
+    b.recs = scratch_.template alloc<double>((size_t)totS * 3 * gen::Rec<N>::kSize);
+    b.costs = scratch_.template alloc<double>(totV);
+    b.maxima = scratch_.template alloc<double>((size_t)totS * 9);
+    b.xeval = scratch_.template alloc<double>(totS);
+    b.x = scratch_.template alloc<double>(totS);
+    b.g = scratch_.template alloc<double>(totS);
+    b.d = scratch_.template alloc<double>(totS);
+    b.ix = scratch_.template alloc<int>(totS);
+    b.hist_s = scratch_.template alloc<double>((size_t)mf * totS);
+    b.hist_y = scratch_.template alloc<double>((size_t)mf * totS);
+    b.opt = scratch_.template alloc<PlisScalars>(B);
+    for (int k = 0; k < 2; ++k) {
+      b.act_prob[k] = scratch_.template alloc<int>(B);
+      b.act_vtx[k] = scratch_.template alloc<int>(totV);
+      b.act_seg[k] = scratch_.template alloc<int>(totS);
+    }
+    be_.h2d(d_vtx_off, vtx_off, sizeof(int) * ((size_t)B + 1));
+    be_.h2d(d_ws_inst, ws_inst.data(), sizeof(long long) * totV);
+    be_.h2d(d_ws_prob, ws_prob.data(), sizeof(long long) * B);
+    be_.h2d(b.vmask, vmask, totV);
+    be_.h2d(b.vval, vval, sizeof(double) * (size_t)totV * H * TG_D);
+    be_.h2d(b.vfree, gv.vfree.data(), sizeof(int) * gv.vfree.size());
+    be_.h2d(b.np, gv.np.data(), sizeof(int) * B);
+    be_.h2d(b.hbw, gv.hbw.data(), sizeof(int) * B);
+    be_.h2d(b.times, times, sizeof(double) * totS);
+    be_.dev_memset(b.stats + 9, 0, 6 * sizeof(int));
+    be_.for_each(B, PlisBeginFn{b, P.max_evals}); launches(1);
+    // maxeval is tested between iterations only, so a line search may overrun it: loop until no problem is left running
+    const int eval_cap = (P.max_evals > 0 ? P.max_evals : 1000) + 64;
+    for (int e = 0; e < eval_cap; ++e) {
+      const int nbuf = (e & 1) ^ 1;
+      be_.dev_memset(b.stats + 7, 0, sizeof(int));
+      be_.dev_memset(b.stats + 9 + 3 * nbuf, 0, 3 * sizeof(int));
+      be_.for_each((size_t)totS * 3, gen::MellingerHeadFn<N>{b});
+      be_.for_each((size_t)totS * 3 * N, gen::MellingerHrowFn<N>{b});
+      be_.for_each_warp((size_t)totV, gen::MellingerSolveFn<N>{b, d_ws_inst, d_ws});
+      be_.for_each(B, PlisAdvanceFn{b, P.max_evals, P.f_rel, P.x_rel, nullptr, nbuf});
+      launches(4);
+      counters.mellinger_launches += 1;
+      int running = 0;
+      be_.d2h(&running, b.stats + 7, sizeof(int));
+      if (running == 0) break;
+    }
+    be_.for_each(B, PlisFinishFn{b}); launches(1);
+    scale_loop_n<N>(b, P.limits);
+    // the final solve at the stretched times
+    be_.for_each((size_t)totS, gen::RecordHeadFn<N>{b.r, b.times, b.recs});
+    be_.for_each((size_t)totS * N, gen::RecordHrowFn<N>{b.recs});
+    be_.for_each_warp((size_t)B, gen::SolveFn<N>{b.r, d_vtx_off, b.vmask, b.vfree, b.vval, b.np, b.hbw, b.recs, d_ws_prob, d_ws, b.coef, d_cost});
+    launches(3);
+    std::vector<ProbState> ps(B);
+    be_.d2h(ps.data(), b.ps, sizeof(ProbState) * B);
+    for (int p = 0; p < B; ++p) {
+      if (nlopt_code) nlopt_code[p] = ps[p].nlopt_code;
+      if (n_evals) n_evals[p] = ps[p].n_evals;
+      if (n_scale_passes) n_scale_passes[p] = ps[p].n_scale_passes;
+      if (final_cost) final_cost[p] = ps[p].final_cost;
+      const int S = so[p + 1] - so[p];
+      counters.evals += ps[p].n_evals;
+      counters.solves += (long long)ps[p].n_evals * (S == 1 ? 1 : S + 1) + 1;
+      if (ps[p].n_evals > 0) counters.root_finds += (long long)(ps[p].n_scale_passes + 1) * 9 * S;
+    }
+    counters.segment_setups += totS;
+    be_.d2h(times, b.times, sizeof(double) * totS);
+    if (coef) be_.d2h(coef, b.coef, sizeof(double) * (size_t)totS * TG_D * N);
+    return true;
+  }
 
   size_t objective_chunk = (size_t)1 << 15;
   size_t sweep_chunk = (size_t)1 << 17;
@@ -1498,6 +1686,49 @@ class Pipeline {
       run_lists("completion");
       launches(1);
     }
+  }
+
+  // scale_loop for N-coefficient segments: the same passes, with exact maxima for every segment that changed (no certificates)
+  template <int N>
+  void scale_loop_n(BatchPtrs& b, const double* L9) {
+    const size_t totS = (size_t)b.totS;
+    gen::ScaleFn<N> sf{b, {}, scratch_.template alloc<uint8_t>(totS)};
+    ScaleCheckFn cf{b, {}, scale_tolerance};
+    for (int i = 0; i < 9; ++i) { sf.L[i] = L9[i]; cf.L[i] = L9[i]; }
+    uint8_t* wflag = scratch_.template alloc<uint8_t>(totS);
+    int* work = scratch_.template alloc<int>(totS);
+    int* n_work = scratch_.template alloc<int>(1);
+    extrema_segments_n<N>(b.coef, b.times, b.maxima, totS, nullptr, nullptr);
+    counters.root_finds_executed += (long long)totS * 9;
+    for (int pass = 0; pass < 20; ++pass) {
+      be_.dev_memset(b.stats + 1, 0, sizeof(int));
+      be_.for_each(totS, sf);
+      be_.for_each(totS, ExtremaWorkFn{b.prob_of_seg, b.ps, sf.changed, wflag});
+      be_.select_flagged(wflag, work, n_work, (int)totS);
+      extrema_segments_n<N>(b.coef, b.times, b.maxima, totS, work, n_work);
+      be_.for_each((size_t)b.B, cf);
+      launches(3);
+      int st[2];  // stats[1]: problems still to scale
+      be_.d2h(st, b.stats, sizeof(st));
+      int nw = 0;
+      be_.d2h(&nw, n_work, sizeof(int));
+      counters.root_finds_executed += (long long)nw * 9;
+      if (st[1] == 0) break;
+    }
+  }
+  template <int N>
+  void extrema_segments_n(const double* coef, const double* times, double* maxima, size_t n_max, const int* work, const int* n_dev) {
+    if (n_max == 0) return;
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 0>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 1>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 2>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 3>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 4>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 5>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 6>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 7>{coef, times, maxima, work, n_dev});
+    be_.for_each_scratch(n_max, gen::ExtremaFn<N, 8>{coef, times, maxima, work, n_dev});
+    launches(9);
   }
 
   // TG_TRACE_PRUNE=1: prints how many (segment, quantity) pairs still need root finding after each certificate stage

@@ -1,9 +1,15 @@
 #!/usr/bin/env python3
-"""Measures the general-shape path (tg_solve_linear_batch_nd, csrc/tg_generic.cuh) on one GPU beside the CPU oracle compiled for the
-same N: B problems of 11 vertices (10 segments), linear optimisation only.  Prints one JSON object per shape; the N = 10, D = 4 line
-also times the tuned kernels on the same problems.  Usage (GPU box): python tools/bench_general_shape.py > profiles/rNN_general_shape.json"""
+"""Measures the general-shape path (csrc/tg_generic.cuh) on one GPU beside the CPU oracle compiled for the same N, on B problems of 11
+vertices (10 segments):
+  * linear optimisation (tg_solve_linear_batch_nd), B = $TG_GS_B (65536), five shapes;
+  * Mellinger time allocation (tg_time_alloc_batch_nd), B = $TG_GS_TA_B (16384), D = 4, N in {6, 8, 10, 12}.
+Prints the card (name, power limit, max SM clock) first, then one JSON object per measurement; the N = 10, D = 4 lines also time the
+tuned kernels on the same problems and say whether both paths give the same bits.
+Usage (GPU box): python tools/bench_general_shape.py > profiles/rNN_general_shape.json"""
+import ctypes as C
 import json
 import os
+import subprocess
 import sys
 import time
 
@@ -29,9 +35,62 @@ def problems(n_coef, dims, B, V=11, seed=0):
     return off, mask.reshape(-1), vals.reshape(B * V, H, dims), times.reshape(-1)
 
 
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True)
+    return {"card": q.stdout.strip()}
+
+
+def time_alloc_lines(ctx, B):
+    """PolynomialOptimizationNonLinear<N>(4)::optimize() with the Mellinger method for B problems per call."""
+    for n_coef in (6, 8, 10, 12):
+        r = 2
+        off, mask, vals, times = problems(n_coef, 4, B, seed=7)
+        P = ctx.L.default_params(derivative_to_optimize=r)
+        ms = []
+        for rep in range(4):
+            out = ctx.time_alloc_batch_nd(n_coef, 4, off, mask, vals, times, P)
+            ms.append(ctx.last_device_ms())
+        dev = float(np.median(ms[1:]))
+        line = {"time_alloc": {"N": n_coef, "D": 4, "derivative_to_optimize": r}, "problems": B, "segments_per_problem": 10,
+                "device_ms": dev, "problems_per_s_device": B / (1e-3 * dev) if dev > 0 else None,
+                "mean_evaluations": float(out["n_evals"].mean()), "mean_scale_passes": float(out["n_scale_passes"].mean()),
+                "note": "device_ms = CUDA events around the call (copies in and out included); no Bernstein pruning, dense evaluation launches"}
+        ctx.set_profiling(True)
+        ctx.time_alloc_batch_nd(n_coef, 4, off, mask, vals, times, P)
+        prof = ctx.profile()
+        ctx.set_profiling(False)
+        line["kernel_ms"] = {k: [round(v[0], 3), int(v[1])] for k, v in prof.items()}  # kernel: [ms, launches]
+        if n_coef == 10:
+            tm = []
+            for rep in range(4):
+                tuned = ctx.time_alloc_batch(off, mask, vals, times, P)
+                tm.append(ctx.last_device_ms())
+            line["tuned_kernels_device_ms"] = float(np.median(tm[1:]))
+            line["general_equals_tuned_bit_for_bit"] = bool(all(np.array_equal(out[k], tuned[k]) for k in out))
+        orc = O.OracleN(n_coef)
+        v4 = vals  # D = 4 already
+        Po = O.Params()
+        C.memmove(C.byref(Po), C.byref(P), C.sizeof(O.Params))
+        nb, same, t0 = 64, True, time.perf_counter()
+        for p in range(nb):
+            t = np.array(times[p * 10:(p + 1) * 10])
+            c = np.zeros((10, 4, n_coef))
+            code, ev, ps, cost = C.c_int(), C.c_int(), C.c_int(), C.c_double()
+            m = np.ascontiguousarray(mask[p * 11:(p + 1) * 11])
+            vv = np.ascontiguousarray(v4[p * 11:(p + 1) * 11])
+            orc.lib.orc_time_alloc(11, m.ctypes.data_as(C.POINTER(C.c_uint8)), vv.ctypes.data_as(C.POINTER(C.c_double)),
+                                   t.ctypes.data_as(C.POINTER(C.c_double)), r, C.byref(Po), c.ctypes.data_as(C.POINTER(C.c_double)), C.byref(code),
+                                   C.byref(ev), C.byref(ps), C.byref(cost))
+            same = same and np.array_equal(t, out["times"][p * 10:(p + 1) * 10]) and np.array_equal(c, out["coef"][p * 10:(p + 1) * 10])
+        line["cpu_oracle_problems_per_s_one_thread"] = nb / (time.perf_counter() - t0)
+        line["bit_exact_vs_oracle_first_64"] = bool(same)
+        print(json.dumps(line), flush=True)
+
+
 def main():
     B = int(os.environ.get("TG_GS_B", "65536"))
     ctx = tg.Context(tg.Library(), 0)
+    print(json.dumps(card()), flush=True)
     for n_coef, dims, r in ((6, 3, 2), (8, 4, 3), (10, 4, 2), (12, 4, 4), (12, 1, 5)):
         off, mask, vals, times = problems(n_coef, dims, B)
         ms, wall = [], []
@@ -73,6 +132,7 @@ def main():
         line["cpu_oracle_problems_per_s_one_thread"] = nb / cpu
         line["bit_exact_vs_oracle_first_256"] = bool(same)
         print(json.dumps(line), flush=True)
+    time_alloc_lines(ctx, int(os.environ.get("TG_GS_TA_B", "16384")))
 
 
 if __name__ == "__main__":
