@@ -222,6 +222,35 @@ int tg_objective_batch(tg_ctx* ctx, int V, const uint8_t* vmask, const double* v
                        int nvar, double time_penalty, int use_soft_constraints, double soft_constraint_weight, int n_constraints,
                        const int* con_derivative, const double* con_value, double* total, double* parts, double* coef);
 
+/* tg_time_alloc_dfo_batch = PolynomialOptimizationNonLinear<10>::optimize() with the derivative-free time-allocation methods
+ *   (optimizeTime / optimizeTimeAndFreeConstraints, nl_impl.h:120-157, 429-536) for B problems in one call.  The reference hands
+ *   the objective to NLopt's LN_BOBYQA; here the objective (tg_objective_batch's, bit for bit), the bounds
+ *   (kOptimizationTimeLowerBound; setFreeEndpointDerivativeHardConstraints, nl_impl.h:764-805, including its counter that only
+ *   advances for derivatives <= derivative_to_optimize), the initial steps (nl_impl.h:488-495) and the stopping rules are the
+ *   reference's, and the search is a bound-constrained coordinate pattern search (2n candidates per iteration; first strict
+ *   minimum accepted when it improves, every step halved otherwise; codes 3 ftol_rel, 4 xtol_rel, 5 max_iterations).  Methods 3, 4
+ *   start the free derivatives at the linear solution of the initial times (nl_impl.h:436-462).
+ *   Inputs as tg_time_alloc_batch: vtx_off[B+1], vmask[totV], vval[totV][5][4]; times[totS] initial times in, allocated out.
+ *   The constraints (addMaximumMagnitudeConstraint, nl_impl.h:538-565) are shared by every problem: at most 16, dimension 0..3,
+ *   derivative 1..4, value != 0.  Outputs (any may be NULL): coef[totS][4][10] at the final point; vval_out[totV][5][4] (methods 3, 4)
+ *   the fixed values with every free slot at its final variable; code[B]; n_iterations[B]; total[B] the best objective;
+ *   parts[B][3] = {cost_trajectory, cost_time, cost_soft_constraints} at the final point.  TG_ERR_INVALID, with no output written,
+ *   for B < 1, a problem with fewer than two vertices, a method other than 0, 1, 3, 4, derivative_to_optimize outside 2..4 or an
+ *   invalid constraint.  max_iterations <= 0 runs no iteration (code 5). */
+typedef struct tg_dfo_params {
+  int time_alloc_method;          /* 0, 1, 3 or 4 */
+  int derivative_to_optimize;     /* 2 .. 4 */
+  int max_iterations;             /* batched search iterations (10) */
+  double f_rel, x_rel, initial_stepsize_rel;  /* 0.05, 0.1, 0.1 */
+  double time_penalty;            /* 500 */
+  int use_soft_constraints;       /* 1 */
+  double soft_constraint_weight;  /* 100 */
+} tg_dfo_params;
+void tg_default_dfo_params(tg_dfo_params* p);
+int tg_time_alloc_dfo_batch(tg_ctx* ctx, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                            const tg_dfo_params* params, int n_constraints, const int* con_dimension, const int* con_derivative,
+                            const double* con_value, double* coef, double* vval_out, int* code, int* n_iterations, double* total, double* parts);
+
 /* The steps either side of the path (SURVEY.md 8f ranks 1-2), batched, one path per thread --------------------------------
  * tg_preprocess_paths = MrsTrajectoryGeneration::preprocessPath (src/mrs_trajectory_generation.cpp:431-500): optional path
  *   straightener (config/public/trajectory_generation.yaml:20-23) then the min_waypoint_distance filter (:27).

@@ -35,6 +35,22 @@ class Params(C.Structure):
     ]
 
 
+class DfoParams(C.Structure):
+    """tg_dfo_params (include/tg_b200.h): the NonlinearOptimizationParameters fields the derivative-free methods read."""
+
+    _fields_ = [
+        ("time_alloc_method", C.c_int),
+        ("derivative_to_optimize", C.c_int),
+        ("max_iterations", C.c_int),
+        ("f_rel", C.c_double),
+        ("x_rel", C.c_double),
+        ("initial_stepsize_rel", C.c_double),
+        ("time_penalty", C.c_double),
+        ("use_soft_constraints", C.c_int),
+        ("soft_constraint_weight", C.c_double),
+    ]
+
+
 class Result(C.Structure):
     """tg_result (include/tg_b200.h)."""
 
@@ -131,6 +147,9 @@ class Library:
         L.tg_time_alloc_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.POINTER(Params), _dp, _ip, _ip, _ip, _dp]
         L.tg_objective_batch.argtypes = [C.c_void_p, C.c_int, _u8p, _dp, C.c_int, C.c_int, C.c_longlong, _dp, C.c_int, C.c_double, C.c_int, C.c_double,
                                          C.c_int, _ip, _dp, _dp, _dp, _dp]
+        L.tg_default_dfo_params.argtypes = [C.POINTER(DfoParams)]
+        L.tg_time_alloc_dfo_batch.argtypes = [C.c_void_p, C.c_int, _ip, _u8p, _dp, _dp, C.POINTER(DfoParams), C.c_int, _ip, _ip, _dp, _dp, _dp, _ip,
+                                              _ip, _dp, _dp]
         L.tg_max_magnitude_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
         L.tg_scale_times_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp, _ip, _u8p]
         L.tg_sweep_costs.argtypes = [C.c_void_p, C.c_int, _u8p, _dp, C.c_int, C.c_longlong, _dp, C.c_int, _dp, _llp, _dp]
@@ -152,6 +171,13 @@ class Library:
                     p.limits[i] = x
             else:
                 setattr(p, k, v)
+        return p
+
+    def default_dfo_params(self, **kw):
+        p = DfoParams()
+        self.lib.tg_default_dfo_params(C.byref(p))
+        for k, v in kw.items():
+            setattr(p, k, v)
         return p
 
     @staticmethod
@@ -340,6 +366,32 @@ class Context:
         self._check(self.L.lib.tg_time_alloc_batch(self.h, B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times), C.byref(P), _p(coef),
                                                    _p(code, _ip), _p(evals, _ip), _p(passes, _ip), _p(cost)))
         return {"times": times, "coef": coef, "nlopt_code": code, "n_evals": evals, "n_scale_passes": passes, "final_cost": cost}
+
+    def time_alloc_dfo_batch(self, vtx_off, vmask, vval, times, params=None, constraints=()):
+        """PolynomialOptimizationNonLinear::optimize() with a derivative-free method (0, 1, 3, 4) for B problems given as vertices.
+        constraints: (dimension, derivative, value) shared by every problem.  Returns a dict with the allocated times, the
+        coefficients at the final point, vval (methods 3, 4: the free slots at their final values), code / n_iterations / total per
+        problem and parts [B][3] = cost_trajectory, cost_time, cost_soft_constraints."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        vmask = np.ascontiguousarray(vmask, dtype=np.uint8)
+        vval = np.ascontiguousarray(vval, dtype=np.float64)
+        times = np.array(times, dtype=np.float64, copy=True)
+        B = len(vtx_off) - 1
+        totS = int(vtx_off[-1]) - B
+        P = params or self.L.default_dfo_params()
+        cdim = np.ascontiguousarray([c[0] for c in constraints], dtype=np.int32)
+        cder = np.ascontiguousarray([c[1] for c in constraints], dtype=np.int32)
+        cval = np.ascontiguousarray([c[2] for c in constraints], dtype=np.float64)
+        coef = np.empty((totS, D, N))
+        vval_out = vval.copy() if P.time_alloc_method >= 3 else None
+        code = np.zeros(B, dtype=np.int32)
+        iters = np.zeros(B, dtype=np.int32)
+        total = np.zeros(B)
+        parts = np.zeros((B, 3))
+        self._check(self.L.lib.tg_time_alloc_dfo_batch(self.h, B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times), C.byref(P), len(cdim),
+                                                       _p(cdim, _ip), _p(cder, _ip), _p(cval), _p(coef), _p(vval_out), _p(code, _ip),
+                                                       _p(iters, _ip), _p(total), _p(parts)))
+        return {"times": times, "coef": coef, "vval": vval_out, "code": code, "n_iterations": iters, "total": total, "parts": parts}
 
     # ---- the steps either side of the path (SURVEY.md 8f) ---------------------------------------------------------------
     def preprocess_paths(self, wp_off, wp, stop_at=None, min_waypoint_distance=0.05, straightener=False, max_deviation=0.05, max_hdg_deviation=0.1):

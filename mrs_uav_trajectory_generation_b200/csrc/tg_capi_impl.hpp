@@ -588,6 +588,50 @@ int tg_objective_batch(tg_ctx* ctx, int V, const uint8_t* vmask, const double* v
   });
 }
 
+void tg_default_dfo_params(tg_dfo_params* p) {
+  if (!p) return;
+  p->time_alloc_method = 0;
+  p->derivative_to_optimize = 2;
+  p->max_iterations = 10;
+  p->f_rel = 0.05;
+  p->x_rel = 0.1;
+  p->initial_stepsize_rel = 0.1;
+  p->time_penalty = 500.0;
+  p->use_soft_constraints = 1;
+  p->soft_constraint_weight = 100.0;
+}
+
+int tg_time_alloc_dfo_batch(tg_ctx* ctx, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                            const tg_dfo_params* params, int n_constraints, const int* con_dimension, const int* con_derivative,
+                            const double* con_value, double* coef, double* vval_out, int* code, int* n_iterations, double* total, double* parts) {
+  static_assert(sizeof(tg_dfo_params) == sizeof(tg::DfoParams), "tg_dfo_params / tg::DfoParams layout mismatch");
+  return tg_guard(ctx, [&]() -> int {
+    if (B < 1 || !vtx_off || !vmask || !vval || !times || !params || n_constraints < 0 ||
+        (n_constraints > 0 && (!con_dimension || !con_derivative || !con_value))) {
+      ctx->err = "invalid argument";
+      return TG_ERR_INVALID;
+    }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) { ctx->err = "every problem needs at least two vertices"; return TG_ERR_INVALID; }
+    const int m = params->time_alloc_method;
+    if (!(m == 0 || m == 1 || m == 3 || m == 4)) { ctx->err = "time_alloc_method must be 0, 1, 3 or 4"; return TG_ERR_INVALID; }
+    if (params->derivative_to_optimize < 2 || params->derivative_to_optimize > 4) { ctx->err = "derivative_to_optimize must be 2..4"; return TG_ERR_INVALID; }
+    if (n_constraints > 16) { ctx->err = "at most 16 constraints"; return TG_ERR_INVALID; }
+    for (int c = 0; c < n_constraints; ++c)
+      if (con_derivative[c] < 1 || con_derivative[c] > 4 || con_dimension[c] < 0 || con_dimension[c] > 3 || !(con_value[c] != 0.0)) {
+        ctx->err = "constraints need dimension 0..3, derivative 1..4 and a non-zero value";
+        return TG_ERR_INVALID;
+      }
+    tg::DfoParams P;
+    std::memcpy(&P, params, sizeof(P));
+    ctx->be.timer_start();
+    ctx->pipe.dfo_batch(B, vtx_off, vmask, vval, times, P, n_constraints, con_dimension, con_derivative, con_value, coef, vval_out, code,
+                        n_iterations, total, parts);
+    ctx->last_ms = ctx->be.timer_stop();
+    return TG_OK;
+  });
+}
+
 int tg_scale_times_batch(tg_ctx* ctx, int B, const int* seg_off, double* coef, double* times, const double* limits9, int* passes,
                          uint8_t* within) {
   return tg_guard(ctx, [&]() -> int {

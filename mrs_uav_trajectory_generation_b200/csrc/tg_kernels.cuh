@@ -322,36 +322,43 @@ struct FillFreeFn {
 // total = cost_trajectory + cost_time + cost_soft_constraints (nl_impl.h:613, 721); soft constraints as
 // min(maximum_cost, exp(relative_violation * weight)) summed in constraint order (nl_impl.h:740-762), the maxima of the
 // distinct derivatives precomputed per candidate (maxval[derivative - 1][k])
-struct ObjCombineFn {
-  int S, method, ncon;
+struct ObjTerms {
+  int method, ncon;
   double time_penalty, soft_weight;
   int use_soft;
-  const double* times;   // [K][S]
-  const double* costs;   // [K] trajectory cost
-  const double* maxval;  // [4][K]
-  size_t K;
   int con_deriv[16];
   double con_value[16];
-  double* total;
-  double* parts;  // optional [K][3]
-  TG_HD void operator()(size_t k) const {
-    const double cost_traj = costs[k];
-    double total_time = 0.0;
-    for (int s = 0; s < S; ++s) total_time = total_time + times[k * (size_t)S + s];
+  // maxval[(derivative - 1) * stride] = computeMaximumOfMagnitude(derivative).value of the candidate; parts optional [3]
+  TG_HD double combine(double cost_traj, double total_time, const double* maxval, size_t stride, double* parts) const {
     const double cost_time = (method == 1 || method == 4) ? total_time * time_penalty : total_time * total_time * time_penalty;
     double cost_con = 0.0;
     if (use_soft)
       for (int c = 0; c < ncon; ++c) {
-        const double abs_violation = maxval[(size_t)(con_deriv[c] - 1) * K + k] - con_value[c];
+        const double abs_violation = maxval[(size_t)(con_deriv[c] - 1) * stride] - con_value[c];
         const double relative_violation = abs_violation / con_value[c];
         cost_con = cost_con + dmin(1.0e12, tgdm::dexp(relative_violation * soft_weight));
       }
     if (parts) {
-      parts[3 * k + 0] = cost_traj;
-      parts[3 * k + 1] = cost_time;
-      parts[3 * k + 2] = cost_con;
+      parts[0] = cost_traj;
+      parts[1] = cost_time;
+      parts[2] = cost_con;
     }
-    total[k] = cost_traj + cost_time + cost_con;
+    return cost_traj + cost_time + cost_con;
+  }
+};
+struct ObjCombineFn {
+  int S;
+  ObjTerms terms;
+  const double* times;   // [K][S]
+  const double* costs;   // [K] trajectory cost
+  const double* maxval;  // [4][K]
+  size_t K;
+  double* total;
+  double* parts;  // optional [K][3]
+  TG_HD void operator()(size_t k) const {
+    double total_time = 0.0;
+    for (int s = 0; s < S; ++s) total_time = total_time + times[k * (size_t)S + s];
+    total[k] = terms.combine(costs[k], total_time, maxval + k, K, parts ? parts + 3 * k : nullptr);
   }
 };
 
@@ -378,6 +385,34 @@ TG_HD double cost_partial(const double (&c)[TG_N], const double* __restrict__ Qg
     partial = (b == 0) ? sum * c[R + b] : partial + sum * c[R + b];
   }
   return partial;
+}
+TG_HD double cost_partial_rec(int r, const double (&c)[TG_N], const double* __restrict__ rec) {
+  const double* Q = rec + TG_REC_Q;
+  return (r == 2) ? cost_partial<2>(c, Q) : ((r == 3) ? cost_partial<3>(c, Q) : cost_partial<4>(c, Q));
+}
+// c = A^-1 nd from the segment's record, nd = the ten end-point derivatives of one dimension (0..4 at the start, 0..4 at the end)
+TG_HD void coef_from_endpoints(const double* __restrict__ rec, const double (&nd)[TG_N], double (&c)[TG_N]) {
+  c[0] = 1.0 * nd[0];
+  c[1] = 1.0 * nd[1];
+  c[2] = (1.0 / 2.0) * nd[2];
+  c[3] = (1.0 / 6.0) * nd[3];
+  c[4] = (1.0 / 24.0) * nd[4];
+  double blk[50];  // Dinv (25) then X (25): the first 400 bytes of the record, fetched with 16-byte loads
+#pragma unroll
+  for (int e = 0; e < 50; e += 2) {
+    const Dbl2 t = *reinterpret_cast<const Dbl2*>(rec + e);
+    blk[e] = t.x;
+    blk[e + 1] = t.y;
+  }
+#pragma unroll
+  for (int a = 0; a < TG_HALF; ++a) {
+    double acc = blk[TG_REC_X + a * 5] * nd[0];
+#pragma unroll
+    for (int k = 1; k < 5; ++k) acc = acc + blk[TG_REC_X + a * 5 + k] * nd[k];
+#pragma unroll
+    for (int k = 0; k < 5; ++k) acc = acc + blk[TG_REC_DINV + a * 5 + k] * nd[5 + k];
+    c[TG_HALF + a] = acc;
+  }
 }
 template <class D>
 struct CoefCostFn {
@@ -408,35 +443,12 @@ struct CoefCostFn {
       const uint32_t m = I.vmask[v];
       nd[k] = ((m >> sl) & 1u) ? I.vval[((size_t)v * TG_HALF + sl) * TG_D + d] : I.x_out[(size_t)(I.vfree[v] + free_rank(m, sl)) * 4 + d];
     }
-    c[0] = 1.0 * nd[0];
-    c[1] = 1.0 * nd[1];
-    c[2] = (1.0 / 2.0) * nd[2];
-    c[3] = (1.0 / 6.0) * nd[3];
-    c[4] = (1.0 / 24.0) * nd[4];
-    double blk[50];  // Dinv (25) then X (25): the first 400 bytes of the record, fetched with 16-byte loads
-#pragma unroll
-    for (int e = 0; e < 50; e += 2) {
-      const Dbl2 t = *reinterpret_cast<const Dbl2*>(rec + e);
-      blk[e] = t.x;
-      blk[e + 1] = t.y;
-    }
-#pragma unroll
-    for (int a = 0; a < TG_HALF; ++a) {
-      double acc = blk[TG_REC_X + a * 5] * nd[0];
-#pragma unroll
-      for (int k = 1; k < 5; ++k) acc = acc + blk[TG_REC_X + a * 5 + k] * nd[k];
-#pragma unroll
-      for (int k = 0; k < 5; ++k) acc = acc + blk[TG_REC_DINV + a * 5 + k] * nd[5 + k];
-      c[TG_HALF + a] = acc;
-    }
+    coef_from_endpoints(rec, nd, c);
     if (I.coef_out) {
 #pragma unroll
       for (int a = 0; a < TG_N; a += 2) store2(I.coef_out + it * TG_N + a, c[a], c[a + 1]);
     }
-    if (I.cost_out) {
-      const double* Q = rec + TG_REC_Q;
-      part[item] = (I.r == 2) ? cost_partial<2>(c, Q) : ((I.r == 3) ? cost_partial<3>(c, Q) : cost_partial<4>(c, Q));
-    }
+    if (I.cost_out) part[item] = cost_partial_rec(I.r, c, rec);
   }
 };
 // The same for all points of a Mellinger evaluation (SolveProblemDesc mode 1), organised by PROBLEM: 128 consecutive items

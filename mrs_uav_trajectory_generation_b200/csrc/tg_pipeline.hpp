@@ -19,6 +19,7 @@
 #include <vector>
 
 #include "tg_kernels.cuh"
+#include "tg_dfo.cuh"
 #include "tg_generic.cuh"
 
 namespace tg {
@@ -795,7 +796,8 @@ class Pipeline {
     launches(2);
   }
 
-  bool coef_cost_by_problem(size_t, const SolveSweepDesc&, const BatchPtrs&, const std::vector<SolveBucket>*, int) { return false; }
+  template <class D>
+  bool coef_cost_by_problem(size_t, const D&, const BatchPtrs&, const std::vector<SolveBucket>*, int) { return false; }
   bool coef_cost_by_problem(size_t, const SolveProblemDesc& desc, const BatchPtrs& b, const std::vector<SolveBucket>*, int per) {
     if (desc.mellinger != 1) return false;
     be_.for_each((size_t)b.B * 128, CoefCostGradFn{CoefCostFn<SolveProblemDesc>{desc, per, b.part, 0, per}, 0, nullptr});
@@ -1286,11 +1288,8 @@ class Pipeline {
           counters.root_finds += (long long)n;
           counters.root_finds_executed += (long long)n;
         }
-      ObjCombineFn cf{S, method, ncon, time_penalty, soft_weight, use_soft, d_T, d_costs, d_max, (size_t)chunk, {}, {}, d_total, d_parts};
-      for (int c = 0; c < ncon; ++c) {
-        cf.con_deriv[c] = con_deriv[c];
-        cf.con_value[c] = con_value[c];
-      }
+      const ObjCombineFn cf{S, obj_terms(method, time_penalty, use_soft, soft_weight, ncon, con_deriv, con_value), d_T, d_costs, d_max, (size_t)chunk,
+                            d_total, d_parts};
       be_.for_each((size_t)kc, cf);
       launches(1);
       be_.d2h(total + k0, d_total, sizeof(double) * (size_t)kc);
@@ -1298,6 +1297,231 @@ class Pipeline {
       if (coef) be_.d2h(coef + (size_t)k0 * S * TG_D * TG_N, d_coef, sizeof(double) * (size_t)kc * S * TG_D * TG_N);
     }
     return 0;
+  }
+  static ObjTerms obj_terms(int method, double time_penalty, int use_soft, double soft_weight, int ncon, const int* con_deriv, const double* con_value) {
+    ObjTerms t{method, ncon, time_penalty, soft_weight, use_soft, {}, {}};
+    for (int c = 0; c < ncon; ++c) {
+      t.con_deriv[c] = con_deriv[c];
+      t.con_value[c] = con_value[c];
+    }
+    return t;
+  }
+
+  // The derivative-free time allocation (tg_dfo.cuh) for B problems given as vertices; the caller has validated the inputs.
+  // Problems are cut into groups of consecutive problems of at most seg_budget candidate segments (the segments the candidates of
+  // one iteration recompute: S per candidate for methods 0, 1, two for 3, 4); a group runs its whole search before the next starts.
+  void dfo_batch(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const DfoParams& Q, int ncon, const int* con_dim,
+                 const int* con_deriv, const double* con_value, double* coef, double* vval_out, int* code, int* n_iter, double* total, double* parts) {
+    const bool with_free = Q.time_alloc_method >= 3;
+    std::vector<size_t> units(B);
+    for (int p = 0; p < B; ++p) {
+      const int V = vtx_off[p + 1] - vtx_off[p], S = V - 1;
+      int nf = 0;
+      for (int v = vtx_off[p]; v < vtx_off[p + 1]; ++v)
+        for (int k = 0; k < TG_HALF; ++k) nf += ((vmask[v] >> k) & 1u) ? 0 : 1;
+      const size_t n = (size_t)(with_free ? S + TG_D * nf : S);
+      units[p] = 2 * n * (size_t)(with_free ? 2 : S);
+    }
+    for (int p0 = 0; p0 < B;) {
+      int p1 = p0 + 1;
+      size_t u = units[p0];
+      while (p1 < B && u + units[p1] <= seg_budget) u += units[p1++];
+      dfo_group(p0, p1, vtx_off, vmask, vval, times, Q, ncon, con_dim, con_deriv, con_value, coef, vval_out, code, n_iter, total, parts);
+      p0 = p1;
+    }
+  }
+  void dfo_group(int p0, int p1, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const DfoParams& Q, int ncon,
+                 const int* con_dim, const int* con_deriv, const double* con_value, double* coef, double* vval_out, int* code, int* n_iter,
+                 double* total, double* parts) {
+    scratch_.reset();
+    const int G = p1 - p0, method = Q.time_alloc_method;
+    const bool with_free = method >= 3;
+    const size_t gv0 = (size_t)vtx_off[p0], gs0 = gv0 - (size_t)p0;
+    std::vector<int> so(G + 1);
+    for (int i = 0; i <= G; ++i) so[i] = vtx_off[p0 + i] - (int)gv0 - i;
+    Bare bb = bare_batch(G, so.data(), Q.derivative_to_optimize);
+    BatchPtrs& b = bb.b;
+    const int totS = b.totS, totV = b.totV;
+    b.vmask = scratch_.template alloc<uint8_t>(totV);
+    b.vval = scratch_.template alloc<double>((size_t)totV * TG_HALF * TG_D);
+    b.vfree = scratch_.template alloc<int>((size_t)totV + G);
+    b.np = scratch_.template alloc<int>(G);
+    b.hbw = scratch_.template alloc<int>(G);
+    b.fmax = scratch_.template alloc<int>(G);
+    b.times = scratch_.template alloc<double>(totS);
+    b.coef = scratch_.template alloc<double>((size_t)totS * TG_D * TG_N);
+    b.recs = scratch_.template alloc<double>((size_t)totS * 3 * TG_REC_SIZE);
+    be_.h2d(b.vmask, vmask + gv0, totV);
+    be_.h2d(b.vval, vval + gv0 * TG_HALF * TG_D, sizeof(double) * (size_t)totV * TG_HALF * TG_D);
+    be_.h2d(b.times, times + gs0, sizeof(double) * totS);
+    be_.for_each(G, PrepareFn{b, 0});
+    launches(1);
+    int stats[16];
+    be_.d2h(stats, b.stats, sizeof(stats));
+    std::vector<int> np(G);
+    be_.d2h(np.data(), b.np, sizeof(int) * G);
+    // per-problem layout of the variables, candidates (2 n) and candidate items
+    std::vector<DfoProb> hp(G);
+    size_t totN = 0, totCand = 0, totItems = 0;
+    for (int i = 0; i < G; ++i) {
+      DfoProb& P = hp[i];
+      std::memset(&P, 0, sizeof(P));
+      P.S = so[i + 1] - so[i];
+      P.n_free = np[i];
+      P.n = with_free ? P.S + TG_D * P.n_free : P.S;
+      P.s0 = so[i];
+      P.x0 = (int)totN;
+      P.c0 = (int)totCand;
+      P.i0 = (int)totItems;
+      totN += (size_t)P.n;
+      totCand += 2 * (size_t)P.n;
+      totItems += 2 * (size_t)P.n * (size_t)(with_free ? 2 : P.S);
+    }
+    DfoBatch d;
+    std::memset(&d, 0, sizeof(d));
+    d.prob = scratch_.template alloc<DfoProb>(G);
+    be_.h2d(d.prob, hp.data(), sizeof(DfoProb) * G);
+    d.method = method;
+    d.max_iter = Q.max_iterations;
+    d.ipc_free = 2;
+    d.f_rel = Q.f_rel;
+    d.x_rel = Q.x_rel;
+    d.step_rel = Q.initial_stepsize_rel;
+    d.obj = obj_terms(method, Q.time_penalty, Q.use_soft_constraints, Q.soft_constraint_weight, ncon, con_deriv, con_value);
+    for (int c = 0; c < ncon; ++c) d.con_dim[c] = con_dim[c];
+    d.x = scratch_.template alloc<double>(totN);
+    d.lo = scratch_.template alloc<double>(totN);
+    d.hi = scratch_.template alloc<double>(totN);
+    d.step = scratch_.template alloc<double>(totN);
+    d.cand_prob = scratch_.template alloc<int>(totCand);
+    d.item_cand = with_free ? nullptr : scratch_.template alloc<int>(totItems);
+    d.ctot = scratch_.template alloc<double>(totCand);
+    d.ccost = with_free ? nullptr : scratch_.template alloc<double>(totCand);
+    d.ccoef = scratch_.template alloc<double>(totItems * TG_D * TG_N);
+    d.cpart = with_free ? scratch_.template alloc<double>(totItems * 4) : nullptr;
+    bool need[4] = {false, false, false, false};
+    for (int c = 0; c < ncon; ++c) need[con_deriv[c] - 1] = Q.use_soft_constraints != 0;
+    d.csv = scratch_.template alloc<double>(4 * totItems);
+    d.bcost = scratch_.template alloc<double>(G);
+    d.bpart = scratch_.template alloc<double>((size_t)totS * 4);
+    d.bsv = scratch_.template alloc<double>((size_t)4 * totS);
+    d.btot = scratch_.template alloc<double>(G);
+    d.bparts = scratch_.template alloc<double>((size_t)3 * G);
+    d.totS = (size_t)totS;
+    d.totItems = totItems;
+    for (int k = 0; k < 2; ++k) {
+      d.lists[k][0] = scratch_.template alloc<int>(G);
+      d.lists[k][1] = scratch_.template alloc<int>(totS);
+      d.lists[k][2] = scratch_.template alloc<int>(totCand);
+      d.lists[k][3] = scratch_.template alloc<int>(totItems);
+    }
+    d.cnt = scratch_.template alloc<int>(9);
+    alloc_solution_buffers(b, with_free ? (size_t)G : totCand, stats);
+    d.b = b;
+    be_.for_each(G, DfoMapFn{d});
+    launches(1);
+    if (with_free) {  // x0 of the free derivatives: the linear solution at the initial times (solveLinear + getFreeConstraints)
+      be_.for_each(totS, SetupBaseFn{b, b.times});
+      solve_with_outputs((size_t)G, stats, SolveProblemDesc{b, 0, nullptr, nullptr}, b);
+      be_.for_each(totV, DfoFreeInitFn{d});
+      launches(3);
+      counters.solves += G;
+      counters.segment_setups += totS;
+    }
+    be_.for_each(G, DfoBeginFn{d});
+    be_.dev_memset(d.cnt, 0, 9 * sizeof(int));
+    launches(1);
+    dfo_base_eval(d, stats, need, 1);
+    int back[5];
+    be_.d2h(back, d.cnt, sizeof(back));
+    for (int it = 0; it < Q.max_iterations && back[0] > 0; ++it) {
+      const int buf = it & 1, nbuf = buf ^ 1;
+      const bool sparse = (size_t)back[0] * 2 < (size_t)G;
+      const int* const* L = sparse ? d.lists[buf] : nullptr;
+      const size_t nprob = sparse ? (size_t)back[1] : (size_t)G, nseg = sparse ? (size_t)back[2] : (size_t)totS;
+      const size_t ncand = sparse ? (size_t)back[3] : totCand, nitem = sparse ? (size_t)back[4] : totItems;
+      be_.dev_memset(d.cnt, 0, sizeof(int));
+      be_.dev_memset(d.cnt + 1 + 4 * nbuf, 0, 4 * sizeof(int));
+      be_.for_each(nseg * 3, DfoRecsFn{d, L ? L[1] : nullptr, 3, 0});
+      launches(1);
+      if (with_free) {
+        be_.for_each(nseg * 4, DfoBaseCoefFn{d, L ? L[1] : nullptr, 0});
+        dfo_maxima(d, need, L ? L[1] : nullptr, nseg, 1, 0);
+        be_.for_each(nitem, DfoItemFn{d, L ? L[3] : nullptr});
+        launches(2);
+      } else {
+        solve_with_outputs(ncand, stats, DfoSolveDesc{d, 0, L ? L[2] : nullptr}, b);
+        launches(1);
+      }
+      dfo_maxima(d, need, L ? L[3] : nullptr, nitem, 0, 0);
+      be_.for_each(ncand, DfoTotalFn{d, L ? L[2] : nullptr});
+      be_.for_each(nprob, DfoAdvanceFn{d, L ? L[0] : nullptr, nbuf});
+      launches(2);
+      // work of the running problems (the lists hold exactly them, dense launches or not)
+      counters.segment_setups += (long long)back[2] * 3;
+      counters.evals += (long long)back[3];
+      if (!with_free) counters.solves += back[3];
+      for (int k = 0; k < 4; ++k)
+        if (need[k]) {
+          counters.root_finds += (long long)back[4] + (with_free ? back[2] : 0);
+          counters.root_finds_executed += (long long)back[4] + (with_free ? back[2] : 0);
+        }
+      int nb[5];
+      be_.d2h(nb, d.cnt, sizeof(int));
+      be_.d2h(nb + 1, d.cnt + 1 + 4 * nbuf, 4 * sizeof(int));
+      std::memcpy(back, nb, sizeof(back));
+    }
+    dfo_base_eval(d, stats, need, 0);  // the final point, with coefficients and the three terms
+    double* d_times = scratch_.template alloc<double>(totS);
+    be_.for_each(totS, DfoTimesOutFn{d, d_times});
+    launches(1);
+    be_.d2h(times + gs0, d_times, sizeof(double) * totS);
+    if (coef) be_.d2h(coef + gs0 * TG_D * TG_N, b.coef, sizeof(double) * (size_t)totS * TG_D * TG_N);
+    if (vval_out && with_free) {
+      double* d_vv = scratch_.template alloc<double>((size_t)totV * TG_HALF * TG_D);
+      be_.for_each(totV, DfoVvalOutFn{d, d_vv});
+      launches(1);
+      be_.d2h(vval_out + gv0 * TG_HALF * TG_D, d_vv, sizeof(double) * (size_t)totV * TG_HALF * TG_D);
+    }
+    be_.d2h(hp.data(), d.prob, sizeof(DfoProb) * G);
+    for (int i = 0; i < G; ++i) {
+      if (code) code[p0 + i] = hp[i].code;
+      if (n_iter) n_iter[p0 + i] = hp[i].iterations;
+      if (total) total[p0 + i] = hp[i].f;
+    }
+    if (parts) be_.d2h(parts + 3 * (size_t)p0, d.bparts, sizeof(double) * 3 * G);
+  }
+  // the objective at every problem's current x: records, coefficients (a linear solve for methods 0, 1), maxima, total
+  void dfo_base_eval(const DfoBatch& d, const int* stats, const bool* need, int start) {
+    const int G = d.b.B, totS = d.b.totS;
+    be_.for_each((size_t)totS, DfoRecsFn{d, nullptr, 1, 1});
+    if (d.method >= 3) {
+      be_.for_each((size_t)totS * 4, DfoBaseCoefFn{d, nullptr, 1});
+    } else {
+      solve_with_outputs((size_t)G, stats, DfoSolveDesc{d, 1, nullptr}, d.b);
+      counters.solves += G;
+    }
+    dfo_maxima(d, need, nullptr, (size_t)totS, 1, 1);
+    be_.for_each((size_t)G, DfoBaseTotalFn{d, start});
+    launches(3);
+    counters.segment_setups += totS;
+    counters.evals += G;
+  }
+  void dfo_maxima(const DfoBatch& d, const bool* need, const int* list, size_t n, int base, int all) {
+    for (int k = 0; k < 4; ++k) {
+      if (!need[k] || n == 0) continue;
+      switch (k + 1) {
+        case 1: be_.for_each_scratch(n, DfoMaxFn<1>{d, list, base, all}); break;
+        case 2: be_.for_each_scratch(n, DfoMaxFn<2>{d, list, base, all}); break;
+        case 3: be_.for_each_scratch(n, DfoMaxFn<3>{d, list, base, all}); break;
+        default: be_.for_each_scratch(n, DfoMaxFn<4>{d, list, base, all}); break;
+      }
+      launches(1);
+      if (base && all) {
+        counters.root_finds += (long long)n;
+        counters.root_finds_executed += (long long)n;
+      }
+    }
   }
   // ---- general-shape path (tg_generic.cuh): PolynomialOptimization<N> for N = 6, 8, 10, 12 on 4 (zero-padded) dimensions ----------
   // setupFromVertices + solveLinear + getSegments + computeCost for B problems.  The vertex bookkeeping (first free unknown per
