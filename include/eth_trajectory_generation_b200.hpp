@@ -518,6 +518,7 @@ class PolynomialOptimization {
     vertices_ = vertices;
     segment_times_ = segment_times;
     solved_ = false;
+    free_state_ = kFreeNone;
     return b200::pack_vertices(vertices_, &mask_, &vals_, N / 2, (int)dimension_);
   }
   // the node's shape: tuned kernels
@@ -532,6 +533,7 @@ class PolynomialOptimization {
     }
     segment_times_ = segment_times;
     solved_ = false;
+    free_state_ = kFreeNone;
   }
   // lin_impl.h:340-373 (+ updateSegmentsFromCompactConstraints 263-282)
   bool solveLinear() {
@@ -549,7 +551,81 @@ class PolynomialOptimization {
       return false;
     }
     solved_ = true;
+    free_state_ = kFreeFromSolve;
     return true;
+  }
+  // ---- free and fixed constraints (lin_impl.h:183-257, 513-522) ----------------------------------------------------------
+  // Both are dimension-major: getDimension() vectors; within a vector vertex-major with the derivative ascending.
+  size_t getNumberFreeConstraints() const { return (size_t)countFree(); }
+  size_t getNumberFixedConstraints() const { return mask_.size() * (size_t)(N / 2) - (size_t)countFree(); }
+  size_t getNumberAllConstraints() const { return segment_times_.size() * (size_t)N; }  // N/2 start and N/2 end rows per segment
+  void getFixedConstraints(std::vector<Vector>* fixed_constraints) const {
+    if (!fixed_constraints) return;
+    constexpr int H = N / 2;
+    const size_t dims = dimension_;
+    fixed_constraints->assign(dims, b200::make_vector(getNumberFixedConstraints(), 0.0));
+    size_t i = 0;
+    for (size_t v = 0; v < mask_.size(); ++v)
+      for (int k = 0; k < H; ++k) {
+        if (!((mask_[v] >> k) & 1u)) continue;
+        for (size_t d = 0; d < dims; ++d) (*fixed_constraints)[d][i] = vals_[(v * H + k) * dims + d];
+        ++i;
+      }
+  }
+  // After solveLinear(): the free derivatives d_p the solve found (fetched from the device on the first request at the current times
+  // and kept).  After setFreeConstraints(): what was set.  Otherwise (no solve yet, or updateSegmentTimes / a nonlinear optimisation
+  // since) there is no linear solution to read: a message, and zero vectors.
+  void getFreeConstraints(std::vector<Vector>* free_constraints) const {
+    if (!free_constraints) return;
+    const size_t dims = dimension_, nf = getNumberFreeConstraints();
+    if (free_state_ == kFreeFromSolve) {
+      b200::Context& c = b200::Context::instance();
+      const int vtx_off[2] = {0, (int)vertices_.size()};
+      free_.assign(std::max<size_t>(dims * nf, 1), 0.0);
+      c.check(tg_solve_linear_free_batch_nd(c.get(), N, (int)dims, 1, vtx_off, mask_.data(), vals_.data(), segment_times_.data(),
+                                            derivative_to_optimize_, nullptr, nullptr, free_.data()),
+              "tg_solve_linear_free_batch_nd");
+      free_state_ = kFreeKnown;
+    }
+    if (free_state_ == kFreeNone) {
+      std::printf("[PolynomialOptimization]: getFreeConstraints: no linear solution (call solveLinear or setFreeConstraints first)\n");
+      free_constraints->assign(dims, b200::make_vector(nf, 0.0));
+      return;
+    }
+    free_constraints->assign(dims, b200::make_vector(nf, 0.0));
+    for (size_t d = 0; d < dims; ++d)
+      for (size_t i = 0; i < nf; ++i) (*free_constraints)[d][i] = free_[d * nf + i];
+  }
+  // lin_impl.h:519-522: the segments (and the cost) become A^-1 [fixed ; free] at the current times.  The wrong number of vectors or
+  // of entries is refused with a message and leaves the state as it was (the reference's CHECK prints and goes on with the sizes given).
+  void setFreeConstraints(const std::vector<Vector>& free_constraints) {
+    const size_t dims = dimension_, nf = getNumberFreeConstraints();
+    if (vertices_.empty()) {
+      std::printf("[PolynomialOptimization]: setFreeConstraints before setupFromVertices\n");
+      return;
+    }
+    bool ok = free_constraints.size() == dims;
+    for (size_t d = 0; ok && d < dims; ++d) ok = (size_t)free_constraints[d].size() == nf;
+    if (!ok) {
+      std::printf("[PolynomialOptimization]: setFreeConstraints needs %zu vectors of %zu free derivatives\n", dims, nf);
+      return;
+    }
+    std::vector<double> flat(std::max<size_t>(dims * nf, 1), 0.0);
+    for (size_t d = 0; d < dims; ++d)
+      for (size_t i = 0; i < nf; ++i) flat[d * nf + i] = free_constraints[d][i];
+    const int V = (int)vertices_.size();
+    const int vtx_off[2] = {0, V};
+    std::vector<double> coef((size_t)(V - 1) * dims * N);
+    double cost = 0.0;
+    b200::Context& c = b200::Context::instance();
+    c.check(tg_set_free_constraints_batch_nd(c.get(), N, (int)dims, 1, vtx_off, mask_.data(), vals_.data(), segment_times_.data(),
+                                             derivative_to_optimize_, flat.data(), coef.data(), &cost),
+            "tg_set_free_constraints_batch_nd");
+    coef_ = std::move(coef);
+    cost_ = cost;
+    free_ = std::move(flat);
+    solved_ = true;
+    free_state_ = kFreeKnown;
   }
   double computeCost() const { return cost_; }  // lin_impl.h:127-141
   void getSegmentTimes(std::vector<double>* segment_times) const {
@@ -604,9 +680,20 @@ class PolynomialOptimization {
     coef_ = coef;
     cost_ = cost;
     solved_ = true;
+    free_state_ = kFreeNone;
   }
 
  private:
+  int countFree() const {
+    int n = 0;
+    for (uint8_t m : mask_)
+      for (int k = 0; k < N / 2; ++k) n += ((m >> k) & 1u) ? 0 : 1;
+    return n;
+  }
+  // where getFreeConstraints reads from: nothing, the solve of solveLinear (not fetched yet), or free_
+  enum FreeState { kFreeNone, kFreeFromSolve, kFreeKnown };
+  mutable FreeState free_state_ = kFreeNone;
+  mutable std::vector<double> free_;  // [D][n_free]
   size_t dimension_;
   int derivative_to_optimize_;
   Vertex::Vector vertices_;

@@ -177,6 +177,24 @@ int tg_evaluate_batch_nd(tg_ctx* ctx, int N, int D, int S, const double* coef, c
                          double* out, uint8_t* ok);
 int tg_sample_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times, double dt, int* counts,
                        double* samples, double* full);
+/* Free and fixed constraints of PolynomialOptimization<N> (lin_impl.h:183-257, 513-522) on the same shapes, inputs as in
+ *   tg_solve_linear_batch_nd.  The free derivatives d_p of a problem are dimension-major: D vectors of n_free entries, and within a
+ *   dimension vertex-major with the derivative ascending; n_free = the clear mask bits below N/2 over the problem's vertices,
+ *   n_fixed = (S+1)*N/2 - n_free.  free[] holds the problems' D*n_free blocks one after the other, in problem order.
+ * tg_solve_linear_free_batch_nd = setupFromVertices + solveLinear + getFreeConstraints + getSegments + computeCost
+ *   (lin_impl.h:340-373, 513-516, 263-282, 127-141): coef[totS][D][N] and cost[B] carry tg_solve_linear_batch_nd's bits, free the
+ *   d_p the solve found.  Any output may be NULL.
+ * tg_set_free_constraints_batch_nd = setFreeConstraints + getSegments + computeCost (lin_impl.h:519-522 -> 263-282, 127-141): the
+ *   coefficients A^-1 [fixed ; free] of every (segment, dimension) from the given free[] and the cost 1/2 sum c^T Q c in (segment,
+ *   dimension) order, with no solve; K candidate free vectors of one problem are K problems.  Non-finite free values are not
+ *   refused and propagate.  coef and cost may be NULL.  Setting the free derivatives a solve returned reproduces its coef and cost
+ *   bit for bit.
+ *   Both refuse with TG_ERR_INVALID, writing no output, N outside {6, 8, 10, 12}, D outside 1..4, r outside 0 .. N/2-1, B < 1
+ *   and a problem with fewer than two vertices. */
+int tg_solve_linear_free_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval,
+                                  const double* times, int r, double* coef, double* cost, double* free);
+int tg_set_free_constraints_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval,
+                                     const double* times, int r, const double* free, double* coef, double* cost);
 /* The nonlinear half on the same shapes, with the contracts of the N = 10 entry points above (coef[totS][D][N] everywhere):
  *   tg_extrema_batch_nd        = tg_extrema_batch: Trajectory::computeMaxDerivatives{Horizontal,Vertical,Heading}
  *                                (eth/trajectory.cpp:422-565) -> maxima[totS][9]; a missing dimension has zero maxima.

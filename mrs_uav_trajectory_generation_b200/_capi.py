@@ -139,6 +139,8 @@ class Library:
         L.tg_evaluate_batch.argtypes = [C.c_void_p, C.c_int, _dp, _dp, C.c_int, _dp, C.c_int, _dp, _u8p]
         L.tg_extrema_batch.argtypes = [C.c_void_p, C.c_int, _dp, _dp, _dp]
         L.tg_solve_linear_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.c_int, _dp, _dp]
+        L.tg_solve_linear_free_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.c_int, _dp, _dp, _dp]
+        L.tg_set_free_constraints_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.c_int, _dp, _dp, _dp]
         L.tg_evaluate_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, C.c_int, _dp, _u8p]
         L.tg_sample_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_double, _ip, _dp, _dp]
         L.tg_extrema_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp]
@@ -476,6 +478,53 @@ class Context:
         cost = np.empty(B)
         self._check(self.L.lib.tg_solve_linear_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times),
                                                         int(r), _p(coef), _p(cost)))
+        return coef, cost
+
+    @staticmethod
+    def free_counts(n_coef, vtx_off, vmask):
+        """n_free of every problem: the clear mask bits below n_coef/2 over its vertices."""
+        bits = (np.asarray(vmask, dtype=np.uint8)[:, None] >> np.arange(n_coef // 2, dtype=np.uint8)) & 1
+        cs = np.concatenate([[0], np.cumsum(n_coef // 2 - bits.sum(axis=1, dtype=np.int64))])
+        off = np.asarray(vtx_off, dtype=np.int64)
+        return cs[off[1:]] - cs[off[:-1]]
+
+    def solve_linear_free_batch_nd(self, n_coef, dim, vtx_off, vmask, vval, times, r=2):
+        """solveLinear + getFreeConstraints + getSegments + computeCost: (coef [totS][dim][n_coef], cost [B], free), free = one
+        [dim][n_free] array per problem (the d_p of lin_impl.h:340-373, dimension-major)."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        vmask = np.ascontiguousarray(vmask, dtype=np.uint8)
+        vval = np.ascontiguousarray(vval, dtype=np.float64)
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        B = len(vtx_off) - 1
+        totS = int(vtx_off[-1]) - B
+        assert vval.size == int(vtx_off[-1]) * (n_coef // 2) * dim and times.size == totS
+        nf = self.free_counts(n_coef, vtx_off, vmask)
+        coef = np.empty((totS, dim, n_coef))
+        cost = np.empty(B)
+        free = np.empty(max(int(nf.sum()) * dim, 1))
+        self._check(self.L.lib.tg_solve_linear_free_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times),
+                                                             int(r), _p(coef), _p(cost), _p(free)))
+        off = np.concatenate([[0], np.cumsum(nf * dim)])
+        return coef, cost, [free[off[p]:off[p + 1]].reshape(dim, nf[p]) for p in range(B)]
+
+    def set_free_constraints_batch_nd(self, n_coef, dim, vtx_off, vmask, vval, times, free, r=2):
+        """setFreeConstraints + getSegments + computeCost: free = one [dim][n_free] array per problem -> (coef, cost)."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        vmask = np.ascontiguousarray(vmask, dtype=np.uint8)
+        vval = np.ascontiguousarray(vval, dtype=np.float64)
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        B = len(vtx_off) - 1
+        totS = int(vtx_off[-1]) - B
+        assert vval.size == int(vtx_off[-1]) * (n_coef // 2) * dim and times.size == totS and len(free) == B
+        nf = self.free_counts(n_coef, vtx_off, vmask)
+        for p in range(B):
+            if np.shape(free[p]) != (dim, nf[p]):
+                raise ValueError(f"problem {p}: the free constraints are [{dim}][{nf[p]}], got {np.shape(free[p])}")
+        flat = np.ascontiguousarray(np.concatenate([np.asarray(f, dtype=np.float64).reshape(-1) for f in free] + [np.zeros(1)]))
+        coef = np.empty((totS, dim, n_coef))
+        cost = np.empty(B)
+        self._check(self.L.lib.tg_set_free_constraints_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval),
+                                                                _p(times), int(r), _p(flat), _p(coef), _p(cost)))
         return coef, cost
 
     def evaluate_nd(self, n_coef, dim, coef, times, t, derivative=0):

@@ -186,9 +186,16 @@ class PolynomialOptimization:
         self._lists = None
         self.derivative_to_optimize = derivative_order.INVALID
         self.coef = self.cost = None
+        self._free = None  # per problem [dimension][n_free] once known; "solve" = the solve's, not fetched yet
 
     def _c(self):
         return self._ctx or default_context()
+
+    def _packed(self):
+        return pack_vertices(self._lists, self.N // 2, self.dimension)
+
+    def _out(self, per_problem):
+        return per_problem[0] if self._single else per_problem
 
     def setupFromVertices(self, vertices, times, derivative_to_optimize):  # lin_impl.h:61-106
         if not (0 <= derivative_to_optimize <= self.N // 2 - 1):  # kHighestDerivativeToOptimize (lin.h:55, lin_impl.h:63-66)
@@ -203,13 +210,16 @@ class PolynomialOptimization:
                 return False
         self.derivative_to_optimize = derivative_to_optimize
         self._single = single
+        self._free = None
         return True
 
     def updateSegmentTimes(self, times):  # lin_impl.h:288-304
         self._times = [np.asarray(times, dtype=np.float64)] if self._single else [np.asarray(t, dtype=np.float64) for t in times]
+        self._free = None
 
     def solveLinear(self):  # lin_impl.h:340-373
-        vtx_off, masks, vals = pack_vertices(self._lists, self.N // 2, self.dimension)
+        vtx_off, masks, vals = self._packed()
+        self._free = "solve"
         self._seg_off = vtx_off - np.arange(len(vtx_off), dtype=np.int32)
         if self.N == N and self.dimension == D and self.derivative_to_optimize >= 2:
             self.coef, self.cost = self._c().solve_linear_batch(vtx_off, masks, vals, np.concatenate(self._times), self.derivative_to_optimize)
@@ -231,6 +241,61 @@ class PolynomialOptimization:
     def getSegments(self, index=0):  # lin.h:177
         t = self.getTrajectory(index)
         return t.coef, t.times
+
+    # ---- free and fixed constraints (lin_impl.h:183-257, 513-522): lists of `dimension` vectors, each vertex-major with the derivative
+    # ascending; for a batch, one such list per problem
+    def _counts(self):
+        vtx_off, masks, _ = self._packed()
+        nf = Context.free_counts(self.N, vtx_off, masks)
+        nv = np.diff(vtx_off)
+        return nf, nv * (self.N // 2) - nf, (nv - 1) * self.N
+
+    def getNumberFreeConstraints(self):
+        return self._out([int(x) for x in self._counts()[0]])
+
+    def getNumberFixedConstraints(self):
+        return self._out([int(x) for x in self._counts()[1]])
+
+    def getNumberAllConstraints(self):  # N/2 start and N/2 end rows per segment
+        return self._out([int(x) for x in self._counts()[2]])
+
+    def getFixedConstraints(self):
+        vtx_off, masks, vals = self._packed()
+        bits = ((masks[:, None] >> np.arange(self.N // 2)) & 1).astype(bool)  # [V][N/2], vertex-major then derivative
+        return self._out([[vals[vtx_off[p]:vtx_off[p + 1]][bits[vtx_off[p]:vtx_off[p + 1]], d].copy() for d in range(self.dimension)]
+                          for p in range(len(vtx_off) - 1)])
+
+    def getFreeConstraints(self):
+        """After solveLinear: the free derivatives d_p of the solve (fetched on the first request).  After setFreeConstraints: what was
+        set.  Otherwise (no solve yet, or updateSegmentTimes since): a message and zero vectors."""
+        if isinstance(self._free, str):
+            vtx_off, masks, vals = self._packed()
+            _, _, free = self._c().solve_linear_free_batch_nd(self.N, self.dimension, vtx_off, masks, vals, np.concatenate(self._times),
+                                                              self.derivative_to_optimize)
+            self._free = free
+        if self._free is None:
+            print("getFreeConstraints: no linear solution (call solveLinear or setFreeConstraints first)")
+            return self._out([[np.zeros(n) for _ in range(self.dimension)] for n in self._counts()[0]])
+        return self._out([[row.copy() for row in f] for f in self._free])
+
+    def setFreeConstraints(self, free_constraints):
+        """lin_impl.h:519-522: the segments and the cost become A^-1 [fixed ; free] at the current times.  The wrong number of vectors
+        or of entries is refused with a message (returns False) and changes nothing."""
+        per_problem = [free_constraints] if self._single else list(free_constraints)
+        nf = self._counts()[0]
+        try:
+            free = [np.array([np.asarray(v, dtype=np.float64).reshape(-1) for v in f], dtype=np.float64) for f in per_problem]
+        except ValueError:
+            free = None
+        if free is None or len(free) != len(nf) or any(f.shape != (self.dimension, n) for f, n in zip(free, nf)):
+            print("setFreeConstraints: needs %d vectors of n_free entries per problem (n_free = %s)" % (self.dimension, list(nf)))
+            return False
+        vtx_off, masks, vals = self._packed()
+        self.coef, self.cost = self._c().set_free_constraints_batch_nd(self.N, self.dimension, vtx_off, masks, vals, np.concatenate(self._times),
+                                                                       free, self.derivative_to_optimize)
+        self._seg_off = vtx_off - np.arange(len(vtx_off), dtype=np.int32)
+        self._free = free
+        return True
 
 
 class NonlinearOptimizationParameters:

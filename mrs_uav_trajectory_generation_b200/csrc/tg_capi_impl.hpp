@@ -323,6 +323,38 @@ inline bool tg_segments_ok(int B, const int* seg_off) {
     if (seg_off[p + 1] - seg_off[p] < 1) return false;
   return true;
 }
+// n_free of every problem: the clear mask bits below N/2 over its vertices
+inline std::vector<int> tg_free_counts(int N, int B, const int* vtx_off, const uint8_t* vmask) {
+  std::vector<int> nf(B, 0);
+  for (int p = 0; p < B; ++p)
+    for (int v = vtx_off[p]; v < vtx_off[p + 1]; ++v)
+      for (int k = 0; k < N / 2; ++k) nf[p] += ((vmask[v] >> k) & 1u) ? 0 : 1;
+  return nf;
+}
+// free derivatives, D x n_free per problem <-> 4 x n_free per problem (dimension-major; missing dimensions zero)
+inline size_t tg_free_total(const std::vector<int>& nf, int D) {
+  size_t tot = 0;
+  for (int n : nf) tot += (size_t)D * n;
+  return tot;
+}
+inline std::vector<double> tg_pad_free(const double* free, const std::vector<int>& nf, int D) {
+  std::vector<double> out(std::max<size_t>(tg_free_total(nf, TG_D), 1), 0.0);
+  size_t i = 0, o = 0;
+  for (int n : nf) {
+    std::memcpy(out.data() + o, free + i, sizeof(double) * (size_t)D * n);
+    i += (size_t)D * n;
+    o += (size_t)TG_D * n;
+  }
+  return out;
+}
+inline void tg_strip_free(const double* f4, const std::vector<int>& nf, int D, double* free) {
+  size_t i = 0, o = 0;
+  for (int n : nf) {
+    std::memcpy(free + o, f4 + i, sizeof(double) * (size_t)D * n);
+    i += (size_t)TG_D * n;
+    o += (size_t)D * n;
+  }
+}
 template <class F>
 inline void tg_dispatch_n(int N, F&& f) {
   switch (N) {
@@ -351,6 +383,51 @@ int tg_solve_linear_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_of
     if (coef)
       for (size_t s = 0; s < totS; ++s)
         for (int d = 0; d < D; ++d) std::memcpy(coef + (s * D + d) * N, &c4[(s * TG_D + d) * N], sizeof(double) * N);
+    return TG_OK;
+  });
+}
+
+int tg_solve_linear_free_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval,
+                                  const double* times, int r, double* coef, double* cost, double* free) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !vtx_off || !vmask || !vval || !times || r < 0 || r > N / 2 - 1) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) { ctx->err = "every problem needs at least two vertices"; return TG_ERR_INVALID; }
+    const size_t totV = (size_t)vtx_off[B], totS = totV - (size_t)B;
+    const std::vector<int> nf = tg_free_counts(N, B, vtx_off, vmask);
+    const std::vector<double> vv = tg_pad_dims(vval, totV * (size_t)(N / 2), D);
+    std::vector<double> c4(coef ? totS * TG_D * N : 0), f4(free ? std::max<size_t>(tg_free_total(nf, TG_D), 1) : 0);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto n) {
+      ctx->pipe.template linear_batch_n<decltype(n)::value>(B, vtx_off, vmask, vv.data(), times, r, coef ? c4.data() : nullptr, cost,
+                                                            free ? f4.data() : nullptr);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (coef) tg_strip_coef(c4.data(), totS, N, D, coef);
+    if (free) tg_strip_free(f4.data(), nf, D, free);
+    return TG_OK;
+  });
+}
+
+int tg_set_free_constraints_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval,
+                                     const double* times, int r, const double* free, double* coef, double* cost) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !vtx_off || !vmask || !vval || !times || !free || r < 0 || r > N / 2 - 1) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) { ctx->err = "every problem needs at least two vertices"; return TG_ERR_INVALID; }
+    const size_t totV = (size_t)vtx_off[B], totS = totV - (size_t)B;
+    const std::vector<int> nf = tg_free_counts(N, B, vtx_off, vmask);
+    const std::vector<double> vv = tg_pad_dims(vval, totV * (size_t)(N / 2), D);
+    const std::vector<double> f4 = tg_pad_free(free, nf, D);
+    std::vector<double> c4(coef ? totS * TG_D * N : 0);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto n) {
+      ctx->pipe.template set_free_batch_n<decltype(n)::value>(B, vtx_off, vmask, vv.data(), times, r, f4.data(), coef ? c4.data() : nullptr, cost);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (coef) tg_strip_coef(c4.data(), totS, N, D, coef);
     return TG_OK;
   });
 }

@@ -11,6 +11,9 @@
 //   record_hrow<N>   one thread per (segment, row a)   row a of H = (A^-T Q) A^-1 (lin_impl.h:320)
 //   solve_warp<N>    one warp per problem              reduced banded system, LU without pivoting, coefficients, cost
 //                                                      (lin_impl.h:310-373, 263-282, 127-141) -- the phases of tg_solve.cuh
+//   SolveFreeFn<N>                                     solve_warp<N> that also writes the free derivatives d_p (getFreeConstraints)
+//   SetFreeFn<N>, SetFreeCostFn                        setFreeConstraints: coefficients and cost from given d_p, one thread per
+//                                                      (segment, dimension), with solve_warp's coef_from_endpoints / cost_partial
 //   poly_eval_n<N>, sample_eval_n<N>                   Trajectory::evaluate / sampleWholeTrajectory (eth/trajectory.cpp:55-151,
 //                                                      eth/trajectory_sampling.cpp:49-124)
 //   ExtremaFn<N, Q>, MaxMagnitudeSegFn<N, K>           per-segment maxima (tg_poly.cuh over N), one thread per segment
@@ -171,6 +174,7 @@ struct Problem {
   double* coef;          // [S][4][N], or null
   double* cost;          // scalar
   double* ws;            // solve_ws_doubles<N>(S, np, hbw) doubles
+  double* dp = nullptr;  // [4][np]: the free derivatives d_p, dimension-major (getFreeConstraints, lin_impl.h:513-516), or null
 };
 // the record segment s is solved with: variant 0 for every segment of the point itself; for the point perturbed along segment
 // n-1, variant 1 (T + 0.1) on that segment and variant 2 (T - 0.1/(S-1)) on the others (nl_impl.h:282-323)
@@ -184,6 +188,36 @@ template <int N>
 TG_HD size_t ws_doubles(int S, int np, int hbw) {
   const size_t V = (size_t)S + 1;
   return (size_t)np * row_stride(hbw) + 4 * (size_t)np + (size_t)S * TG_D * N + (size_t)S * TG_D + (V * (N / 2) + 1) / 2 + 2;
+}
+
+// coefficient a of one (segment, dimension) = row a of A^-1 against the N end-point derivatives (derivatives 0 .. N/2-1 at
+// vertex s, then at vertex s+1; nd(k) returns derivative k), a dense sum over ascending k (lin_impl.h:271-280)
+template <int N, class Endpoint>
+TG_HD double coef_from_endpoints(const double* Ai_row, const Endpoint& nd) {
+  double c = 0.0;
+  for (int k = 0; k < N; ++k) {
+    const double e = nd(k);  // before the load of A^-1 and without __restrict__: solve_warp's phase 4 compiles as it did inline
+    const double t = Ai_row[k] * e;
+    c = (k == 0) ? t : c + t;
+  }
+  return c;
+}
+// (c^T Q) c of one (segment, dimension), dense (lin_impl.h:135-137)
+template <int N>
+TG_HD double cost_partial(const double* __restrict__ Q, const double* __restrict__ c) {
+  double partial = 0.0;
+  for (int b = 0; b < N; ++b) {
+    double sum = c[0] * Q[0 * N + b];
+    for (int k = 1; k < N; ++k) sum = sum + c[k] * Q[k * N + b];
+    partial = (b == 0) ? sum * c[b] : partial + sum * c[b];
+  }
+  return partial;
+}
+// rank of derivative a among the free (clear) bits of a vertex mask: the slot's offset from the vertex's first free unknown
+TG_HD int free_rank(uint32_t mask, int a) {
+  int rank = 0;
+  for (int q = 0; q < a; ++q) rank += ((mask >> q) & 1u) ? 0 : 1;
+  return rank;
 }
 
 template <int N>
@@ -201,9 +235,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
     for (int it = lane; it < V * H; it += 32) {
       const int v = it / H, a = it - v * H;
       const uint32_t m = P.vmask[v];
-      int rank = 0;
-      for (int q = 0; q < a; ++q) rank += ((m >> q) & 1u) ? 0 : 1;
-      slot[it] = ((m >> a) & 1u) ? -1 : P.vfree[v] + rank;
+      slot[it] = ((m >> a) & 1u) ? -1 : P.vfree[v] + free_rank(m, a);
     }
     for (int e = lane; e < np * W; e += 32) rows[e] = 0.0;
   }
@@ -275,6 +307,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
         const double* rj = rows + (size_t)j * W;
         const double xj = rj[RB + d] * rj[RB + TG_D];
         if (ri == 0) xs[j * 4 + d] = xj;
+        if (ri == 0 && P.dp) P.dp[(size_t)d * np + j] = xj;
         const int i0 = imax(0, j - hbw);
         for (int i = j - 1 - ri; i >= i0; i -= 8) {
           double* rw = rows + (size_t)i * W;
@@ -288,13 +321,10 @@ TG_HD void solve_warp(const Problem& P, int lane) {
     for (int it = lane; it < S * TG_D * N; it += 32) {
       const int s = it / (TG_D * N), rem = it - s * (TG_D * N), d = rem / N, a = rem - d * N;
       const double* Ai = problem_rec<N>(P, s) + Rec<N>::kAinv + a * N;
-      double c = 0.0;
-      for (int k = 0; k < N; ++k) {
+      const double c = coef_from_endpoints<N>(Ai, [&](int k) {
         const int j = slot[s * H + k];  // the slots of vertex s and of vertex s+1 are contiguous in the table
-        const double nd = (j >= 0) ? xs[j * 4 + d] : P.vval[((size_t)s * H + k) * TG_D + d];
-        const double t = Ai[k] * nd;
-        c = (k == 0) ? t : c + t;
-      }
+        return (j >= 0) ? xs[j * 4 + d] : P.vval[((size_t)s * H + k) * TG_D + d];
+      });
       cf[it] = c;
       if (P.coef) P.coef[it] = c;
     }
@@ -303,15 +333,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
   TG_PHASE(lane) {
     for (int it = lane; it < S * TG_D; it += 32) {
       const int s = it / TG_D;
-      const double* Q = problem_rec<N>(P, s) + Rec<N>::kQ;
-      const double* c = cf + (size_t)it * N;
-      double partial = 0.0;
-      for (int b = 0; b < N; ++b) {
-        double sum = c[0] * Q[0 * N + b];
-        for (int k = 1; k < N; ++k) sum = sum + c[k] * Q[k * N + b];
-        partial = (b == 0) ? sum * c[b] : partial + sum * c[b];
-      }
-      part[it] = partial;
+      part[it] = cost_partial<N>(problem_rec<N>(P, s) + Rec<N>::kQ, cf + (size_t)it * N);
     }
   }
   // ---- phase 6: total in (segment, dimension) order (lin_impl.h:131-140)
@@ -394,7 +416,8 @@ struct SolveFn {  // one warp per problem
   double* ws;
   double* coef;             // [totS][4][N]
   double* cost;             // [B]
-  TG_HD void operator()(size_t p, int lane) const {
+  TG_HD void operator()(size_t p, int lane) const { solve_warp<N>(problem(p), lane); }
+  TG_HD Problem problem(size_t p) const {
     const int v0 = vtx_off[p], s0 = v0 - (int)p;
     Problem P;
     P.S = vtx_off[p + 1] - v0 - 1;
@@ -410,7 +433,65 @@ struct SolveFn {  // one warp per problem
     P.coef = coef + (size_t)s0 * TG_D * N;
     P.cost = cost + p;
     P.ws = ws + ws_off[p];
+    return P;
+  }
+};
+// SolveFn that also writes every problem's free derivatives d_p (getFreeConstraints after solveLinear, lin_impl.h:340-373, 513-516)
+template <int N>
+struct SolveFreeFn {
+  SolveFn<N> solve;
+  const long long* dp_off;  // [B]: offset of problem p's [4][np] block in dp
+  double* dp;
+  TG_HD void operator()(size_t p, int lane) const {
+    Problem P = solve.problem(p);
+    P.dp = dp + dp_off[p];
     solve_warp<N>(P, lane);
+  }
+};
+// setFreeConstraints + getSegments (lin_impl.h:519-522 -> updateSegmentsFromCompactConstraints 263-282): one thread per (segment,
+// dimension) computes the coefficients from the fixed values and the caller's free vector, with the functions phases 4 and 5 of
+// solve_warp use, and the cost partial; SetFreeCostFn then adds the partials as phase 6 does.  Reads A^-1 and Q of the record heads
+// only (RecordHeadFn): no row of H is needed without a solve.
+template <int N>
+struct SetFreeFn {
+  const int* prob_of_seg;   // [totS]
+  const uint8_t* vmask;     // [totV]
+  const int* vfree;         // [totV + B], as in SolveFn
+  const double* vval;       // [totV][N/2][4]
+  const long long* dp_off;  // [B]
+  const int* np;            // [B]
+  const double* dp;         // problem p: [4][np[p]] at dp_off[p]
+  const double* recs;       // [totS][Rec<N>::kSize]
+  double* coef;             // [totS][4][N]
+  double* part;             // [totS][4]
+  TG_HD void operator()(size_t it) const {
+    constexpr int H = N / 2;
+    const size_t gs = it / TG_D;
+    const int d = (int)(it - gs * TG_D), p = prob_of_seg[gs];
+    const int v = (int)gs + p;  // first vertex of the segment: segment s of problem p joins vertices vtx_off[p] + s and + s + 1
+    const int* vf = vfree + v + p;  // problem p's table starts at vtx_off[p] + p
+    const double* x = dp + dp_off[p] + (size_t)d * np[p];
+    const double* rec = recs + gs * Rec<N>::kSize;
+    double c[N];
+    for (int a = 0; a < N; ++a)
+      c[a] = coef_from_endpoints<N>(rec + Rec<N>::kAinv + a * N, [&](int k) {
+        const int w = k / H, b = k - w * H;
+        const uint32_t m = vmask[v + w];
+        return ((m >> b) & 1u) ? vval[((size_t)(v + w) * H + b) * TG_D + d] : x[vf[w] + free_rank(m, b)];
+      });
+    for (int a = 0; a < N; ++a) coef[it * N + a] = c[a];
+    part[it] = cost_partial<N>(rec + Rec<N>::kQ, c);
+  }
+};
+struct SetFreeCostFn {  // one thread per problem: the total in (segment, dimension) order (lin_impl.h:131-140)
+  const int* vtx_off;
+  const double* part;
+  double* cost;
+  TG_HD void operator()(size_t p) const {
+    const int s0 = vtx_off[p] - (int)p, S = vtx_off[p + 1] - vtx_off[p] - 1;
+    double total = 0.0;
+    for (int it = 0; it < S * TG_D; ++it) total += part[(size_t)s0 * TG_D + it];
+    cost[p] = 0.5 * total;
   }
 };
 // Trajectory::evaluate(t, derivative) (eth/trajectory.cpp:55-87): one thread per query time

@@ -1554,8 +1554,16 @@ class Pipeline {
     }
     return g;
   }
+  // offset of every problem's [4][n_free] block of free derivatives (dimension-major, problems in order); the total at [B]
+  static std::vector<long long> gen_dp_offsets(const std::vector<int>& np) {
+    std::vector<long long> off(np.size() + 1, 0);
+    for (size_t p = 0; p < np.size(); ++p) off[p + 1] = off[p] + (long long)TG_D * np[p];
+    return off;
+  }
+  // dp (optional): the free derivatives d_p of every problem after the solve, [4][n_free] per problem (gen_dp_offsets)
   template <int N>
-  bool linear_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, const double* times, int r, double* coef, double* cost) {
+  bool linear_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, const double* times, int r, double* coef, double* cost,
+                      double* dp = nullptr) {
     constexpr int H = N / 2;
     scratch_.reset();
     const int totV = vtx_off[B], totS = totV - B;
@@ -1591,9 +1599,67 @@ class Pipeline {
     be_.h2d(d_ws_off, ws_off.data(), sizeof(long long) * B);
     be_.for_each((size_t)totS, gen::RecordHeadFn<N>{r, d_times, d_recs});
     be_.for_each((size_t)totS * N, gen::RecordHrowFn<N>{d_recs});
-    be_.for_each_warp((size_t)B, gen::SolveFn<N>{r, d_vtx_off, d_vmask, d_vfree, d_vval, d_np, d_hbw, d_recs, d_ws_off, d_ws, d_coef, d_cost});
+    const gen::SolveFn<N> solve{r, d_vtx_off, d_vmask, d_vfree, d_vval, d_np, d_hbw, d_recs, d_ws_off, d_ws, d_coef, d_cost};
+    std::vector<long long> dp_off;
+    double* d_dp = nullptr;
+    if (dp) {
+      dp_off = gen_dp_offsets(np);
+      long long* d_dp_off = scratch_.template alloc<long long>(B);
+      d_dp = scratch_.template alloc<double>((size_t)std::max<long long>(dp_off[B], 1));
+      be_.h2d(d_dp_off, dp_off.data(), sizeof(long long) * B);
+      be_.for_each_warp((size_t)B, gen::SolveFreeFn<N>{solve, d_dp_off, d_dp});
+    } else {
+      be_.for_each_warp((size_t)B, solve);
+    }
     launches(3);
     counters.solves += B;
+    counters.segment_setups += totS;
+    if (coef) be_.d2h(coef, d_coef, sizeof(double) * (size_t)totS * TG_D * N);
+    if (cost) be_.d2h(cost, d_cost, sizeof(double) * B);
+    if (dp) be_.d2h(dp, d_dp, sizeof(double) * (size_t)dp_off[B]);
+    return true;
+  }
+  // setFreeConstraints + getSegments + computeCost (lin_impl.h:519-522, 263-282, 127-141) for B problems: the coefficients from the
+  // fixed values and the given free derivatives dp ([4][n_free] per problem, gen_dp_offsets), without a solve.
+  template <int N>
+  bool set_free_batch_n(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, const double* times, int r, const double* dp,
+                        double* coef, double* cost) {
+    constexpr int H = N / 2;
+    scratch_.reset();
+    const int totV = vtx_off[B], totS = totV - B;
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) return false;
+    const GenVertices gv = gen_vertices<N>(B, vtx_off, vmask);
+    const std::vector<long long> dp_off = gen_dp_offsets(gv.np);
+    std::vector<int> prob_of_seg(totS);
+    for (int p = 0; p < B; ++p)
+      for (int s = vtx_off[p] - p; s < vtx_off[p + 1] - p - 1; ++s) prob_of_seg[s] = p;
+    int* d_vtx_off = scratch_.template alloc<int>((size_t)B + 1);
+    int* d_prob_of_seg = scratch_.template alloc<int>(totS);
+    uint8_t* d_vmask = scratch_.template alloc<uint8_t>(totV);
+    int* d_vfree = scratch_.template alloc<int>(gv.vfree.size());
+    double* d_vval = scratch_.template alloc<double>((size_t)totV * H * TG_D);
+    long long* d_dp_off = scratch_.template alloc<long long>(B);
+    int* d_np = scratch_.template alloc<int>(B);
+    double* d_dp = scratch_.template alloc<double>((size_t)std::max<long long>(dp_off[B], 1));
+    double* d_times = scratch_.template alloc<double>(totS);
+    double* d_recs = scratch_.template alloc<double>((size_t)totS * gen::Rec<N>::kSize);
+    double* d_coef = scratch_.template alloc<double>((size_t)totS * TG_D * N);
+    double* d_part = scratch_.template alloc<double>((size_t)totS * TG_D);
+    double* d_cost = scratch_.template alloc<double>(B);
+    be_.h2d(d_vtx_off, vtx_off, sizeof(int) * ((size_t)B + 1));
+    be_.h2d(d_prob_of_seg, prob_of_seg.data(), sizeof(int) * (size_t)totS);
+    be_.h2d(d_vmask, vmask, totV);
+    be_.h2d(d_vfree, gv.vfree.data(), sizeof(int) * gv.vfree.size());
+    be_.h2d(d_vval, vval, sizeof(double) * (size_t)totV * H * TG_D);
+    be_.h2d(d_dp_off, dp_off.data(), sizeof(long long) * B);
+    be_.h2d(d_np, gv.np.data(), sizeof(int) * B);
+    be_.h2d(d_dp, dp, sizeof(double) * (size_t)dp_off[B]);
+    be_.h2d(d_times, times, sizeof(double) * totS);
+    be_.for_each((size_t)totS, gen::RecordHeadFn<N>{r, d_times, d_recs});
+    be_.for_each((size_t)totS * TG_D, gen::SetFreeFn<N>{d_prob_of_seg, d_vmask, d_vfree, d_vval, d_dp_off, d_np, d_dp, d_recs, d_coef, d_part});
+    be_.for_each((size_t)B, gen::SetFreeCostFn{d_vtx_off, d_part, d_cost});
+    launches(3);
     counters.segment_setups += totS;
     if (coef) be_.d2h(coef, d_coef, sizeof(double) * (size_t)totS * TG_D * N);
     if (cost) be_.d2h(cost, d_cost, sizeof(double) * B);
