@@ -682,6 +682,13 @@ class PolynomialOptimization {
     solved_ = true;
     free_state_ = kFreeNone;
   }
+  // used by optimizeTimeDerivativeFreeBatch: the state after updateSegmentTimes(times) + solveLinear() (free null: getFreeConstraints
+  // fetches the solve's d_p on request), or + setFreeConstraints(free) (free [D][n_free]); coef [S][D][N]
+  void adoptDerivativeFree(const std::vector<double>& times, const std::vector<double>& coef, double cost, const std::vector<double>* free) {
+    adopt(times, coef, cost);
+    free_state_ = free ? kFreeKnown : kFreeFromSolve;
+    if (free) free_ = *free;
+  }
 
  private:
   int countFree() const {
@@ -962,6 +969,153 @@ class PolynomialOptimizationNonLinear {
   std::vector<int> constraint_derivative_;   // in the order the constraints were added (inequality_constraints_, nl.h:223)
   std::vector<double> constraint_value_;
 };
+
+// ---- the derivative-free time allocation on PolynomialOptimization<N> of every shape --------------------------------------
+// A maximum-magnitude constraint as addMaximumMagnitudeConstraint takes it (nl_impl.h:538-565).
+struct MagnitudeConstraint {
+  int dimension;
+  int derivative;
+  double maximum_value;
+};
+namespace b200 {
+inline void split_constraints(const std::vector<MagnitudeConstraint>& constraints, std::vector<int>* dim, std::vector<int>* deriv, std::vector<double>* value) {
+  for (const MagnitudeConstraint& c : constraints) {
+    dim->push_back(c.dimension);
+    deriv->push_back(c.derivative);
+    value->push_back(c.maximum_value);
+  }
+}
+inline bool dfo_method(const NonlinearOptimizationParameters& q) {
+  const int m = (int)q.time_alloc_method;
+  return m == 0 || m == 1 || m == 3 || m == 4;
+}
+}  // namespace b200
+
+// objectiveFunctionTime / objectiveFunctionTimeAndConstraints (nl_impl.h:567-722) of the problem set up in `problem` at K candidate
+// vectors in one call (tg_objective_batch_nd): x = the S segment times (kSquaredTime, kRichterTime), then for the ...AndConstraints
+// methods the free derivatives, getDimension() x n_free dimension-major as getFreeConstraints lists them.  parts (optional):
+// K x {cost_trajectory, cost_time, cost_soft_constraints}.  Returns false, with a message, when the call is refused.
+template <int N>
+bool evaluateObjectives(const PolynomialOptimization<N>& problem, const NonlinearOptimizationParameters& parameters,
+                        const std::vector<MagnitudeConstraint>& constraints, const std::vector<std::vector<double>>& x, std::vector<double>* total,
+                        std::vector<double>* parts = nullptr) {
+  if (!total || x.empty() || !b200::dfo_method(parameters)) return false;
+  const size_t nvar = x.front().size();
+  std::vector<double> flat;
+  flat.reserve(x.size() * nvar);
+  for (const std::vector<double>& xi : x) {
+    if (xi.size() != nvar) return false;
+    flat.insert(flat.end(), xi.begin(), xi.end());
+  }
+  std::vector<int> cdim, cder;
+  std::vector<double> cval;
+  b200::split_constraints(constraints, &cdim, &cder, &cval);
+  std::vector<double> tot(x.size()), pa(3 * x.size());
+  b200::Context& c = b200::Context::instance();
+  const int rc = tg_objective_batch_nd(c.get(), N, (int)problem.getDimension(), (int)problem.vertexMasks().size(), problem.vertexMasks().data(),
+                                       problem.vertexValues().data(), problem.getDerivativeToOptimize(), (int)parameters.time_alloc_method,
+                                       (long long)x.size(), flat.data(), (int)nvar, parameters.time_penalty, parameters.use_soft_constraints ? 1 : 0,
+                                       parameters.soft_constraint_weight, (int)cder.size(), cder.data(), cval.data(), tot.data(), pa.data(), nullptr);
+  if (rc != TG_OK) {
+    std::printf("[evaluateObjectives]: %s\n", tg_last_error(c.get()));
+    return false;
+  }
+  *total = tot;
+  if (parts) *parts = pa;
+  return true;
+}
+
+// PolynomialOptimizationNonLinear<N>::optimize() with a derivative-free method (optimizeTime / optimizeTimeAndFreeConstraints,
+// nl_impl.h:120-157, 429-536; the search of PolynomialOptimizationNonLinear<10>::optimizeBatch) for many problems set up with
+// setupFromVertices, of one shape N, one dimension and one derivative_to_optimize, in ONE device call (tg_time_alloc_dfo_batch_nd;
+// N = 10 on 4 dimensions with derivative_to_optimize >= 2 on the tuned tg_time_alloc_dfo_batch, which gives the same bits).  Not a
+// reference name.  Afterwards every problem is in the state the reference's poly_opt_ is in: kSquaredTime / kRichterTime
+// updateSegmentTimes(final) + solveLinear() (getFreeConstraints returns that solve's d_p), the ...AndConstraints methods
+// updateSegmentTimes(final) + setFreeConstraints(final free derivatives).  codes / infos (optional) get each problem's code and
+// OptimizationInfo.  Returns false, touching nothing, for an empty list, a problem not set up, mixed shapes, the Mellinger method or
+// a refused call.
+template <int N>
+bool optimizeTimeDerivativeFreeBatch(std::vector<PolynomialOptimization<N>*>& problems, const NonlinearOptimizationParameters& parameters,
+                                     const std::vector<MagnitudeConstraint>& constraints, std::vector<int>* codes,
+                                     std::vector<OptimizationInfo>* infos) {
+  if (problems.empty() || !b200::dfo_method(parameters) || !problems[0]) return false;
+  const PolynomialOptimization<N>& f = *problems[0];
+  const int dims = (int)f.getDimension(), r = f.getDerivativeToOptimize(), H = N / 2;
+  const int B = (int)problems.size();
+  std::vector<int> vtx_off(1, 0);
+  std::vector<uint8_t> mask;
+  std::vector<double> vals, times;
+  for (const PolynomialOptimization<N>* o : problems) {
+    if (!o || (int)o->getDimension() != dims || o->getDerivativeToOptimize() != r || o->vertexMasks().size() < 2) return false;
+    std::vector<double> t;
+    o->getSegmentTimes(&t);
+    mask.insert(mask.end(), o->vertexMasks().begin(), o->vertexMasks().end());
+    vals.insert(vals.end(), o->vertexValues().begin(), o->vertexValues().end());
+    times.insert(times.end(), t.begin(), t.end());
+    vtx_off.push_back((int)mask.size());
+  }
+  std::vector<int> cdim, cder;
+  std::vector<double> cval;
+  b200::split_constraints(constraints, &cdim, &cder, &cval);
+  tg_dfo_params P;
+  tg_default_dfo_params(&P);
+  P.time_alloc_method = (int)parameters.time_alloc_method;
+  P.derivative_to_optimize = r;
+  P.max_iterations = parameters.max_iterations;
+  P.f_rel = parameters.f_rel;
+  P.x_rel = parameters.x_rel;
+  P.initial_stepsize_rel = parameters.initial_stepsize_rel;
+  P.time_penalty = parameters.time_penalty;
+  P.use_soft_constraints = parameters.use_soft_constraints ? 1 : 0;
+  P.soft_constraint_weight = parameters.soft_constraint_weight;
+  const bool with_free = P.time_alloc_method >= 3;
+  std::vector<double> coef(times.size() * dims * N), vv(with_free ? vals.size() : 0), total(B), parts(3 * (size_t)B);
+  std::vector<int> code(B), iters(B);
+  b200::Context& c = b200::Context::instance();
+  const bool tuned = N == b200::kN && dims == b200::kD && r >= derivative_order::ACCELERATION;
+  const int rc = tuned ? tg_time_alloc_dfo_batch(c.get(), B, vtx_off.data(), mask.data(), vals.data(), times.data(), &P, (int)cder.size(), cdim.data(),
+                                                 cder.data(), cval.data(), coef.data(), with_free ? vv.data() : nullptr, code.data(), iters.data(),
+                                                 total.data(), parts.data())
+                       : tg_time_alloc_dfo_batch_nd(c.get(), N, dims, B, vtx_off.data(), mask.data(), vals.data(), times.data(), &P, (int)cder.size(),
+                                                    cdim.data(), cder.data(), cval.data(), coef.data(), with_free ? vv.data() : nullptr, code.data(),
+                                                    iters.data(), total.data(), parts.data());
+  if (rc != TG_OK) {
+    std::printf("[optimizeTimeDerivativeFreeBatch]: %s\n", tg_last_error(c.get()));
+    return false;
+  }
+  if (codes) codes->assign(code.begin(), code.end());
+  if (infos) infos->assign(B, OptimizationInfo());
+  size_t s0 = 0;
+  for (int p = 0; p < B; ++p) {
+    PolynomialOptimization<N>& o = *problems[p];
+    const int v0 = vtx_off[p], V = vtx_off[p + 1] - v0;
+    const size_t S = (size_t)V - 1;
+    std::vector<double> free;
+    if (with_free) {  // the free slots of vval_out, dimension-major (getFreeConstraints' layout)
+      const size_t nf = o.getNumberFreeConstraints();
+      free.assign(std::max<size_t>((size_t)dims * nf, 1), 0.0);
+      size_t j = 0;
+      for (int v = 0; v < V; ++v)
+        for (int k = 0; k < H; ++k) {
+          if ((mask[v0 + v] >> k) & 1u) continue;
+          for (int d = 0; d < dims; ++d) free[(size_t)d * nf + j] = vv[(((size_t)v0 + v) * H + k) * dims + d];
+          ++j;
+        }
+    }
+    o.adoptDerivativeFree(std::vector<double>(times.begin() + s0, times.begin() + s0 + S),
+                          std::vector<double>(coef.begin() + s0 * dims * N, coef.begin() + (s0 + S) * dims * N), parts[3 * p], with_free ? &free : nullptr);
+    if (infos) {
+      OptimizationInfo& info = (*infos)[p];
+      info.cost_trajectory = parts[3 * p];
+      info.cost_time = parts[3 * p + 1];
+      info.cost_soft_constraints = parts[3 * p + 2];
+      info.n_iterations = iters[p];
+      info.stopping_reason = code[p];
+    }
+    s0 += S;
+  }
+  return true;
+}
 
 // ---- batch entry: the numeric core of optimize() / findTrajectory for many paths (node.cpp:620-851, 857-1209) -------------
 struct Waypoint {

@@ -269,6 +269,27 @@ int tg_time_alloc_dfo_batch(tg_ctx* ctx, int B, const int* vtx_off, const uint8_
                             const tg_dfo_params* params, int n_constraints, const int* con_dimension, const int* con_derivative,
                             const double* con_value, double* coef, double* vval_out, int* code, int* n_iterations, double* total, double* parts);
 
+/* The derivative-free time allocation for PolynomialOptimization<N>, N in {6, 8, 10, 12}, D in 1..4 dimensions:
+ * tg_objective_batch_nd      = tg_objective_batch over N coefficients and D dimensions: vval[V][N/2][D]; x[K][nvar], nvar = S
+ *                              (methods 0, 1) or S + D * n_free (methods 3, 4; the free derivatives dimension-major, D x n_free,
+ *                              the layout of tg_solve_linear_free_batch_nd); coef (optional) [K][S][D][N].
+ * tg_time_alloc_dfo_batch_nd = tg_time_alloc_dfo_batch over N coefficients and D dimensions: the same search, bounds, steps and
+ *                              codes, with variables for the D dimensions only (n = S or S + D * n_free); vval, vval_out
+ *                              [totV][N/2][D], coef[totS][D][N]; the other outputs as tg_time_alloc_dfo_batch.  A constraint is
+ *                              shared by every problem as there (dimension 0..3: a bound that lands outside the variables is
+ *                              dropped); its magnitude is taken over the D dimensions.
+ *   derivative_to_optimize (r) is 0 .. N/2-1 in both.  Both refuse with TG_ERR_INVALID, writing no output, N outside {6, 8, 10, 12},
+ *   D outside 1..4, r outside 0 .. N/2-1, a method other than 0, 1, 3, 4, K or B < 1, a problem with fewer than two vertices, more
+ *   than 16 constraints or one with a dimension outside 0..3, a derivative outside 1..4 or a zero value, and a wrong nvar.
+ *   Non-finite inputs are not refused and propagate. */
+int tg_objective_batch_nd(tg_ctx* ctx, int N, int D, int V, const uint8_t* vmask, const double* vval, int r, int time_alloc_method, long long K,
+                          const double* x, int nvar, double time_penalty, int use_soft_constraints, double soft_constraint_weight,
+                          int n_constraints, const int* con_derivative, const double* con_value, double* total, double* parts, double* coef);
+int tg_time_alloc_dfo_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                               const tg_dfo_params* params, int n_constraints, const int* con_dimension, const int* con_derivative,
+                               const double* con_value, double* coef, double* vval_out, int* code, int* n_iterations, double* total,
+                               double* parts);
+
 /* The steps either side of the path (SURVEY.md 8f ranks 1-2), batched, one path per thread --------------------------------
  * tg_preprocess_paths = MrsTrajectoryGeneration::preprocessPath (src/mrs_trajectory_generation.cpp:431-500): optional path
  *   straightener (config/public/trajectory_generation.yaml:20-23) then the min_waypoint_distance filter (:27).

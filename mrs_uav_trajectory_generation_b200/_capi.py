@@ -152,6 +152,10 @@ class Library:
         L.tg_default_dfo_params.argtypes = [C.POINTER(DfoParams)]
         L.tg_time_alloc_dfo_batch.argtypes = [C.c_void_p, C.c_int, _ip, _u8p, _dp, _dp, C.POINTER(DfoParams), C.c_int, _ip, _ip, _dp, _dp, _dp, _ip,
                                               _ip, _dp, _dp]
+        L.tg_objective_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _u8p, _dp, C.c_int, C.c_int, C.c_longlong, _dp, C.c_int, C.c_double,
+                                            C.c_int, C.c_double, C.c_int, _ip, _dp, _dp, _dp, _dp]
+        L.tg_time_alloc_dfo_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.POINTER(DfoParams), C.c_int, _ip, _ip,
+                                                 _dp, _dp, _dp, _ip, _ip, _dp, _dp]
         L.tg_max_magnitude_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
         L.tg_scale_times_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp, _ip, _u8p]
         L.tg_sweep_costs.argtypes = [C.c_void_p, C.c_int, _u8p, _dp, C.c_int, C.c_longlong, _dp, C.c_int, _dp, _llp, _dp]
@@ -608,6 +612,48 @@ class Context:
         self._check(self.L.lib.tg_time_alloc_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times), C.byref(P),
                                                       _p(coef), _p(code, _ip), _p(evals, _ip), _p(passes, _ip), _p(cost)))
         return {"times": times, "coef": coef, "nlopt_code": code, "n_evals": evals, "n_scale_passes": passes, "final_cost": cost}
+
+    def objective_nd(self, n_coef, dim, mask, vals, r, method, x, time_penalty=500.0, use_soft=True, soft_weight=100.0, con_deriv=(),
+                     con_value=(), want_coef=False):
+        """objective() for PolynomialOptimizationNonLinear<n_coef>(dim): vals [V][n_coef/2][dim]; x [K][nvar], nvar = S or S + dim * n_free
+        (the free derivatives dimension-major) -> total[K], parts[K][3] (and coef [K][S][dim][n_coef] with want_coef)."""
+        mask = np.ascontiguousarray(mask, dtype=np.uint8)
+        vals = np.ascontiguousarray(vals, dtype=np.float64)
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        K, nvar = x.shape
+        cd = np.ascontiguousarray(con_deriv, dtype=np.int32)
+        cv = np.ascontiguousarray(con_value, dtype=np.float64)
+        total, parts = np.empty(K), np.empty((K, 3))
+        coef = np.empty((K, len(mask) - 1, dim, n_coef)) if want_coef else None
+        self._check(self.L.lib.tg_objective_batch_nd(self.h, int(n_coef), int(dim), len(mask), _p(mask, _u8p), _p(vals), int(r), int(method), K, _p(x),
+                                                     nvar, float(time_penalty), int(bool(use_soft)), float(soft_weight), len(cd), _p(cd, _ip), _p(cv),
+                                                     _p(total), _p(parts), _p(coef) if want_coef else None))
+        return (total, parts, coef) if want_coef else (total, parts)
+
+    def time_alloc_dfo_batch_nd(self, n_coef, dim, vtx_off, vmask, vval, times, params=None, constraints=()):
+        """time_alloc_dfo_batch for PolynomialOptimizationNonLinear<n_coef>(dim): vval [totV][n_coef/2][dim], derivative_to_optimize
+        0 .. n_coef/2-1.  Returns the dict of time_alloc_dfo_batch with coef [totS][dim][n_coef] and vval [totV][n_coef/2][dim]."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        vmask = np.ascontiguousarray(vmask, dtype=np.uint8)
+        vval = np.ascontiguousarray(vval, dtype=np.float64)
+        times = np.array(times, dtype=np.float64, copy=True)
+        B = len(vtx_off) - 1
+        totS = int(vtx_off[-1]) - B
+        assert vval.size == int(vtx_off[-1]) * (n_coef // 2) * dim and times.size == totS
+        P = params or self.L.default_dfo_params()
+        cdim = np.ascontiguousarray([c[0] for c in constraints], dtype=np.int32)
+        cder = np.ascontiguousarray([c[1] for c in constraints], dtype=np.int32)
+        cval = np.ascontiguousarray([c[2] for c in constraints], dtype=np.float64)
+        coef = np.empty((totS, dim, n_coef))
+        vval_out = vval.copy() if P.time_alloc_method >= 3 else None
+        code = np.zeros(B, dtype=np.int32)
+        iters = np.zeros(B, dtype=np.int32)
+        total = np.zeros(B)
+        parts = np.zeros((B, 3))
+        self._check(self.L.lib.tg_time_alloc_dfo_batch_nd(self.h, int(n_coef), int(dim), B, _p(vtx_off, _ip), _p(vmask, _u8p), _p(vval), _p(times),
+                                                          C.byref(P), len(cdim), _p(cdim, _ip), _p(cder, _ip), _p(cval), _p(coef), _p(vval_out),
+                                                          _p(code, _ip), _p(iters, _ip), _p(total), _p(parts)))
+        return {"times": times, "coef": coef, "vval": vval_out, "code": code, "n_iterations": iters, "total": total, "parts": parts}
 
     def extrema(self, coef, times):
         coef = np.ascontiguousarray(coef, dtype=np.float64)

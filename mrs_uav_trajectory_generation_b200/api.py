@@ -323,17 +323,20 @@ class DerivativeFreeTimeAllocation:
     and stopping rules are the reference's and the search itself is ours: a bound-constrained coordinate pattern search whose 2n trial
     points per iteration are evaluated together on the GPU (tg_time_alloc_dfo_batch, here with one problem; TrajectoryGenerator.
     time_alloc_derivative_free runs many).  max_iterations counts those batched iterations, not single evaluations.  Result codes
-    as NLopt: 3 ftol_rel, 4 xtol_rel, 5 maxeval.
+    as NLopt: 3 ftol_rel, 4 xtol_rel, 5 maxeval.  n_coefficients / dimension: the shape of PolynomialOptimization<N> (N in
+    {6, 8, 10, 12}, 1..4 dimensions, derivative_to_optimize 0 .. N/2-1); N = 10 on 4 dimensions runs tg_time_alloc_dfo_batch, every
+    other shape tg_time_alloc_dfo_batch_nd.
     """
 
     kTimeLowerBound = 0.01  # kOptimizationTimeLowerBound (nl.h:143)
 
-    def __init__(self, vertices, times, derivative_to_optimize, parameters, constraints, ctx=None):
+    def __init__(self, vertices, times, derivative_to_optimize, parameters, constraints, ctx=None, n_coefficients=N, dimension=D):
         self.ctx = ctx or default_context()
         self.P = parameters
         self.r = derivative_to_optimize
+        self.N, self.dimension = n_coefficients, dimension
         self.vertices = list(vertices)
-        _, self.mask, self.vals = pack_vertices([vertices])
+        _, self.mask, self.vals = pack_vertices([vertices], n_coefficients // 2, dimension)
         self.times0 = np.asarray(times, dtype=np.float64)
         self.S = len(self.times0)
         self.constraints = list(constraints)  # (dimension, derivative, value) in the order they were added
@@ -341,16 +344,23 @@ class DerivativeFreeTimeAllocation:
 
     def optimize(self):
         vtx_off = np.array([0, len(self.mask)], dtype=np.int32)
-        out = self.ctx.time_alloc_dfo_batch(vtx_off, self.mask, self.vals, self.times0, _dfo_params(self.ctx, self.P, self.r), self.constraints)
+        out = _dfo_batch(self.ctx, self.N, self.dimension, vtx_off, self.mask, self.vals, self.times0, _dfo_params(self.ctx, self.P, self.r),
+                         self.constraints)
         self.times, self.coef = out["times"], out["coef"]
         self.x = self.times.copy()
         if self.with_free:  # x = the times, then the free derivatives dimension-major (getFreeConstraints, vertex-major slots)
-            free = [out["vval"][v, k] for v in range(len(self.mask)) for k in range(HALF) if not (self.mask[v] >> k) & 1]
-            self.x = np.concatenate([self.x, np.array(free).reshape(-1, D).T.reshape(-1)])
+            free = [out["vval"][v, k] for v in range(len(self.mask)) for k in range(self.N // 2) if not (self.mask[v] >> k) & 1]
+            self.x = np.concatenate([self.x, np.array(free).reshape(-1, self.dimension).T.reshape(-1)])
         self.cost = float(out["total"][0])
         self.cost_parts = out["parts"][0]
         self.n_iterations = int(out["n_iterations"][0])
         return int(out["code"][0])
+
+
+def _dfo_batch(ctx, n_coef, dim, vtx_off, masks, vals, times, params, constraints):
+    if (n_coef, dim) == (N, D) and params.derivative_to_optimize >= 2:  # the tuned kernels: the same bits
+        return ctx.time_alloc_dfo_batch(vtx_off, masks, vals, times, params, constraints)
+    return ctx.time_alloc_dfo_batch_nd(n_coef, dim, vtx_off, masks, vals, times, params, constraints)
 
 
 def _dfo_params(ctx, P, r):
@@ -567,13 +577,16 @@ class TrajectoryGenerator:
                 placed[i] = (br, k)
         return placed, resolved
 
-    def time_alloc_derivative_free(self, vertex_lists, times_list, parameters, constraints=(), derivative_to_optimize=2):
-        """PolynomialOptimizationNonLinear<10>::optimize() with a derivative-free method (parameters.time_alloc_method 0, 1, 3 or 4) for
-        many problems in one call.  vertex_lists: one list of Vertex(4) per problem; times_list: their initial segment times;
-        constraints: (dimension, derivative, value) added to every problem.  Returns ([Trajectory], codes[B])."""
-        vtx_off, masks, vals = pack_vertices(vertex_lists)
+    def time_alloc_derivative_free(self, vertex_lists, times_list, parameters, constraints=(), derivative_to_optimize=2, n_coefficients=N,
+                                   dimension=D):
+        """PolynomialOptimizationNonLinear<N>::optimize() with a derivative-free method (parameters.time_alloc_method 0, 1, 3 or 4) for
+        many problems in one call.  vertex_lists: one list of Vertex(dimension) per problem; times_list: their initial segment times;
+        constraints: (dimension, derivative, value) added to every problem; n_coefficients in {6, 8, 10, 12}, dimension 1..4.  Returns
+        ([Trajectory], codes[B])."""
+        vtx_off, masks, vals = pack_vertices(vertex_lists, n_coefficients // 2, dimension)
         times = np.concatenate([np.asarray(t, dtype=np.float64) for t in times_list])
-        out = self.ctx.time_alloc_dfo_batch(vtx_off, masks, vals, times, _dfo_params(self.ctx, parameters, derivative_to_optimize), list(constraints))
+        out = _dfo_batch(self.ctx, n_coefficients, dimension, vtx_off, masks, vals, times, _dfo_params(self.ctx, parameters, derivative_to_optimize),
+                         list(constraints))
         seg_off = vtx_off - np.arange(len(vtx_off), dtype=np.int32)
         trajs = [Trajectory(out["coef"][seg_off[p]:seg_off[p + 1]], out["times"][seg_off[p]:seg_off[p + 1]], self.ctx) for p in range(len(vertex_lists))]
         return trajs, out["code"]

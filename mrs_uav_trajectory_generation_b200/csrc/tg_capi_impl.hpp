@@ -709,6 +709,93 @@ int tg_time_alloc_dfo_batch(tg_ctx* ctx, int B, const int* vtx_off, const uint8_
   });
 }
 
+namespace {
+// the constraint rules of tg_time_alloc_dfo_batch (con_dimension may be null: tg_objective_batch_nd has no dimensions)
+inline bool tg_dfo_constraints_ok(int n, const int* dim, const int* deriv, const double* value) {
+  if (n < 0 || n > 16 || (n > 0 && (!deriv || !value))) return false;
+  for (int c = 0; c < n; ++c)
+    if (deriv[c] < 1 || deriv[c] > 4 || (dim && (dim[c] < 0 || dim[c] > 3)) || !(value[c] != 0.0)) return false;
+  return true;
+}
+inline bool tg_dfo_method_ok(int m) { return m == 0 || m == 1 || m == 3 || m == 4; }
+}  // namespace
+
+int tg_objective_batch_nd(tg_ctx* ctx, int N, int D, int V, const uint8_t* vmask, const double* vval, int r, int time_alloc_method, long long K,
+                          const double* x, int nvar, double time_penalty, int use_soft_constraints, double soft_constraint_weight,
+                          int n_constraints, const int* con_derivative, const double* con_value, double* total, double* parts, double* coef) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (V < 2 || !vmask || !vval || r < 0 || r > N / 2 - 1 || K < 1 || !x || !total) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    if (!tg_dfo_method_ok(time_alloc_method)) { ctx->err = "time_alloc_method must be 0, 1, 3 or 4"; return TG_ERR_INVALID; }
+    if (!tg_dfo_constraints_ok(n_constraints, nullptr, con_derivative, con_value)) {
+      ctx->err = "at most 16 constraints, derivatives 1..4, non-zero values";
+      return TG_ERR_INVALID;
+    }
+    const int S = V - 1, nf = tg_free_counts(N, 1, std::vector<int>{0, V}.data(), vmask)[0];
+    const bool with_free = time_alloc_method >= 3;
+    if (nvar != (with_free ? S + D * nf : S)) { ctx->err = "nvar must be S (methods 0, 1) or S + D * n_free (methods 3, 4)"; return TG_ERR_INVALID; }
+    const std::vector<double> vv = tg_pad_dims(vval, (size_t)V * (N / 2), D);
+    // x with the free derivatives of the missing dimensions zero: [K][S + 4 * n_free]
+    const int nvar4 = with_free ? S + TG_D * nf : S;
+    std::vector<double> x4;
+    if (with_free && D < TG_D) {
+      x4.assign((size_t)K * nvar4, 0.0);
+      for (long long k = 0; k < K; ++k) std::memcpy(&x4[(size_t)k * nvar4], x + (size_t)k * nvar, sizeof(double) * nvar);
+    }
+    std::vector<double> c4(coef ? (size_t)K * S * TG_D * N : 0);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto n) {
+      ctx->pipe.template objective_batch_n<decltype(n)::value>(V, vmask, vv.data(), r, time_alloc_method, K, x4.empty() ? x : x4.data(), nvar4,
+                                                               time_penalty, use_soft_constraints, soft_constraint_weight, n_constraints,
+                                                               con_derivative, con_value, total, parts, coef ? c4.data() : nullptr);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (coef) tg_strip_coef(c4.data(), (size_t)K * S, N, D, coef);
+    return TG_OK;
+  });
+}
+
+int tg_time_alloc_dfo_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times,
+                               const tg_dfo_params* params, int n_constraints, const int* con_dimension, const int* con_derivative,
+                               const double* con_value, double* coef, double* vval_out, int* code, int* n_iterations, double* total,
+                               double* parts) {
+  return tg_guard(ctx, [&]() -> int {
+    if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }
+    if (B < 1 || !vtx_off || !vmask || !vval || !times || !params) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] - vtx_off[p] < 2) { ctx->err = "every problem needs at least two vertices"; return TG_ERR_INVALID; }
+    if (!tg_dfo_method_ok(params->time_alloc_method)) { ctx->err = "time_alloc_method must be 0, 1, 3 or 4"; return TG_ERR_INVALID; }
+    if (params->derivative_to_optimize < 0 || params->derivative_to_optimize > N / 2 - 1) {
+      ctx->err = "derivative_to_optimize must be 0 .. N/2-1";
+      return TG_ERR_INVALID;
+    }
+    if (!tg_dfo_constraints_ok(n_constraints, con_dimension, con_derivative, con_value) || (n_constraints > 0 && !con_dimension)) {
+      ctx->err = "at most 16 constraints, with dimension 0..3, derivative 1..4 and a non-zero value";
+      return TG_ERR_INVALID;
+    }
+    tg::DfoParams P;
+    std::memcpy(&P, params, sizeof(P));
+    const size_t totV = (size_t)vtx_off[B], totS = totV - (size_t)B, H = (size_t)(N / 2);
+    const std::vector<double> vv = tg_pad_dims(vval, totV * H, D);
+    std::vector<double> c4(coef ? totS * TG_D * N : 0), v4(vval_out ? totV * H * TG_D : 0);
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto n) {
+      ctx->pipe.template dfo_batch_n<decltype(n)::value>(D, B, vtx_off, vmask, vv.data(), times, P, n_constraints, con_dimension, con_derivative,
+                                                         con_value, coef ? c4.data() : nullptr, vval_out ? v4.data() : nullptr, code,
+                                                         n_iterations, total, parts);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (coef) tg_strip_coef(c4.data(), totS, N, D, coef);
+    if (vval_out) {
+      if (P.time_alloc_method >= 3) {
+        for (size_t i = 0; i < totV * H; ++i)
+          for (int d = 0; d < D; ++d) vval_out[i * D + d] = v4[i * TG_D + d];
+      }
+    }
+    return TG_OK;
+  });
+}
+
 int tg_scale_times_batch(tg_ctx* ctx, int B, const int* seg_off, double* coef, double* times, const double* limits9, int* passes,
                          uint8_t* within) {
   return tg_guard(ctx, [&]() -> int {

@@ -20,6 +20,7 @@
 //   ScaleFn<N>                                         scaleSegmentTimesToMeetConstraints' stretch (eth/trajectory.cpp:610-658)
 //   MellingerHeadFn / HrowFn / SolveFn<N>              one Mellinger evaluation: S+1 solves per running problem (nl_impl.h:282-323);
 //                                                      the optimiser state machine (tg_plis.cuh) does not depend on N
+//   candidate_rec<N>                                   the record rule of a derivative-free candidate's solve (tg_dfo_generic.cuh)
 // Every sum is the DENSE sum over ascending index, exactly as the reference-order restatement writes it (the tuned path skips structural
 // zeros, which is the same IEEE result); for N = 10 this path and the tuned one are compared bit for bit in the tests.
 // D: the device works on 4 right-hand sides; tg_*_nd pad D < 4 with zero dimensions (a zero dimension adds exact zeros to the
@@ -183,6 +184,23 @@ TG_HD const double* problem_rec(const Problem& P, int s) {
   const int which = (P.rec_stride == 1 || P.variant == 0) ? 0 : (s == P.variant - 1 ? 1 : 2);
   return P.recs + ((size_t)s * P.rec_stride + which) * Rec<N>::kSize;
 }
+// the record segment s is solved with by a derivative-free candidate (tg_dfo_generic.cuh), the rule of solve_rec (tg_solve.cuh) for
+// variant <= 0: variant 0 the point itself (record 0 everywhere); variant -(2 i + dir + 1) the point with segment i moved by +step
+// (dir 0) or -step (dir 1): record 1 + dir on segment i and record 0 on every other segment (DESIGN.md 4.4)
+template <int N>
+TG_HD const double* candidate_rec(const Problem& P, int s) {
+  int which = 0;
+  if (P.variant < 0) {
+    const int c = -P.variant - 1;
+    which = (s == (c >> 1)) ? 1 + (c & 1) : 0;
+  }
+  return P.recs + ((size_t)s * P.rec_stride + which) * Rec<N>::kSize;
+}
+template <int N, bool kCandidate>
+TG_HD const double* warp_rec(const Problem& P, int s) {
+  if (kCandidate) return candidate_rec<N>(P, s);
+  return problem_rec<N>(P, s);
+}
 TG_HD int row_stride(int hbw) { return 2 * hbw + 1 + TG_D + 1; }  // band, 4 right-hand sides, reciprocal pivot
 template <int N>
 TG_HD size_t ws_doubles(int S, int np, int hbw) {
@@ -220,7 +238,8 @@ TG_HD int free_rank(uint32_t mask, int a) {
   return rank;
 }
 
-template <int N>
+// kCandidate: the records are selected by candidate_rec (a derivative-free candidate) instead of problem_rec
+template <int N, bool kCandidate = false>
 TG_HD void solve_warp(const Problem& P, int lane) {
   constexpr int H = N / 2;
   (void)lane;
@@ -248,8 +267,8 @@ TG_HD void solve_warp(const Problem& P, int lane) {
         if (i < 0) continue;
         const int v = it / H, a = it - v * H;
         const bool has_p = v > 0, has_c = v < S;
-        const double* hp = has_p ? problem_rec<N>(P, v - 1) + Rec<N>::kH + (H + a) * N : nullptr;
-        const double* hc = has_c ? problem_rec<N>(P, v) + Rec<N>::kH + a * N : nullptr;
+        const double* hp = has_p ? warp_rec<N, kCandidate>(P, v - 1) + Rec<N>::kH + (H + a) * N : nullptr;
+        const double* hc = has_c ? warp_rec<N, kCandidate>(P, v) + Rec<N>::kH + a * N : nullptr;
         double* row = rows + (size_t)i * W;
         double acc0 = 0.0, acc1 = 0.0, acc2 = 0.0, acc3 = 0.0;
         for (int g = 0; g < 3; ++g) {
@@ -320,7 +339,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
   TG_PHASE(lane) {
     for (int it = lane; it < S * TG_D * N; it += 32) {
       const int s = it / (TG_D * N), rem = it - s * (TG_D * N), d = rem / N, a = rem - d * N;
-      const double* Ai = problem_rec<N>(P, s) + Rec<N>::kAinv + a * N;
+      const double* Ai = warp_rec<N, kCandidate>(P, s) + Rec<N>::kAinv + a * N;
       const double c = coef_from_endpoints<N>(Ai, [&](int k) {
         const int j = slot[s * H + k];  // the slots of vertex s and of vertex s+1 are contiguous in the table
         return (j >= 0) ? xs[j * 4 + d] : P.vval[((size_t)s * H + k) * TG_D + d];
@@ -333,7 +352,7 @@ TG_HD void solve_warp(const Problem& P, int lane) {
   TG_PHASE(lane) {
     for (int it = lane; it < S * TG_D; it += 32) {
       const int s = it / TG_D;
-      part[it] = cost_partial<N>(problem_rec<N>(P, s) + Rec<N>::kQ, cf + (size_t)it * N);
+      part[it] = cost_partial<N>(warp_rec<N, kCandidate>(P, s) + Rec<N>::kQ, cf + (size_t)it * N);
     }
   }
   // ---- phase 6: total in (segment, dimension) order (lin_impl.h:131-140)

@@ -20,6 +20,7 @@
 
 #include "tg_kernels.cuh"
 #include "tg_dfo.cuh"
+#include "tg_dfo_generic.cuh"
 #include "tg_generic.cuh"
 
 namespace tg {
@@ -1312,21 +1313,28 @@ class Pipeline {
   // one iteration recompute: S per candidate for methods 0, 1, two for 3, 4); a group runs its whole search before the next starts.
   void dfo_batch(int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const DfoParams& Q, int ncon, const int* con_dim,
                  const int* con_deriv, const double* con_value, double* coef, double* vval_out, int* code, int* n_iter, double* total, double* parts) {
-    const bool with_free = Q.time_alloc_method >= 3;
+    dfo_groups(B, vtx_off, vmask, TG_HALF, TG_D, Q.time_alloc_method >= 3, [&](int p0, int p1) {
+      dfo_group(p0, p1, vtx_off, vmask, vval, times, Q, ncon, con_dim, con_deriv, con_value, coef, vval_out, code, n_iter, total, parts);
+    });
+  }
+  // the groups of dfo_batch / dfo_batch_n: run(p0, p1) for consecutive problems [p0, p1) of at most seg_budget candidate segments
+  // (a problem over its budget alone forms a group); half = N/2 derivatives per vertex, dims = D dimensions with variables
+  template <class Run>
+  void dfo_groups(int B, const int* vtx_off, const uint8_t* vmask, int half, int dims, bool with_free, const Run& run) {
     std::vector<size_t> units(B);
     for (int p = 0; p < B; ++p) {
       const int V = vtx_off[p + 1] - vtx_off[p], S = V - 1;
       int nf = 0;
       for (int v = vtx_off[p]; v < vtx_off[p + 1]; ++v)
-        for (int k = 0; k < TG_HALF; ++k) nf += ((vmask[v] >> k) & 1u) ? 0 : 1;
-      const size_t n = (size_t)(with_free ? S + TG_D * nf : S);
+        for (int k = 0; k < half; ++k) nf += ((vmask[v] >> k) & 1u) ? 0 : 1;
+      const size_t n = (size_t)(with_free ? S + dims * nf : S);
       units[p] = 2 * n * (size_t)(with_free ? 2 : S);
     }
     for (int p0 = 0; p0 < B;) {
       int p1 = p0 + 1;
       size_t u = units[p0];
       while (p1 < B && u + units[p1] <= seg_budget) u += units[p1++];
-      dfo_group(p0, p1, vtx_off, vmask, vval, times, Q, ncon, con_dim, con_deriv, con_value, coef, vval_out, code, n_iter, total, parts);
+      run(p0, p1);
       p0 = p1;
     }
   }
@@ -1895,6 +1903,344 @@ class Pipeline {
     be_.d2h(times, b.times, sizeof(double) * totS);
     if (coef) be_.d2h(coef, b.coef, sizeof(double) * (size_t)totS * TG_D * N);
     return true;
+  }
+
+  // objectiveFunctionTime / objectiveFunctionTimeAndConstraints (objective_batch) of ONE problem of N-coefficient segments at K
+  // candidate vectors; the caller has validated the inputs.  The K candidates are solved as K copies of the problem: methods 0, 1
+  // with linear_batch_n's kernels, 3, 4 with set_free_batch_n's (the free derivatives are read from x in place).  vval: [V][N/2][4];
+  // x: [K][nvar], nvar = S or S + 4 * n_free; coef out: [K][S][4][N].
+  template <int N>
+  void objective_batch_n(int V, const uint8_t* vmask, const double* vval, int r, int method, long long K, const double* x, int nvar,
+                         double time_penalty, int use_soft, double soft_weight, int ncon, const int* con_deriv, const double* con_value,
+                         double* total, double* parts, double* coef) {
+    constexpr int H = N / 2;
+    scratch_.reset();
+    const int S = V - 1;
+    bool need[4] = {false, false, false, false};
+    for (int c = 0; c < ncon; ++c) need[con_deriv[c] - 1] = use_soft != 0;
+    const int one[2] = {0, V};
+    const GenVertices g1 = gen_vertices<N>(1, one, vmask);
+    const long long w = (long long)gen::ws_doubles<N>(S, g1.np[0], g1.hbw[0]);
+    const long long chunk = std::min<long long>(K, (long long)objective_chunk);
+    const size_t C = (size_t)chunk;
+    std::vector<int> vo(C + 1), so(C + 1), vfree(C * (V + 1)), np(C, g1.np[0]), hbw(C, g1.hbw[0]), pos(C * S);
+    std::vector<long long> ws_off(C), dp_off(C);
+    std::vector<uint8_t> vm(C * V);
+    std::vector<double> vv(C * V * H * TG_D);
+    for (size_t k = 0; k <= C; ++k) {
+      vo[k] = (int)(k * V);
+      so[k] = (int)(k * S);
+    }
+    for (size_t k = 0; k < C; ++k) {
+      std::memcpy(&vfree[k * (V + 1)], g1.vfree.data(), sizeof(int) * (V + 1));
+      std::memcpy(&vm[k * V], vmask, V);
+      std::memcpy(&vv[k * V * H * TG_D], vval, sizeof(double) * V * H * TG_D);
+      for (int s = 0; s < S; ++s) pos[k * S + s] = (int)k;
+      ws_off[k] = (long long)k * w;
+      dp_off[k] = (long long)k * nvar + S;
+    }
+    int* d_vo = scratch_.template alloc<int>(C + 1);
+    int* d_so = scratch_.template alloc<int>(C + 1);
+    int* d_pos = scratch_.template alloc<int>(C * S);
+    uint8_t* d_vm = scratch_.template alloc<uint8_t>(C * V);
+    int* d_vfree = scratch_.template alloc<int>(vfree.size());
+    double* d_vv = scratch_.template alloc<double>(vv.size());
+    int* d_np = scratch_.template alloc<int>(C);
+    int* d_hbw = scratch_.template alloc<int>(C);
+    long long* d_ws_off = scratch_.template alloc<long long>(C);
+    long long* d_dp_off = scratch_.template alloc<long long>(C);
+    double* d_ws = method < 3 ? scratch_.template alloc<double>((size_t)std::max<long long>(w * chunk, 1)) : nullptr;
+    double* d_x = scratch_.template alloc<double>(C * nvar);
+    double* d_T = scratch_.template alloc<double>(C * S);
+    double* d_recs = scratch_.template alloc<double>(C * S * gen::Rec<N>::kSize);
+    double* d_coef = scratch_.template alloc<double>(C * S * TG_D * N);
+    double* d_part = scratch_.template alloc<double>(C * S * TG_D);
+    double* d_costs = scratch_.template alloc<double>(C);
+    double* d_sv = scratch_.template alloc<double>(C * S);
+    double* d_st = scratch_.template alloc<double>(C * S);
+    double* d_max = scratch_.template alloc<double>(4 * C);
+    double* d_mt = scratch_.template alloc<double>(C);
+    int* d_mi = scratch_.template alloc<int>(C);
+    double* d_total = scratch_.template alloc<double>(C);
+    double* d_parts = scratch_.template alloc<double>(3 * C);
+    be_.h2d(d_vo, vo.data(), sizeof(int) * (C + 1));
+    be_.h2d(d_so, so.data(), sizeof(int) * (C + 1));
+    be_.h2d(d_pos, pos.data(), sizeof(int) * C * S);
+    be_.h2d(d_vm, vm.data(), C * V);
+    be_.h2d(d_vfree, vfree.data(), sizeof(int) * vfree.size());
+    be_.h2d(d_vv, vv.data(), sizeof(double) * vv.size());
+    be_.h2d(d_np, np.data(), sizeof(int) * C);
+    be_.h2d(d_hbw, hbw.data(), sizeof(int) * C);
+    be_.h2d(d_ws_off, ws_off.data(), sizeof(long long) * C);
+    be_.h2d(d_dp_off, dp_off.data(), sizeof(long long) * C);
+    const ObjTerms terms = obj_terms(method, time_penalty, use_soft, soft_weight, ncon, con_deriv, con_value);
+    std::vector<double> T(C * S);
+    for (long long k0 = 0; k0 < K; k0 += chunk) {
+      const long long kc = std::min(chunk, K - k0);
+      for (long long k = 0; k < kc; ++k) std::memcpy(&T[(size_t)k * S], x + (size_t)(k0 + k) * nvar, sizeof(double) * S);
+      be_.h2d(d_x, x + (size_t)k0 * nvar, sizeof(double) * (size_t)kc * nvar);
+      be_.h2d(d_T, T.data(), sizeof(double) * (size_t)kc * S);
+      const size_t nS = (size_t)kc * S;
+      be_.for_each(nS, gen::RecordHeadFn<N>{r, d_T, d_recs});
+      if (method >= 3) {
+        be_.for_each(nS * TG_D, gen::SetFreeFn<N>{d_pos, d_vm, d_vfree, d_vv, d_dp_off, d_np, d_x, d_recs, d_coef, d_part});
+        be_.for_each((size_t)kc, gen::SetFreeCostFn{d_vo, d_part, d_costs});
+      } else {
+        be_.for_each(nS * N, gen::RecordHrowFn<N>{d_recs});
+        be_.for_each_warp((size_t)kc, gen::SolveFn<N>{r, d_vo, d_vm, d_vfree, d_vv, d_np, d_hbw, d_recs, d_ws_off, d_ws, d_coef, d_costs});
+        counters.solves += kc;
+      }
+      launches(3);
+      counters.segment_setups += (long long)nS;
+      for (int kd = 1; kd <= 4; ++kd) {
+        if (!need[kd - 1]) continue;
+        switch (kd) {
+          case 1: be_.for_each_scratch(nS, gen::MaxMagnitudeSegFn<N, 1>{d_coef, d_T, d_sv, d_st}); break;
+          case 2: be_.for_each_scratch(nS, gen::MaxMagnitudeSegFn<N, 2>{d_coef, d_T, d_sv, d_st}); break;
+          case 3: be_.for_each_scratch(nS, gen::MaxMagnitudeSegFn<N, 3>{d_coef, d_T, d_sv, d_st}); break;
+          default: be_.for_each_scratch(nS, gen::MaxMagnitudeSegFn<N, 4>{d_coef, d_T, d_sv, d_st}); break;
+        }
+        be_.for_each((size_t)kc, MaxMagnitudeReduceFn{d_so, d_sv, d_st, d_max + (size_t)(kd - 1) * C, d_mt, d_mi});
+        launches(2);
+        counters.root_finds += (long long)nS;
+        counters.root_finds_executed += (long long)nS;
+      }
+      be_.for_each((size_t)kc, ObjCombineFn{S, terms, d_T, d_costs, d_max, C, d_total, d_parts});
+      launches(1);
+      be_.d2h(total + k0, d_total, sizeof(double) * (size_t)kc);
+      if (parts) be_.d2h(parts + 3 * (size_t)k0, d_parts, sizeof(double) * 3 * (size_t)kc);
+      if (coef) be_.d2h(coef + (size_t)k0 * S * TG_D * N, d_coef, sizeof(double) * nS * TG_D * N);
+    }
+  }
+
+  // dfo_batch for N-coefficient segments (tg_dfo_generic.cuh): the same search, state, groups and candidate reuse; the caller has
+  // validated the inputs.  The free derivatives of dimensions d < D are variables.  vval, vval_out: [totV][N/2][4] (dimensions
+  // d >= D zero); coef out: [totS][4][N].
+  template <int N>
+  void dfo_batch_n(int D, int B, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const DfoParams& Q, int ncon,
+                   const int* con_dim, const int* con_deriv, const double* con_value, double* coef, double* vval_out, int* code, int* n_iter,
+                   double* total, double* parts) {
+    dfo_groups(B, vtx_off, vmask, N / 2, D, Q.time_alloc_method >= 3, [&](int p0, int p1) {
+      dfo_group_n<N>(D, p0, p1, vtx_off, vmask, vval, times, Q, ncon, con_dim, con_deriv, con_value, coef, vval_out, code, n_iter, total, parts);
+    });
+  }
+  // the workspaces of the linear solves of one group: methods 0, 1 one per candidate, 3, 4 one per problem (the initial solve)
+  struct DfoWorkspace {
+    const long long* off;
+    const long long* size;
+    double* ws;
+  };
+  template <int N>
+  void dfo_group_n(int D, int p0, int p1, const int* vtx_off, const uint8_t* vmask, const double* vval, double* times, const DfoParams& Q, int ncon,
+                   const int* con_dim, const int* con_deriv, const double* con_value, double* coef, double* vval_out, int* code, int* n_iter,
+                   double* total, double* parts) {
+    constexpr int H = N / 2, RS = gen::Rec<N>::kSize;
+    scratch_.reset();
+    const int G = p1 - p0, method = Q.time_alloc_method;
+    const bool with_free = method >= 3;
+    const size_t gv0 = (size_t)vtx_off[p0], gs0 = gv0 - (size_t)p0;
+    std::vector<int> vo(G + 1), so(G + 1);
+    for (int i = 0; i <= G; ++i) {
+      vo[i] = vtx_off[p0 + i] - (int)gv0;
+      so[i] = vo[i] - i;
+    }
+    const GenVertices gv = gen_vertices<N>(G, vo.data(), vmask + gv0);
+    Bare bb = bare_batch(G, so.data(), Q.derivative_to_optimize);
+    BatchPtrs& b = bb.b;
+    const int totS = b.totS, totV = b.totV;
+    b.vmask = scratch_.template alloc<uint8_t>(totV);
+    b.vval = scratch_.template alloc<double>((size_t)totV * H * TG_D);
+    b.vfree = scratch_.template alloc<int>(gv.vfree.size());
+    b.np = scratch_.template alloc<int>(G);
+    b.hbw = scratch_.template alloc<int>(G);
+    b.times = scratch_.template alloc<double>(totS);
+    b.coef = scratch_.template alloc<double>((size_t)totS * TG_D * N);
+    b.recs = scratch_.template alloc<double>((size_t)totS * 3 * RS);
+    be_.h2d(b.vmask, vmask + gv0, totV);
+    be_.h2d(b.vval, vval + gv0 * H * TG_D, sizeof(double) * (size_t)totV * H * TG_D);
+    be_.h2d(b.vfree, gv.vfree.data(), sizeof(int) * gv.vfree.size());
+    be_.h2d(b.np, gv.np.data(), sizeof(int) * G);
+    be_.h2d(b.hbw, gv.hbw.data(), sizeof(int) * G);
+    be_.h2d(b.times, times + gs0, sizeof(double) * totS);
+    // per-problem layout of the variables, candidates (2 n), candidate items and solve workspaces
+    std::vector<DfoProb> hp(G);
+    std::vector<long long> ws_off(G), ws_size(G);
+    size_t totN = 0, totCand = 0, totItems = 0;
+    long long ws_tot = 0;
+    for (int i = 0; i < G; ++i) {
+      DfoProb& P = hp[i];
+      std::memset(&P, 0, sizeof(P));
+      P.S = so[i + 1] - so[i];
+      P.n_free = gv.np[i];
+      P.n = with_free ? P.S + D * P.n_free : P.S;
+      P.s0 = so[i];
+      P.x0 = (int)totN;
+      P.c0 = (int)totCand;
+      P.i0 = (int)totItems;
+      totN += (size_t)P.n;
+      totCand += 2 * (size_t)P.n;
+      totItems += 2 * (size_t)P.n * (size_t)(with_free ? 2 : P.S);
+      ws_size[i] = (long long)gen::ws_doubles<N>(P.S, gv.np[i], gv.hbw[i]);
+      ws_off[i] = ws_tot;
+      ws_tot += ws_size[i] * (with_free ? 1 : 2 * P.n);
+    }
+    DfoBatch d;
+    std::memset(&d, 0, sizeof(d));
+    d.prob = scratch_.template alloc<DfoProb>(G);
+    be_.h2d(d.prob, hp.data(), sizeof(DfoProb) * G);
+    d.method = method;
+    d.max_iter = Q.max_iterations;
+    d.ipc_free = 2;
+    d.f_rel = Q.f_rel;
+    d.x_rel = Q.x_rel;
+    d.step_rel = Q.initial_stepsize_rel;
+    d.obj = obj_terms(method, Q.time_penalty, Q.use_soft_constraints, Q.soft_constraint_weight, ncon, con_deriv, con_value);
+    for (int c = 0; c < ncon; ++c) d.con_dim[c] = con_dim[c];
+    d.x = scratch_.template alloc<double>(totN);
+    d.lo = scratch_.template alloc<double>(totN);
+    d.hi = scratch_.template alloc<double>(totN);
+    d.step = scratch_.template alloc<double>(totN);
+    d.cand_prob = scratch_.template alloc<int>(totCand);
+    d.item_cand = with_free ? nullptr : scratch_.template alloc<int>(totItems);
+    d.ctot = scratch_.template alloc<double>(totCand);
+    d.ccost = with_free ? nullptr : scratch_.template alloc<double>(totCand);
+    d.ccoef = scratch_.template alloc<double>(totItems * TG_D * N);
+    d.cpart = with_free ? scratch_.template alloc<double>(totItems * 4) : nullptr;
+    bool need[4] = {false, false, false, false};
+    for (int c = 0; c < ncon; ++c) need[con_deriv[c] - 1] = Q.use_soft_constraints != 0;
+    d.csv = scratch_.template alloc<double>(4 * totItems);
+    d.bcost = scratch_.template alloc<double>(G);
+    d.bpart = scratch_.template alloc<double>((size_t)totS * 4);
+    d.bsv = scratch_.template alloc<double>((size_t)4 * totS);
+    d.btot = scratch_.template alloc<double>(G);
+    d.bparts = scratch_.template alloc<double>((size_t)3 * G);
+    d.totS = (size_t)totS;
+    d.totItems = totItems;
+    for (int k = 0; k < 2; ++k) {
+      d.lists[k][0] = scratch_.template alloc<int>(G);
+      d.lists[k][1] = scratch_.template alloc<int>(totS);
+      d.lists[k][2] = scratch_.template alloc<int>(totCand);
+      d.lists[k][3] = scratch_.template alloc<int>(totItems);
+    }
+    d.cnt = scratch_.template alloc<int>(9);
+    d.b = b;
+    long long* d_ws_off = scratch_.template alloc<long long>(G);
+    long long* d_ws_size = scratch_.template alloc<long long>(G);
+    be_.h2d(d_ws_off, ws_off.data(), sizeof(long long) * G);
+    be_.h2d(d_ws_size, ws_size.data(), sizeof(long long) * G);
+    const DfoWorkspace ws{d_ws_off, d_ws_size, scratch_.template alloc<double>((size_t)std::max<long long>(ws_tot, 1))};
+    be_.for_each(G, DfoMapFn{d});
+    launches(1);
+    if (with_free) {  // x0 of the free derivatives: the linear solution at the initial times (solveLinear + getFreeConstraints)
+      int* d_vo = scratch_.template alloc<int>((size_t)G + 1);
+      be_.h2d(d_vo, vo.data(), sizeof(int) * ((size_t)G + 1));
+      double* recs0 = scratch_.template alloc<double>((size_t)totS * RS);
+      be_.for_each((size_t)totS, gen::RecordHeadFn<N>{b.r, b.times, recs0});
+      be_.for_each((size_t)totS * N, gen::RecordHrowFn<N>{recs0});
+      be_.for_each_warp((size_t)G, gen::SolveFn<N>{b.r, d_vo, b.vmask, b.vfree, b.vval, b.np, b.hbw, recs0, ws.off, ws.ws, b.coef, d.bcost});
+      be_.for_each(totV, gen::DfoFreeInitFn<N>{d, D});
+      launches(4);
+      counters.solves += G;
+      counters.segment_setups += totS;
+    }
+    be_.for_each(G, DfoBeginFn{d});
+    be_.dev_memset(d.cnt, 0, 9 * sizeof(int));
+    launches(1);
+    dfo_base_eval_n<N>(d, D, ws, need, 1);
+    int back[5];
+    be_.d2h(back, d.cnt, sizeof(back));
+    for (int it = 0; it < Q.max_iterations && back[0] > 0; ++it) {
+      const int buf = it & 1, nbuf = buf ^ 1;
+      const bool sparse = (size_t)back[0] * 2 < (size_t)G;
+      const int* const* L = sparse ? d.lists[buf] : nullptr;
+      const size_t nprob = sparse ? (size_t)back[1] : (size_t)G, nseg = sparse ? (size_t)back[2] : (size_t)totS;
+      const size_t ncand = sparse ? (size_t)back[3] : totCand, nitem = sparse ? (size_t)back[4] : totItems;
+      be_.dev_memset(d.cnt, 0, sizeof(int));
+      be_.dev_memset(d.cnt + 1 + 4 * nbuf, 0, 4 * sizeof(int));
+      be_.for_each(nseg * 3, gen::DfoHeadFn<N>{d, L ? L[1] : nullptr, 3, 0});
+      launches(1);
+      if (with_free) {
+        be_.for_each(nseg * 4, gen::DfoBaseCoefFn<N>{d, L ? L[1] : nullptr, 0, D});
+        dfo_maxima_n<N>(d, need, L ? L[1] : nullptr, nseg, 1, 0);
+        be_.for_each(nitem, gen::DfoItemFn<N>{d, L ? L[3] : nullptr, D});
+        launches(2);
+      } else {
+        be_.for_each(nseg * 3 * N, gen::DfoHrowFn<N>{d, L ? L[1] : nullptr, 3, 0});
+        be_.for_each_warp(ncand, gen::DfoSolveFn<N>{d, 0, L ? L[2] : nullptr, ws.off, ws.size, ws.ws});
+        launches(2);
+      }
+      dfo_maxima_n<N>(d, need, L ? L[3] : nullptr, nitem, 0, 0);
+      be_.for_each(ncand, DfoTotalFn{d, L ? L[2] : nullptr});
+      be_.for_each(nprob, DfoAdvanceFn{d, L ? L[0] : nullptr, nbuf});
+      launches(2);
+      counters.segment_setups += (long long)back[2] * 3;
+      counters.evals += (long long)back[3];
+      if (!with_free) counters.solves += back[3];
+      for (int k = 0; k < 4; ++k)
+        if (need[k]) {
+          counters.root_finds += (long long)back[4] + (with_free ? back[2] : 0);
+          counters.root_finds_executed += (long long)back[4] + (with_free ? back[2] : 0);
+        }
+      int nb[5];
+      be_.d2h(nb, d.cnt, sizeof(int));
+      be_.d2h(nb + 1, d.cnt + 1 + 4 * nbuf, 4 * sizeof(int));
+      std::memcpy(back, nb, sizeof(back));
+    }
+    dfo_base_eval_n<N>(d, D, ws, need, 0);  // the final point, with coefficients and the three terms
+    double* d_times = scratch_.template alloc<double>(totS);
+    be_.for_each(totS, DfoTimesOutFn{d, d_times});
+    launches(1);
+    be_.d2h(times + gs0, d_times, sizeof(double) * totS);
+    if (coef) be_.d2h(coef + gs0 * TG_D * N, b.coef, sizeof(double) * (size_t)totS * TG_D * N);
+    if (vval_out && with_free) {
+      double* d_vv = scratch_.template alloc<double>((size_t)totV * H * TG_D);
+      be_.for_each(totV, gen::DfoVvalOutFn<N>{d, D, d_vv});
+      launches(1);
+      be_.d2h(vval_out + gv0 * H * TG_D, d_vv, sizeof(double) * (size_t)totV * H * TG_D);
+    }
+    be_.d2h(hp.data(), d.prob, sizeof(DfoProb) * G);
+    for (int i = 0; i < G; ++i) {
+      if (code) code[p0 + i] = hp[i].code;
+      if (n_iter) n_iter[p0 + i] = hp[i].iterations;
+      if (total) total[p0 + i] = hp[i].f;
+    }
+    if (parts) be_.d2h(parts + 3 * (size_t)p0, d.bparts, sizeof(double) * 3 * G);
+  }
+  // dfo_base_eval over N coefficients
+  template <int N>
+  void dfo_base_eval_n(const DfoBatch& d, int D, const DfoWorkspace& ws, const bool* need, int start) {
+    const int G = d.b.B, totS = d.b.totS;
+    be_.for_each((size_t)totS, gen::DfoHeadFn<N>{d, nullptr, 1, 1});
+    if (d.method >= 3) {
+      be_.for_each((size_t)totS * 4, gen::DfoBaseCoefFn<N>{d, nullptr, 1, D});
+    } else {
+      be_.for_each((size_t)totS * N, gen::DfoHrowFn<N>{d, nullptr, 1, 1});
+      be_.for_each_warp((size_t)G, gen::DfoSolveFn<N>{d, 1, nullptr, ws.off, ws.size, ws.ws});
+      launches(1);
+      counters.solves += G;
+    }
+    dfo_maxima_n<N>(d, need, nullptr, (size_t)totS, 1, 1);
+    be_.for_each((size_t)G, DfoBaseTotalFn{d, start});
+    launches(3);
+    counters.segment_setups += totS;
+    counters.evals += G;
+  }
+  template <int N>
+  void dfo_maxima_n(const DfoBatch& d, const bool* need, const int* list, size_t n, int base, int all) {
+    for (int k = 0; k < 4; ++k) {
+      if (!need[k] || n == 0) continue;
+      switch (k + 1) {
+        case 1: be_.for_each_scratch(n, gen::DfoMaxFn<N, 1>{d, list, base, all}); break;
+        case 2: be_.for_each_scratch(n, gen::DfoMaxFn<N, 2>{d, list, base, all}); break;
+        case 3: be_.for_each_scratch(n, gen::DfoMaxFn<N, 3>{d, list, base, all}); break;
+        default: be_.for_each_scratch(n, gen::DfoMaxFn<N, 4>{d, list, base, all}); break;
+      }
+      launches(1);
+      if (base && all) {
+        counters.root_finds += (long long)n;
+        counters.root_finds_executed += (long long)n;
+      }
+    }
   }
 
   size_t objective_chunk = (size_t)1 << 15;
