@@ -7,6 +7,7 @@
 //   eth_trajectory_generation::NonlinearOptimizationParameters nl.h:35-110
 //   eth_trajectory_generation::PolynomialOptimizationNonLinear<N>  nl.h:147-197
 //   eth_trajectory_generation::sampleWholeTrajectory           eth/trajectory_sampling.h:44
+//   eth_trajectory_generation::sampleTrajectoryInRange / sampleTrajectoryStartDuration  eth/trajectory_sampling.cpp:49-104, eth/trajectory_sampling.h
 // Same method names, argument meaning and error behaviour (bool returns, print-and-continue -- eth/misc.h:6-38 -- and the
 // NLopt-style int of optimize()).  Every method marshals into the C ABI of include/tg_b200.h, i.e. into the sm_100a
 // kernels of libtg_b200.so; one object = a batch of one.  There is no CPU arithmetic here and no fallback: constructing
@@ -21,7 +22,7 @@
 // own struct when that header is included, or the plain TrajectoryPoint below.
 //
 // Additions that the one-problem-per-object reference API cannot express: TrajectoryGeneratorBatch (the numeric core of
-// optimize()/findTrajectory for many paths in one call, SURVEY.md H7).
+// optimize()/findTrajectory for many paths in one call, SURVEY.md H7) and sampleTrajectoriesInRange (many windows in one call).
 #ifndef ETH_TRAJECTORY_GENERATION_B200_HPP_
 #define ETH_TRAJECTORY_GENERATION_B200_HPP_
 
@@ -354,40 +355,43 @@ inline typename std::enable_if<!has_set_from_yaw<P>::value>::type fill_heading(P
 }
 }  // namespace b200
 
-// sampleWholeTrajectory (eth/trajectory_sampling.cpp:119-124 -> 49-104).  PointVector: std::vector of TrajectoryPoint, or of
-// the reference's eth_mav_msgs::EigenTrajectoryPoint (any allocator) -- same call as in the reference (node.cpp:1166).
-template <class PointVector>
-inline bool sampleWholeTrajectory(const Trajectory& trajectory, double sampling_interval, PointVector* states) {
-  if (!states) return false;
-  states->clear();
-  if (trajectory.empty() || !(sampling_interval > 0.0)) {
-    std::printf("[sampleWholeTrajectory]: empty trajectory or non-positive sampling interval\n");
-    return false;
-  }
-  if (trajectory.D() < 3) {
-    std::printf("[sampleWholeTrajectory]: Dimension has to be at least 3, but is %d\n", trajectory.D());  // eth/trajectory_sampling.cpp:58-61
-    return false;
-  }
+namespace b200 {
+// The windowed walk of tg_sample_range_batch_nd for trajectories of one shape, window p = [t_range[2p], t_range[2p+1]]: one counting
+// call and one call for the rows (p4 v4 a4 j3 s3 yaw, time_from_start_ns), compacted in trajectory order.
+inline void sample_ranges(const std::vector<const Trajectory*>& trajs, const double* t_range, double dt, std::vector<int>* counts,
+                          std::vector<double>* full, std::vector<long long>* t_ns) {
+  const int B = (int)trajs.size(), n_coef = trajs.front()->N(), dims = trajs.front()->D();
+  std::vector<int> seg_off(1, 0);
   std::vector<double> coef, times;
-  trajectory.pack(&coef, &times);
-  const int seg_off[2] = {0, trajectory.K()};
-  const int n_coef = trajectory.N(), dims = trajectory.D();
-  const bool tuned = trajectory.tunedShape();
-  int count = 0;
-  b200::Context& c = b200::Context::instance();
-  auto sample = [&](double* xyzh, double* full) {
-    if (tuned) c.check(tg_sample_batch(c.get(), 1, seg_off, coef.data(), times.data(), sampling_interval, &count, xyzh, full), "tg_sample_batch");
-    else c.check(tg_sample_batch_nd(c.get(), n_coef, dims, 1, seg_off, coef.data(), times.data(), sampling_interval, &count, xyzh, full), "tg_sample_batch_nd");
-  };
-  sample(nullptr, nullptr);
-  if (count <= 0) return false;
-  std::vector<double> xyzh((size_t)count * 4), full((size_t)count * 19);
-  sample(xyzh.data(), full.data());
+  for (const Trajectory* t : trajs) {
+    std::vector<double> c, T;
+    t->pack(&c, &T);
+    coef.insert(coef.end(), c.begin(), c.end());
+    times.insert(times.end(), T.begin(), T.end());
+    seg_off.push_back(seg_off.back() + t->K());
+  }
+  counts->assign(B, 0);
+  Context& c = Context::instance();
+  c.check(tg_sample_range_batch_nd(c.get(), n_coef, dims, B, seg_off.data(), coef.data(), times.data(), t_range, dt, counts->data(), nullptr,
+                                   nullptr, nullptr),
+          "tg_sample_range_batch_nd");
+  size_t rows = 0;
+  for (int n : *counts) rows += (size_t)n;
+  full->resize(rows * 19);
+  t_ns->resize(rows);
+  if (rows)
+    c.check(tg_sample_range_batch_nd(c.get(), n_coef, dims, B, seg_off.data(), coef.data(), times.data(), t_range, dt, counts->data(), nullptr,
+                                     full->data(), t_ns->data()),
+            "tg_sample_range_batch_nd");
+}
+// rows -> the fields of EigenTrajectoryPoint the sampler fills (eth/trajectory_sampling.cpp:73-103)
+template <class PointVector>
+inline void fill_points(int dims, const double* full, const long long* t_ns, int count, PointVector* states) {
   states->resize(count);
   for (int i = 0; i < count; ++i) {
     auto& s = (*states)[i];
-    const double* f = &full[(size_t)i * 19];  // p4 v4 a4 j3 s3 yaw
-    s.time_from_start_ns = (int64_t)((0.0 + sampling_interval * (double)i) * 1.e9);  // eth/trajectory_sampling.cpp:98
+    const double* f = full + (size_t)i * 19;  // p4 v4 a4 j3 s3 yaw
+    s.time_from_start_ns = (int64_t)t_ns[i];  // (min_time + dt * i) * 1e9, eth/trajectory_sampling.cpp:98
     for (int k = 0; k < 3; ++k) {
       s.position_W[k] = f[k];
       s.velocity_W[k] = f[4 + k];
@@ -395,71 +399,124 @@ inline bool sampleWholeTrajectory(const Trajectory& trajectory, double sampling_
       s.jerk_W[k] = f[12 + k];
       s.snap_W[k] = f[15 + k];
     }
-    if (dims == 4) b200::fill_heading(s, f);  // eth/trajectory_sampling.cpp:99-103: only a 4-dimensional trajectory sets the yaw
+    if (dims == 4) fill_heading(s, f);  // eth/trajectory_sampling.cpp:99-103: only a 4-dimensional trajectory sets the yaw
+  }
+}
+inline bool sampling_refused(const char* who, const Trajectory& trajectory, double sampling_interval) {
+  if (trajectory.empty() || !(sampling_interval > 0.0)) {
+    std::printf("[%s]: empty trajectory or non-positive sampling interval\n", who);
+    return true;
+  }
+  if (trajectory.D() < 3) {
+    std::printf("[%s]: Dimension has to be at least 3, but is %d\n", who, trajectory.D());  // eth/trajectory_sampling.cpp:58-61
+    return true;
+  }
+  return false;
+}
+}  // namespace b200
+
+// sampleTrajectoryInRange (eth/trajectory_sampling.cpp:49-104).  PointVector: std::vector of TrajectoryPoint, or of the reference's
+// eth_mav_msgs::EigenTrajectoryPoint (any allocator).  As upstream, a window outside [getMinTime(), getMaxTime()] is refused (false,
+// no states); inside it the samples are evaluateRange's walk (DESIGN.md §4.3), which may return no state.  One device call.
+template <class PointVector>
+inline bool sampleTrajectoryInRange(const Trajectory& trajectory, double min_time, double max_time, double sampling_interval, PointVector* states) {
+  if (!states) return false;
+  states->clear();
+  if (b200::sampling_refused("sampleTrajectoryInRange", trajectory, sampling_interval)) return false;
+  if (!(min_time >= trajectory.getMinTime() && max_time <= trajectory.getMaxTime())) {
+    std::printf("[sampleTrajectoryInRange]: Sample time should be within [%g %g] but is [%g %g]\n", trajectory.getMinTime(), trajectory.getMaxTime(),
+                min_time, max_time);
+    return false;
+  }
+  const double t_range[2] = {min_time, max_time};
+  std::vector<int> counts;
+  std::vector<double> full;
+  std::vector<long long> t_ns;
+  b200::sample_ranges({&trajectory}, t_range, sampling_interval, &counts, &full, &t_ns);
+  b200::fill_points(trajectory.D(), full.data(), t_ns.data(), counts[0], states);
+  return true;
+}
+// sampleTrajectoryStartDuration: sampleTrajectoryInRange over [start_time, start_time + duration]
+template <class PointVector>
+inline bool sampleTrajectoryStartDuration(const Trajectory& trajectory, double start_time, double duration, double sampling_interval,
+                                          PointVector* states) {
+  return sampleTrajectoryInRange(trajectory, start_time, start_time + duration, sampling_interval, states);
+}
+// sampleWholeTrajectory (eth/trajectory_sampling.cpp:119-124): sampleTrajectoryInRange over [getMinTime(), getMaxTime()], false when
+// that gives no sample (a trajectory of zero duration) -- same call as in the reference (node.cpp:1166).
+template <class PointVector>
+inline bool sampleWholeTrajectory(const Trajectory& trajectory, double sampling_interval, PointVector* states) {
+  if (!states) return false;
+  return sampleTrajectoryInRange(trajectory, trajectory.getMinTime(), trajectory.getMaxTime(), sampling_interval, states) && !states->empty();
+}
+// Not a reference name: sampleTrajectoryInRange's walk for many trajectories of one shape in one device call, window i = windows[i] =
+// {min_time, max_time}, states_per_trajectory[i] filled as sampleTrajectoryInRange fills its states.  It applies no range check: a
+// window running past a trajectory's end stops at that end, as "the next H seconds" of a trajectory near its end should.  false, with
+// nothing filled, for an empty list, mismatched sizes or shapes, or what sampleTrajectoryInRange refuses for any trajectory.
+template <class PointVector>
+inline bool sampleTrajectoriesInRange(const std::vector<Trajectory>& trajectories, const std::vector<std::pair<double, double>>& windows,
+                                      double sampling_interval, std::vector<PointVector>* states_per_trajectory) {
+  if (!states_per_trajectory) return false;
+  states_per_trajectory->clear();
+  if (trajectories.empty() || windows.size() != trajectories.size()) {
+    std::printf("[sampleTrajectoriesInRange]: one window per trajectory is needed\n");
+    return false;
+  }
+  std::vector<const Trajectory*> trajs;
+  std::vector<double> t_range;
+  for (size_t i = 0; i < trajectories.size(); ++i) {
+    const Trajectory& t = trajectories[i];
+    if (b200::sampling_refused("sampleTrajectoriesInRange", t, sampling_interval)) return false;
+    if (t.N() != trajectories.front().N() || t.D() != trajectories.front().D()) {
+      std::printf("[sampleTrajectoriesInRange]: every trajectory must have the same shape\n");
+      return false;
+    }
+    trajs.push_back(&t);
+    t_range.push_back(windows[i].first);
+    t_range.push_back(windows[i].second);
+  }
+  std::vector<int> counts;
+  std::vector<double> full;
+  std::vector<long long> t_ns;
+  b200::sample_ranges(trajs, t_range.data(), sampling_interval, &counts, &full, &t_ns);
+  states_per_trajectory->resize(trajs.size());
+  size_t row = 0;
+  for (size_t i = 0; i < trajs.size(); ++i) {
+    b200::fill_points(trajs[i]->D(), full.data() + row * 19, t_ns.data() + row, counts[i], &(*states_per_trajectory)[i]);
+    row += (size_t)counts[i];
   }
   return true;
 }
 
 inline void Trajectory::evaluateRange(double t_start, double t_end, double dt, int derivative, std::vector<Vector>* result,
                                       std::vector<double>* sampling_times) const {
-  // eth/trajectory.cpp:93-151: the accumulated walk t_start, t_start + dt, ... (< t_end), every sample evaluated in ALL
-  // dimensions for any derivative 0..N-1 on the device (tg_evaluate_batch); out-of-range start: prints and returns nothing
+  // eth/trajectory.cpp:93-151 in one device call (tg_evaluate_range_batch_nd): the walk from the start of the segment holding t_start
+  // while the accumulated time is below t_end, derivative `derivative` of every dimension; a start past the end prints and returns
+  // nothing
   if (!result) return;
   result->clear();
   if (sampling_times) sampling_times->clear();
   if (segments_.empty() || !(dt > 0.0)) return;
-  if (t_start > getMaxTime() || t_start < 0.0) {
-    std::printf("[Trajectory]: start time out of range of the trajectory!\n");
-    return;
-  }
-  // the reference keeps two running sums, accumulated_time and time_in_segment, and evaluates segment i at time_in_segment
-  std::vector<double> ts;
-  std::vector<int> seg_of;
-  double acc = 0.0;
-  size_t i = 0;
-  for (i = 0; i < segments_.size(); ++i) {
-    acc += segments_[i].getTime();
-    if (acc > t_start) break;
-  }
-  if (i >= segments_.size()) i = segments_.size() - 1;
-  acc -= segments_[i].getTime();
-  double in_seg = t_start - acc;
-  while (acc < t_end) {
-    if (in_seg > segments_[i].getTime()) {
-      in_seg = in_seg - segments_[i].getTime();
-      if (++i >= segments_.size()) break;
-      continue;
-    }
-    ts.push_back(in_seg);
-    seg_of.push_back((int)i);
-    if (sampling_times) sampling_times->push_back(acc);
-    in_seg += dt;
-    acc += dt;
-  }
-  if (ts.empty()) return;
+  if (t_start > getMaxTime()) std::printf("[Trajectory]: start time out of range of the trajectory!\n");
+  std::vector<double> coef, times;
+  pack(&coef, &times);
+  const int seg_off[2] = {0, K()};
+  const double t_range[2] = {t_start, t_end};
   const int dims = D();
-  std::vector<double> out(ts.size() * (size_t)dims);
-  std::vector<uint8_t> ok(ts.size());
+  int count = 0;
   b200::Context& c = b200::Context::instance();
-  const bool tuned = tunedShape();
-  // one device call per run of samples that fall into the same segment: that segment alone, evaluated at time_in_segment
-  for (size_t k0 = 0; k0 < ts.size();) {
-    size_t k1 = k0;
-    while (k1 < ts.size() && seg_of[k1] == seg_of[k0]) ++k1;
-    const Segment& sg = segments_[seg_of[k0]];
-    const double T = sg.getTime();
-    if (tuned)
-      c.check(tg_evaluate_batch(c.get(), 1, sg.data(), &T, (int)(k1 - k0), ts.data() + k0, derivative, out.data() + k0 * dims, ok.data() + k0), "tg_evaluate_batch");
-    else
-      c.check(tg_evaluate_batch_nd(c.get(), N(), dims, 1, sg.data(), &T, (int)(k1 - k0), ts.data() + k0, derivative, out.data() + k0 * dims, ok.data() + k0),
-              "tg_evaluate_batch_nd");
-    k0 = k1;
-  }
-  for (size_t k = 0; k < ts.size(); ++k) {
+  c.check(tg_evaluate_range_batch_nd(c.get(), N(), dims, 1, seg_off, coef.data(), times.data(), t_range, dt, derivative, &count, nullptr, nullptr),
+          "tg_evaluate_range_batch_nd");
+  if (count == 0) return;
+  std::vector<double> out((size_t)count * dims), st(count);
+  c.check(tg_evaluate_range_batch_nd(c.get(), N(), dims, 1, seg_off, coef.data(), times.data(), t_range, dt, derivative, &count, out.data(), st.data()),
+          "tg_evaluate_range_batch_nd");
+  for (int k = 0; k < count; ++k) {
     Vector v = b200::make_vector((size_t)dims, 0.0);
-    for (int d = 0; d < dims; ++d) v[d] = out[k * dims + d];
+    for (int d = 0; d < dims; ++d) v[d] = out[(size_t)k * dims + d];
     result->push_back(v);
   }
+  if (sampling_times) sampling_times->assign(st.begin(), st.end());
 }
 
 // ---- vertex marshalling ------------------------------------------------------------------------------------------------

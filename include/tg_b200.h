@@ -177,6 +177,29 @@ int tg_evaluate_batch_nd(tg_ctx* ctx, int N, int D, int S, const double* coef, c
                          double* out, uint8_t* ok);
 int tg_sample_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times, double dt, int* counts,
                        double* samples, double* full);
+/* Sampling and evaluation over a time window per trajectory, shapes as above (coef[totS][D][N]), window p = [t_range[2p], t_range[2p+1]].
+ *   The reference's walk (eth/trajectory.cpp:93-151): accumulated_time starts at the START of the segment holding t_start, samples are
+ *   taken while accumulated_time < t_end, the segment switch is a strict '>' with the time in segment updated by subtraction, and the
+ *   walk ends when it passes the last segment.  So a window starting mid-segment gives more than (t_end - t_start) / dt samples,
+ *   t_end < t_start can give samples, and a window running past the end (t_end = +inf included) stops at the end.  No segment with
+ *   an accumulated time above t_start (t_start >= the end, or only zero-length segments after it) and a NaN window end give 0
+ *   samples.  A negative t_start extrapolates segment 0 to negative times, as the walk does.
+ *   Two-call convention: with every output NULL only counts[B] is filled.  Rows are compacted in trajectory order.
+ * tg_sample_range_batch_nd = the walk of sampleTrajectoryInRange (eth/trajectory_sampling.cpp:49-104) without its range check:
+ *   samples[sum counts][4] (x y z heading), full[sum counts][19] = p4 v4 a4 j3 s3 yaw as tg_sample_batch_nd, and
+ *   t_ns = time_from_start_ns = int64((t_start + dt * k) * 1e9) of sample k (trajectory_sampling.cpp:98), any of them NULL.
+ *   [0, total time] gives tg_sample_batch_nd's rows.
+ * tg_evaluate_range_batch_nd = Trajectory::evaluateRange (eth/trajectory.cpp:93-151): out[sum counts][D] = derivative `derivative`
+ *   of the D dimensions (zeros for derivative >= N, as Trajectory::evaluate gives), sampling_times[sum counts] = the accumulated
+ *   times, either NULL.
+ *   Both refuse with TG_ERR_INVALID, writing no output: N outside {6, 8, 10, 12}, D outside 1..4 (D < 3 for the sampler, as
+ *   eth/trajectory_sampling.cpp:58-61), dt not > 0, a negative derivative, B < 1, a NULL input or a decreasing seg_off.  A window
+ *   whose sample count passes its bound (min(t_end - segment start, end - t_start) / dt + 4, or more than INT_MAX rows in all)
+ *   fails with TG_ERR_CAPACITY, writing no output: a window is never returned short. */
+int tg_sample_range_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times,
+                             const double* t_range, double dt, int* counts, double* samples, double* full, long long* t_ns);
+int tg_evaluate_range_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times,
+                               const double* t_range, double dt, int derivative, int* counts, double* out, double* sampling_times);
 /* Free and fixed constraints of PolynomialOptimization<N> (lin_impl.h:183-257, 513-522) on the same shapes, inputs as in
  *   tg_solve_linear_batch_nd.  The free derivatives d_p of a problem are dimension-major: D vectors of n_free entries, and within a
  *   dimension vertex-major with the derivative ascending; n_free = the clear mask bits below N/2 over the problem's vertices,

@@ -18,6 +18,9 @@ from .api import (  # noqa: F401
     NonlinearOptimizationParameters,
     Trajectory,
     sample_whole_trajectory,
+    sample_trajectory_in_range,
+    sample_trajectory_start_duration,
+    sample_trajectories_in_range,
     TrajectoryGenerator,
     derivative_order,
 )

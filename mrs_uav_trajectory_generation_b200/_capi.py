@@ -143,6 +143,8 @@ class Library:
         L.tg_set_free_constraints_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _u8p, _dp, _dp, C.c_int, _dp, _dp, _dp]
         L.tg_evaluate_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, C.c_int, _dp, C.c_int, _dp, _u8p]
         L.tg_sample_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_double, _ip, _dp, _dp]
+        L.tg_sample_range_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, C.c_double, _ip, _dp, _dp, _llp]
+        L.tg_evaluate_range_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, C.c_double, C.c_int, _ip, _dp, _dp]
         L.tg_extrema_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _dp, _dp, _dp]
         L.tg_max_magnitude_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
         L.tg_scale_times_batch_nd.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, _ip, _dp, _dp, _dp, _ip, _u8p]
@@ -557,6 +559,42 @@ class Context:
         self._check(lib.tg_sample_batch_nd(self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), float(dt), _p(counts, _ip),
                                            _p(samples), _p(fullv)))
         return counts, samples, fullv
+
+    def _range_inputs(self, n_coef, dim, seg_off, coef, times, t_range):
+        seg_off = np.ascontiguousarray(seg_off, dtype=np.int32)
+        coef = np.ascontiguousarray(coef, dtype=np.float64)
+        times = np.ascontiguousarray(times, dtype=np.float64)
+        t_range = np.ascontiguousarray(t_range, dtype=np.float64).reshape(-1, 2)
+        B = len(seg_off) - 1
+        assert coef.size == int(seg_off[-1]) * dim * n_coef and t_range.shape[0] == B
+        return seg_off, coef, times, t_range, B
+
+    def sample_range_batch_nd(self, n_coef, dim, seg_off, coef, times, t_range, dt, full=False):
+        """sampleTrajectoryInRange's walk over window p = t_range[p] = (t_start, t_end) of every trajectory (tg_sample_range_batch_nd):
+        counts [B], samples [sum][4] (x y z heading), full [sum][19] or None, t_ns [sum] (time_from_start_ns), rows in trajectory order."""
+        seg_off, coef, times, t_range, B = self._range_inputs(n_coef, dim, seg_off, coef, times, t_range)
+        counts = np.zeros(B, dtype=np.int32)
+        lib = self.L.lib
+        args = (self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), _p(t_range), float(dt), _p(counts, _ip))
+        self._check(lib.tg_sample_range_batch_nd(*args, None, None, None))
+        tot = int(counts.sum())
+        samples, t_ns = np.empty((tot, 4)), np.empty(tot, dtype=np.int64)
+        fullv = np.empty((tot, 19)) if full else None
+        self._check(lib.tg_sample_range_batch_nd(*args, _p(samples), _p(fullv), _p(t_ns, _llp)))
+        return counts, samples, fullv, t_ns
+
+    def evaluate_range_batch_nd(self, n_coef, dim, seg_off, coef, times, t_range, dt, derivative=0):
+        """Trajectory::evaluateRange over window p = t_range[p] of every trajectory (tg_evaluate_range_batch_nd): counts [B],
+        values [sum][dim] of the derivative, sampling_times [sum], rows in trajectory order."""
+        seg_off, coef, times, t_range, B = self._range_inputs(n_coef, dim, seg_off, coef, times, t_range)
+        counts = np.zeros(B, dtype=np.int32)
+        lib = self.L.lib
+        args = (self.h, int(n_coef), int(dim), B, _p(seg_off, _ip), _p(coef), _p(times), _p(t_range), float(dt), int(derivative), _p(counts, _ip))
+        self._check(lib.tg_evaluate_range_batch_nd(*args, None, None))
+        tot = int(counts.sum())
+        out, st = np.empty((tot, dim)), np.empty(tot)
+        self._check(lib.tg_evaluate_range_batch_nd(*args, _p(out), _p(st)))
+        return counts, out, st
 
     def extrema_nd(self, n_coef, dim, coef, times):
         """Nine maxima per segment of N-coefficient, D-dimensional segments: coef [totS][dim][n_coef] -> maxima [totS][9]."""

@@ -137,6 +137,16 @@ class Trajectory:
             out, ok = self._c().evaluate_nd(n, d, self.coef, self.times, t, derivative)
         return out[0] if np.isscalar(t) else out
 
+    def evaluateRange(self, t_start, t_end, dt, derivative=derivative_order.POSITION):
+        """Trajectory::evaluateRange (eth/trajectory.cpp:93-151) in one device call: (values [M, D], sampling_times [M]).  The walk starts
+        at the start of the segment holding t_start and runs while the accumulated time is below t_end (DESIGN.md §4.3)."""
+        d, n = self.shape()
+        if self.K() == 0:
+            return np.zeros((0, d)), np.zeros(0)
+        seg_off = np.array([0, self.K()], dtype=np.int32)
+        _, out, st = self._c().evaluate_range_batch_nd(n, d, seg_off, self.coef, self.times, [[t_start, t_end]], dt, derivative)
+        return out, st
+
     def computeMaxDerivatives(self):
         """Per-segment maxima [S, 9] = hor v,a,j ; ver v,a,j ; heading v,a,j (eth/trajectory.cpp:422-565)."""
         if self._tuned():
@@ -166,6 +176,38 @@ def sample_whole_trajectory(trajectory, dt, full=False, ctx=None):
         d, n = trajectory.shape()
         counts, samples, fullv = c.sample_batch_nd(n, d, seg_off, trajectory.coef, trajectory.times, dt, full=full)
     return fullv if full else samples
+
+
+def sample_trajectories_in_range(trajectories, windows, dt, full=False, ctx=None):
+    """sampleTrajectoryInRange's walk for many trajectories of one shape in one device call (not a reference name), window i =
+    windows[i] = (min_time, max_time).  No range check: a window running past a trajectory's end stops at that end.
+    Returns counts [B], rows [sum counts, 4] (x, y, z, heading) or, with full=True, [sum counts, 19] = p4 v4 a4 j3 s3 yaw, and
+    time_from_start_ns [sum counts]; the rows of trajectory i follow those of trajectory i - 1."""
+    trajectories = list(trajectories)
+    shapes = {t.shape() for t in trajectories}
+    if len(shapes) != 1 or len(windows) != len(trajectories):
+        raise ValueError("one window per trajectory, every trajectory of the same shape")
+    d, n = shapes.pop()
+    seg_off = np.zeros(len(trajectories) + 1, dtype=np.int32)
+    seg_off[1:] = np.cumsum([t.K() for t in trajectories])
+    coef = np.concatenate([t.coef.reshape(-1) for t in trajectories])
+    times = np.concatenate([t.times for t in trajectories])
+    c = ctx or trajectories[0]._c()
+    counts, samples, fullv, t_ns = c.sample_range_batch_nd(n, d, seg_off, coef, times, np.asarray(windows, dtype=np.float64), dt, full=full)
+    return counts, (fullv if full else samples), t_ns
+
+
+def sample_trajectory_in_range(trajectory, min_time, max_time, dt, full=False, ctx=None):
+    """eth_trajectory_generation::sampleTrajectoryInRange (eth/trajectory_sampling.cpp:49-104): samples [M, 4] or, with full=True,
+    [M, 19] as sample_whole_trajectory.  None, as the reference's false, for a window outside [getMinTime(), getMaxTime()]."""
+    if not (min_time >= trajectory.getMinTime() and max_time <= trajectory.getMaxTime()):
+        return None
+    return sample_trajectories_in_range([trajectory], [(min_time, max_time)], dt, full=full, ctx=ctx)[1]
+
+
+def sample_trajectory_start_duration(trajectory, start_time, duration, dt, full=False, ctx=None):
+    """sampleTrajectoryStartDuration: sample_trajectory_in_range over [start_time, start_time + duration]."""
+    return sample_trajectory_in_range(trajectory, start_time, start_time + duration, dt, full=full, ctx=ctx)
 
 
 class PolynomialOptimization:

@@ -461,6 +461,56 @@ int tg_sample_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, con
   });
 }
 
+namespace {
+// the refusals shared by the windowed entry points; an empty string accepts
+inline const char* tg_range_refusal(int N, int D, int B, const int* seg_off, const double* coef, const double* times, const double* t_range,
+                                    double dt, const int* counts) {
+  if (!tg_shape_ok(N, D)) return "supported shapes: N in {6, 8, 10, 12}, D in 1..4";
+  if (B < 1 || !seg_off || !coef || !times || !t_range || !counts || !(dt > 0.0)) return "invalid argument";
+  if (seg_off[0] != 0) return "seg_off[0] must be 0";
+  for (int p = 0; p < B; ++p)
+    if (seg_off[p + 1] < seg_off[p]) return "seg_off must not decrease";
+  return "";
+}
+}  // namespace
+
+int tg_sample_range_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times,
+                             const double* t_range, double dt, int* counts, double* samples, double* full, long long* t_ns) {
+  return tg_guard(ctx, [&]() -> int {
+    const char* why = tg_range_refusal(N, D, B, seg_off, coef, times, t_range, dt, counts);
+    if (!*why && D < 3) why = "Dimension has to be at least 3";  // eth/trajectory_sampling.cpp:58-61
+    if (*why) { ctx->err = why; return TG_ERR_INVALID; }
+    const std::vector<double> c4 = tg_pad_coef(coef, (size_t)seg_off[B], N, D);
+    bool ok = false;
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) {
+      ok = ctx->pipe.template sample_range_batch_n<decltype(nn)::value>(B, seg_off, c4.data(), times, t_range, dt, counts, samples, full, t_ns);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (!ok) { ctx->err = "a window's sample count passed its bound"; return TG_ERR_CAPACITY; }
+    return TG_OK;
+  });
+}
+
+int tg_evaluate_range_batch_nd(tg_ctx* ctx, int N, int D, int B, const int* seg_off, const double* coef, const double* times,
+                               const double* t_range, double dt, int derivative, int* counts, double* out, double* sampling_times) {
+  return tg_guard(ctx, [&]() -> int {
+    const char* why = tg_range_refusal(N, D, B, seg_off, coef, times, t_range, dt, counts);
+    if (!*why && derivative < 0) why = "derivative must not be negative";
+    if (*why) { ctx->err = why; return TG_ERR_INVALID; }
+    const std::vector<double> c4 = tg_pad_coef(coef, (size_t)seg_off[B], N, D);
+    bool ok = false;
+    ctx->be.timer_start();
+    tg_dispatch_n(N, [&](auto nn) {
+      ok = ctx->pipe.template evaluate_range_batch_n<decltype(nn)::value>(B, D, seg_off, c4.data(), times, t_range, dt, derivative, counts, out,
+                                                                        sampling_times);
+    });
+    ctx->last_ms = ctx->be.timer_stop();
+    if (!ok) { ctx->err = "a window's sample count passed its bound"; return TG_ERR_CAPACITY; }
+    return TG_OK;
+  });
+}
+
 int tg_extrema_batch_nd(tg_ctx* ctx, int N, int D, int totS, const double* coef, const double* times, double* maxima) {
   return tg_guard(ctx, [&]() -> int {
     if (!tg_shape_ok(N, D)) { ctx->err = "supported shapes: N in {6, 8, 10, 12}, D in 1..4"; return TG_ERR_INVALID; }

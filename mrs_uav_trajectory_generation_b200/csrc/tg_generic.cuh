@@ -16,6 +16,7 @@
 //                                                      (segment, dimension), with solve_warp's coef_from_endpoints / cost_partial
 //   poly_eval_n<N>, sample_eval_n<N>                   Trajectory::evaluate / sampleWholeTrajectory (eth/trajectory.cpp:55-151,
 //                                                      eth/trajectory_sampling.cpp:49-124)
+//   RangeWalkFn, EvaluateRangeFn<N>                    sampleTrajectoryInRange / evaluateRange over a window per trajectory
 //   ExtremaFn<N, Q>, MaxMagnitudeSegFn<N, K>           per-segment maxima (tg_poly.cuh over N), one thread per segment
 //   ScaleFn<N>                                         scaleSegmentTimesToMeetConstraints' stretch (eth/trajectory.cpp:610-658)
 //   MellingerHeadFn / HrowFn / SolveFn<N>              one Mellinger evaluation: S+1 solves per running problem (nl_impl.h:282-323);
@@ -694,10 +695,59 @@ struct GenSampleWalkFn {
   int* count;
   TG_HD void operator()(size_t p) const {
     const int cap = smp_off[p + 1] - smp_off[p];
-    const int m = sample_walk(seg_off[p + 1] - seg_off[p], times + seg_off[p], dt, cap, seg_idx + smp_off[p], t_in + smp_off[p]);
+    const int S = seg_off[p + 1] - seg_off[p];
+    const int m = sample_walk(S, times + seg_off[p], 0.0, total_time(S, times + seg_off[p]), dt, cap, seg_idx + smp_off[p], t_in + smp_off[p], nullptr);
     count[p] = m > cap ? cap : m;
   }
 };
+// sampleTrajectoryInRange / evaluateRange (eth/trajectory_sampling.cpp:49-104, eth/trajectory.cpp:93-151): the walk over the window
+// [t_range[2p], t_range[2p+1]] of trajectory p, capped by sample_range_cap.  Without row_off it only counts; with row_off (the
+// exclusive scan of those counts) it writes every sample's segment, time in segment, accumulated time and time_from_start_ns at its
+// compacted row.  A count past the cap raises *overflow: the call fails instead of returning a short window.
+struct RangeWalkFn {
+  const int* seg_off;
+  const double* times;
+  const double* t_range;  // [B][2]
+  double dt;
+  const int* row_off;  // [B+1] or null
+  int* count;          // [B], written by the counting pass
+  int* seg_idx;        // [rows]
+  double* t_in;        // [rows]
+  double* acc;         // [rows]
+  long long* t_ns;     // [rows] or null
+  int* overflow;
+  TG_HD void operator()(size_t p) const {
+    const int s0 = seg_off[p], S = seg_off[p + 1] - s0;
+    const double t_start = t_range[2 * p], t_end = t_range[2 * p + 1];
+    const int cap = sample_range_cap(S, times + s0, t_start, t_end, dt);
+    int m = cap + 1;
+    if (cap >= 0) {
+      const int r = row_off ? row_off[p] : 0;
+      m = sample_walk(S, times + s0, t_start, t_end, dt, cap, row_off ? seg_idx + r : nullptr, t_in + r, acc + r);
+      if (row_off && t_ns)
+        for (int k = 0; k < m && k < cap; ++k) t_ns[r + k] = (long long)((t_start + dt * (double)k) * 1.e9);  // trajectory_sampling.cpp:98
+    }
+    if (m > cap) TG_ATOMIC_ADD(overflow, 1);
+    if (!row_off) count[p] = m > cap ? 0 : m;
+  }
+};
+namespace gen {
+// Trajectory::evaluateRange's values: derivative `deriv` of the D dimensions at every compacted row, zeros for deriv >= N
+template <int N>
+struct EvaluateRangeFn {  // one thread per row
+  const int* seg_off;
+  const int* row_prob;  // row -> trajectory
+  const int* seg_idx;
+  const double* t_in;
+  const double* coef;  // [totS][4][N]
+  int deriv, D;
+  double* out;  // [rows][D]
+  TG_HD void operator()(size_t row) const {
+    const size_t gs = (size_t)seg_off[row_prob[row]] + seg_idx[row];
+    for (int d = 0; d < D; ++d) out[row * D + d] = poly_eval_n<N>(coef + (gs * TG_D + d) * N, t_in[row], deriv);
+  }
+};
+}  // namespace gen
 
 }  // namespace tg
 

@@ -839,7 +839,7 @@ struct SampleWalkFn {
     const int cap = smp_off[p + 1] - smp_off[p];
     ps.sample_cap = cap;
     if (ps.status != kFindOk) { ps.n_samples = 0; return; }
-    const int m = sample_walk(S, b.times + s0, dt, cap, seg_idx + smp_off[p], t_in + smp_off[p]);
+    const int m = sample_walk(S, b.times + s0, 0.0, total_time(S, b.times + s0), dt, cap, seg_idx + smp_off[p], t_in + smp_off[p], nullptr);
     ps.n_samples = m;
     if (m > cap) { ps.n_samples = cap; ps.status = kFindSampleFail; }
   }

@@ -222,11 +222,17 @@ TG_HD void scale_segment(double* __restrict__ coef, double* __restrict__ T, doub
 }
 
 // ---- dt-sampling (eth/trajectory.cpp:93-151): the serial walk.  One thread per problem. ------------------------
-// Writes (segment index, time in segment) per sample when seg_idx != null; returns the sample count.
-TG_HD_NOINLINE int sample_walk(int S, const double* __restrict__ T, double dt, int cap, int* __restrict__ seg_idx, double* __restrict__ t_in) {
-  double t_end = 0.0;
-  for (int i = 0; i < S; ++i) t_end = t_end + T[i];
-  const double t_start = 0.0;
+// Trajectory::max_time_: the segment times accumulated in segment order (eth/trajectory.h:76-83)
+TG_HD double total_time(int S, const double* __restrict__ T) {
+  double t = 0.0;
+  for (int i = 0; i < S; ++i) t = t + T[i];
+  return t;
+}
+// The walk over the window [t_start, t_end]; the whole trajectory is [0, total_time].  Writes (segment index, time in segment) and,
+// when acc_out != null, the accumulated time of every sample below cap when seg_idx != null.  Returns the sample count, or cap + 1:
+// the walk stops as soon as the count passes cap, so that it ends for any window.
+TG_HD_NOINLINE int sample_walk(int S, const double* __restrict__ T, double t_start, double t_end, double dt, int cap, int* __restrict__ seg_idx,
+                               double* __restrict__ t_in, double* __restrict__ acc_out) {
   double acc = 0.0;
   int i = 0;
   for (i = 0; i < S; ++i) {
@@ -248,8 +254,10 @@ TG_HD_NOINLINE int sample_walk(int S, const double* __restrict__ T, double dt, i
     if (seg_idx && m < cap) {
       seg_idx[m] = i;
       t_in[m] = tin;
+      if (acc_out) acc_out[m] = acc;
     }
     ++m;
+    if (m > cap) break;
     tin = tin + dt;
     acc = acc + dt;
   }
@@ -257,11 +265,28 @@ TG_HD_NOINLINE int sample_walk(int S, const double* __restrict__ T, double dt, i
 }
 // upper bound on the sample count, used to size the sample arrays before the walk
 TG_HD int sample_cap(int S, const double* __restrict__ T, double dt) {
-  double t_end = 0.0;
-  for (int i = 0; i < S; ++i) t_end = t_end + T[i];
-  const double n = t_end / dt;
+  const double n = total_time(S, T) / dt;
   if (!(n < 1.0e9)) return 8;
   return (int)n + 4;
+}
+// Bound on the sample count of the window [t_start, t_end], the walk's cap.  Sample k lies at the accumulated time acc0 + k dt < t_end
+// (acc0: start of the segment holding t_start) and at t_start + k dt <= the trajectory's end, so a window running to +inf is bounded
+// by the trajectory; 4 + n / 10^6 absorb the rounding of the two running sums.  0 where the walk emits nothing (no segment holds
+// t_start, a NaN end); -1 when no int bounds the window.
+TG_HD int sample_range_cap(int S, const double* __restrict__ T, double t_start, double t_end, double dt) {
+  double acc = 0.0;
+  int i = 0;
+  for (i = 0; i < S; ++i) {
+    acc = acc + T[i];
+    if (acc > t_start) break;
+  }
+  if (i >= S) return 0;
+  acc = acc - T[i];
+  const double n = dmin(t_end - acc, total_time(S, T) - t_start) / dt;
+  if (n != n) return 0;
+  if (!(n < 1.0e9)) return -1;
+  const double m = dmax(n, 0.0);
+  return (int)(m + m * 1.0e-6) + 4;
 }
 // One sample -> the 4 values getTrajectoryReference emits (node.cpp:1578-1602): x, y, z, yawFromQuaternion(...)
 // full != null additionally receives p4 v4 a4 j3 s3 (19 doubles = the EigenTrajectoryPoint payload).

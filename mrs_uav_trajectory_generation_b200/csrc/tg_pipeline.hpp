@@ -9,6 +9,7 @@
 
 #include <algorithm>
 #include <chrono>
+#include <climits>
 #include <cstdio>
 #include <cstdlib>
 #include <cmath>
@@ -1730,6 +1731,99 @@ class Pipeline {
       if (samples) be_.d2h(samples + 4 * (size_t)dst[p], d_xyzh + 4 * (size_t)smp_off[p], sizeof(double) * 4 * (size_t)counts[p]);
       if (full) be_.d2h(full + 19 * (size_t)dst[p], d_full + 19 * (size_t)smp_off[p], sizeof(double) * 19 * (size_t)counts[p]);
     }
+  }
+  // The windowed dt walk of sampleTrajectoryInRange / evaluateRange for B trajectories of N-coefficient segments, window
+  // p = [t_range[2p], t_range[2p+1]]: the trajectories go up, a counting walk gives counts[B]; when rows are wanted, the device
+  // scans the counts and walks again, writing each sample at its compacted row, and row_prob maps rows to trajectories.
+  // false: some window's count passed its bound (sample_range_cap); counts is then not written.
+  struct RangeRows {
+    int* seg_off;
+    double* coef;
+    int* count;
+    int* row_off;
+    int* row_prob;
+    int* seg_idx;
+    double* t_in;
+    double* acc;
+    long long* t_ns;
+    size_t rows;
+  };
+  template <int N>
+  bool range_walk(int B, const int* seg_off, const double* coef, const double* times, const double* t_range, double dt, int* counts,
+                  bool rows_wanted, bool want_tns, RangeRows* w) {
+    scratch_.reset();
+    const int totS = seg_off[B];
+    w->seg_off = scratch_.template alloc<int>((size_t)B + 1);
+    double* d_times = scratch_.template alloc<double>(std::max(totS, 1));
+    double* d_range = scratch_.template alloc<double>((size_t)B * 2);
+    int* d_count = w->count = scratch_.template alloc<int>((size_t)B + 1);
+    int* d_overflow = scratch_.template alloc<int>(1);
+    be_.h2d(w->seg_off, seg_off, sizeof(int) * ((size_t)B + 1));
+    be_.h2d(d_times, times, sizeof(double) * totS);
+    be_.h2d(d_range, t_range, sizeof(double) * 2 * (size_t)B);
+    be_.dev_memset(d_overflow, 0, sizeof(int));
+    be_.for_each(B, RangeWalkFn{w->seg_off, d_times, d_range, dt, nullptr, d_count, nullptr, nullptr, nullptr, nullptr, d_overflow});
+    launches(1);
+    int overflow = 0;
+    std::vector<int> cnt(B);
+    be_.d2h(&overflow, d_overflow, sizeof(int));
+    if (overflow) return false;
+    be_.d2h(cnt.data(), d_count, sizeof(int) * B);
+    long long rows = 0;
+    for (int p = 0; p < B; ++p) rows += cnt[p];
+    if (rows > (long long)INT_MAX) return false;
+    std::copy(cnt.begin(), cnt.end(), counts);
+    counters.samples += rows;
+    w->rows = (size_t)rows;
+    if (!rows_wanted || rows == 0) return true;
+    w->coef = scratch_.template alloc<double>((size_t)std::max(totS, 1) * TG_D * N);
+    be_.h2d(w->coef, coef, sizeof(double) * (size_t)totS * TG_D * N);
+    w->row_off = scratch_.template alloc<int>((size_t)B + 1);
+    w->row_prob = scratch_.template alloc<int>(w->rows);
+    w->seg_idx = scratch_.template alloc<int>(w->rows);
+    w->t_in = scratch_.template alloc<double>(w->rows);
+    w->acc = scratch_.template alloc<double>(w->rows);
+    w->t_ns = want_tns ? scratch_.template alloc<long long>(w->rows) : nullptr;
+    be_.exclusive_scan(d_count, w->row_off, B);
+    be_.for_each(B, RangeWalkFn{w->seg_off, d_times, d_range, dt, w->row_off, d_count, w->seg_idx, w->t_in, w->acc, w->t_ns, d_overflow});
+    be_.for_each(B, SlotProblemFn{B, w->row_off, w->row_prob});
+    launches(3);
+    return true;
+  }
+  // sampleTrajectoryInRange: the sample record of every row (gen::SampleEvalFn over the compacted rows) and time_from_start_ns;
+  // each output array comes back in one copy
+  template <int N>
+  bool sample_range_batch_n(int B, const int* seg_off, const double* coef, const double* times, const double* t_range, double dt, int* counts,
+                            double* samples, double* full, long long* t_ns) {
+    RangeRows w;
+    if (!range_walk<N>(B, seg_off, coef, times, t_range, dt, counts, samples || full || t_ns, t_ns != nullptr, &w)) return false;
+    if ((!samples && !full && !t_ns) || w.rows == 0) return true;
+    double* d_xyzh = samples ? scratch_.template alloc<double>(w.rows * 4) : nullptr;
+    double* d_full = full ? scratch_.template alloc<double>(w.rows * 19) : nullptr;
+    if (samples || full) {
+      be_.for_each(w.rows, gen::SampleEvalFn<N>{w.seg_off, w.row_off, w.row_prob, w.count, w.seg_idx, w.t_in, w.coef, d_xyzh, d_full});
+      launches(1);
+    }
+    if (samples) be_.d2h(samples, d_xyzh, sizeof(double) * 4 * w.rows);
+    if (full) be_.d2h(full, d_full, sizeof(double) * 19 * w.rows);
+    if (t_ns) be_.d2h(t_ns, w.t_ns, sizeof(long long) * w.rows);
+    return true;
+  }
+  // Trajectory::evaluateRange: derivative `deriv` of the D dimensions at every row ([rows][D]) and the accumulated sampling times
+  template <int N>
+  bool evaluate_range_batch_n(int B, int D, const int* seg_off, const double* coef, const double* times, const double* t_range, double dt, int deriv,
+                              int* counts, double* out, double* sampling_times) {
+    RangeRows w;
+    if (!range_walk<N>(B, seg_off, coef, times, t_range, dt, counts, out || sampling_times, false, &w)) return false;
+    if ((!out && !sampling_times) || w.rows == 0) return true;
+    if (out) {
+      double* d_out = scratch_.template alloc<double>(w.rows * D);
+      be_.for_each(w.rows, gen::EvaluateRangeFn<N>{w.seg_off, w.row_prob, w.seg_idx, w.t_in, w.coef, deriv, D, d_out});
+      launches(1);
+      be_.d2h(out, d_out, sizeof(double) * D * w.rows);
+    }
+    if (sampling_times) be_.d2h(sampling_times, w.acc, sizeof(double) * w.rows);
+    return true;
   }
   // per-segment maxima of |v|,|a|,|j| for the three dimension groups, N-coefficient segments
   template <int N>
