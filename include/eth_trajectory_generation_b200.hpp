@@ -8,6 +8,7 @@
 //   eth_trajectory_generation::PolynomialOptimizationNonLinear<N>  nl.h:147-197
 //   eth_trajectory_generation::sampleWholeTrajectory           eth/trajectory_sampling.h:44
 //   eth_trajectory_generation::sampleTrajectoryInRange / sampleTrajectoryStartDuration  eth/trajectory_sampling.cpp:49-104, eth/trajectory_sampling.h
+//   eth_trajectory_generation::estimateSegmentTimes / estimateSegmentTimesBaca   eth/vertex.cpp:491-565, 301-485
 // Same method names, argument meaning and error behaviour (bool returns, print-and-continue -- eth/misc.h:6-38 -- and the
 // NLopt-style int of optimize()).  Every method marshals into the C ABI of include/tg_b200.h, i.e. into the sm_100a
 // kernels of libtg_b200.so; one object = a batch of one.  There is no CPU arithmetic here and no fallback: constructing
@@ -22,7 +23,8 @@
 // own struct when that header is included, or the plain TrajectoryPoint below.
 //
 // Additions that the one-problem-per-object reference API cannot express: TrajectoryGeneratorBatch (the numeric core of
-// optimize()/findTrajectory for many paths in one call, SURVEY.md H7) and sampleTrajectoriesInRange (many windows in one call).
+// optimize()/findTrajectory for many paths in one call, SURVEY.md H7), sampleTrajectoriesInRange (many windows in one call) and
+// estimateSegmentTimesBatch (many vertex lists in one call).
 #ifndef ETH_TRAJECTORY_GENERATION_B200_HPP_
 #define ETH_TRAJECTORY_GENERATION_B200_HPP_
 
@@ -542,7 +544,88 @@ inline bool pack_vertices(const Vertex::Vector& vertices, std::vector<uint8_t>* 
   }
   return true;
 }
+
+// tg_estimate_segment_times_batch over vertex lists: the POSITION constraint of every vertex (x y z heading) goes up, the Euclidean
+// and / or Baca times of list i come back as (*euclid)[i] / (*baca)[i].  false, with a message and nothing filled, for an empty list,
+// a vertex that is not 4-dimensional or one without a POSITION constraint (the reference reads the heading as [3] of it).
+inline bool estimate_times(const char* who, const std::vector<const Vertex::Vector*>& lists, const double* L8, std::vector<std::vector<double>>* euclid,
+                           std::vector<std::vector<double>>* baca) {
+  std::vector<int> vtx_off(1, 0);
+  std::vector<double> pos4;
+  Vertex::ConstraintValue p;
+  for (const Vertex::Vector* vl : lists) {
+    if (vl->empty()) {
+      std::printf("[%s]: a vertex list is empty\n", who);
+      return false;
+    }
+    for (const Vertex& v : *vl) {
+      if (v.D() != (size_t)kD || !v.getConstraint(derivative_order::POSITION, &p)) {
+        std::printf("[%s]: every vertex needs %d dimensions (x, y, z, heading) and a POSITION constraint\n", who, kD);
+        return false;
+      }
+      for (int d = 0; d < kD; ++d) pos4.push_back(p[d]);
+    }
+    vtx_off.push_back(vtx_off.back() + (int)vl->size());
+  }
+  const int B = (int)lists.size();
+  const size_t totS = (size_t)(vtx_off[B] - B);
+  std::vector<double> e(euclid ? totS : 0), b(baca ? totS : 0);
+  Context& c = Context::instance();
+  c.check(tg_estimate_segment_times_batch(c.get(), B, vtx_off.data(), pos4.data(), L8, euclid ? e.data() : nullptr, baca ? b.data() : nullptr),
+          "tg_estimate_segment_times_batch");
+  if (euclid) euclid->resize(B);
+  if (baca) baca->resize(B);
+  for (int i = 0; i < B; ++i) {
+    const size_t s0 = (size_t)(vtx_off[i] - i), s1 = (size_t)(vtx_off[i + 1] - i - 1);
+    if (euclid) (*euclid)[i].assign(e.begin() + s0, e.begin() + s1);
+    if (baca) (*baca)[i].assign(b.begin() + s0, b.begin() + s1);
+  }
+  return true;
+}
 }  // namespace b200
+
+// ---- initial segment times (eth/vertex.cpp:301-565) --------------------------------------------------------------------------
+// estimateSegmentTimes (the Euclidean estimate, eth/vertex.cpp:491-565) and estimateSegmentTimesBaca (301-485) with the reference's
+// argument list, as findTrajectory calls them (node.cpp:1045-1056); one device call each, the kernels of the optimisation pipeline.
+// A list that is empty, not 4-dimensional or has a vertex without a POSITION constraint prints a message and gives an empty vector.
+inline std::vector<double> estimateSegmentTimes(const Vertex::Vector& vertices, double v_max_horizontal, double v_max_vertical, double a_max_horizontal,
+                                                double a_max_vertical, double j_max_horizontal, double j_max_vertical, double v_max_heading,
+                                                double a_max_heading) {
+  const double L8[8] = {v_max_horizontal, v_max_vertical, a_max_horizontal, a_max_vertical, j_max_horizontal, j_max_vertical, v_max_heading, a_max_heading};
+  std::vector<std::vector<double>> out;
+  if (!b200::estimate_times("estimateSegmentTimes", {&vertices}, L8, &out, nullptr)) return {};
+  return out[0];
+}
+// the name SURVEY.md §8a gives the Euclidean estimate
+inline std::vector<double> estimateSegmentTimesEuclidean(const Vertex::Vector& vertices, double v_max_horizontal, double v_max_vertical,
+                                                         double a_max_horizontal, double a_max_vertical, double j_max_horizontal, double j_max_vertical,
+                                                         double v_max_heading, double a_max_heading) {
+  return estimateSegmentTimes(vertices, v_max_horizontal, v_max_vertical, a_max_horizontal, a_max_vertical, j_max_horizontal, j_max_vertical,
+                              v_max_heading, a_max_heading);
+}
+inline std::vector<double> estimateSegmentTimesBaca(const Vertex::Vector& vertices, double v_max_horizontal, double v_max_vertical, double a_max_horizontal,
+                                                    double a_max_vertical, double j_max_horizontal, double j_max_vertical, double v_max_heading,
+                                                    double a_max_heading) {
+  const double L8[8] = {v_max_horizontal, v_max_vertical, a_max_horizontal, a_max_vertical, j_max_horizontal, j_max_vertical, v_max_heading, a_max_heading};
+  std::vector<std::vector<double>> out;
+  if (!b200::estimate_times("estimateSegmentTimesBaca", {&vertices}, L8, nullptr, &out)) return {};
+  return out[0];
+}
+// Not a reference name: both estimates for many vertex lists in one device call; (*euclidean)[i] / (*baca)[i] are the times of
+// vertex_lists[i], either pointer may be null.  false, with a message and nothing filled, for no list, both pointers null, or what
+// estimateSegmentTimes refuses for any list.
+inline bool estimateSegmentTimesBatch(const std::vector<Vertex::Vector>& vertex_lists, double v_max_horizontal, double v_max_vertical,
+                                      double a_max_horizontal, double a_max_vertical, double j_max_horizontal, double j_max_vertical, double v_max_heading,
+                                      double a_max_heading, std::vector<std::vector<double>>* euclidean, std::vector<std::vector<double>>* baca) {
+  if (vertex_lists.empty() || (!euclidean && !baca)) {
+    std::printf("[estimateSegmentTimesBatch]: no vertex list or no output\n");
+    return false;
+  }
+  const double L8[8] = {v_max_horizontal, v_max_vertical, a_max_horizontal, a_max_vertical, j_max_horizontal, j_max_vertical, v_max_heading, a_max_heading};
+  std::vector<const Vertex::Vector*> lists;
+  for (const Vertex::Vector& vl : vertex_lists) lists.push_back(&vl);
+  return b200::estimate_times("estimateSegmentTimesBatch", lists, L8, euclidean, baca);
+}
 
 // ---- PolynomialOptimization<N> (lin.h:60-233) -----------------------------------------------------------------------------
 // N = 10 on 4 dimensions with derivative_to_optimize 2..4 (the node's shape, node.cpp:902, 907-921, 1063) runs on the tuned kernels;

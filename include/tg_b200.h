@@ -162,6 +162,15 @@ int tg_max_magnitude_batch(tg_ctx* ctx, int B, const int* seg_off, const double*
  *   coef/times; passes[B], within[B]. */
 int tg_scale_times_batch(tg_ctx* ctx, int B, const int* seg_off, double* coef, double* times, const double* limits9, int* passes,
                          uint8_t* within);
+/* tg_estimate_segment_times_batch = estimateSegmentTimes (= Euclidean, eth/vertex.cpp:491-565) and estimateSegmentTimesBaca
+ *   (301-485), as findTrajectory calls them (node.cpp:1045-1056), for B vertex lists, with the device functions the pipeline uses.
+ *   vtx_off[B+1]; pos4[totV][4] = x y z heading (the POSITION constraint); limits8 = v_h, v_v, a_h, a_v, j_h, j_v, heading speed,
+ *   heading acceleration (the reference's argument order).  Outputs [totS], segment s of problem p at vtx_off[p] - p + s; either
+ *   may be NULL, not both.  A list of one vertex has no segment.  TG_ERR_INVALID, with no output written, for B < 1, a NULL input,
+ *   both outputs NULL, vtx_off[0] != 0 or a list of no vertex.  Non-finite positions or limits are not refused: they give what the
+ *   formulas give. */
+int tg_estimate_segment_times_batch(tg_ctx* ctx, int B, const int* vtx_off, const double* pos4, const double* limits8, double* euclid,
+                                    double* baca);
 /* General shape: the reference's classes are templates over the number of coefficients N (lin.h:46-55: even; Polynomial::kMaxN = 12,
  *   eth/polynomial.h:45-48) and take the dimension D at run time (Vertex(D), PolynomialOptimization<N>(D), Trajectory::D()).
  *   The three entry points below are tg_solve_linear_batch / tg_evaluate_batch / tg_sample_batch for N in {6, 8, 10, 12},

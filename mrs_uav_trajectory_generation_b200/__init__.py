@@ -21,6 +21,10 @@ from .api import (  # noqa: F401
     sample_trajectory_in_range,
     sample_trajectory_start_duration,
     sample_trajectories_in_range,
+    estimate_segment_times,
+    estimate_segment_times_euclidean,
+    estimate_segment_times_baca,
+    estimate_segment_times_batch,
     TrajectoryGenerator,
     derivative_order,
 )

@@ -160,6 +160,7 @@ class Library:
                                                  _dp, _dp, _dp, _ip, _ip, _dp, _dp]
         L.tg_max_magnitude_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, C.c_int, _dp, _dp, _ip]
         L.tg_scale_times_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp, _ip, _u8p]
+        L.tg_estimate_segment_times_batch.argtypes = [C.c_void_p, C.c_int, _ip, _dp, _dp, _dp, _dp]
         L.tg_sweep_costs.argtypes = [C.c_void_p, C.c_int, _u8p, _dp, C.c_int, C.c_longlong, _dp, C.c_int, _dp, _llp, _dp]
         L.tg_default_params.argtypes = [C.POINTER(Params)]
         L.tg_set_profiling.argtypes = [C.c_void_p, C.c_int]
@@ -400,6 +401,23 @@ class Context:
                                                        _p(cdim, _ip), _p(cder, _ip), _p(cval), _p(coef), _p(vval_out), _p(code, _ip),
                                                        _p(iters, _ip), _p(total), _p(parts)))
         return {"times": times, "coef": coef, "vval": vval_out, "code": code, "n_iterations": iters, "total": total, "parts": parts}
+
+    def estimate_segment_times_batch(self, vtx_off, pos4, limits8, euclidean=True, baca=True):
+        """estimateSegmentTimes (Euclidean) and estimateSegmentTimesBaca (eth/vertex.cpp:491-565, 301-485) for B vertex lists
+        (tg_estimate_segment_times_batch): vtx_off int32[B+1], pos4 float64[totV, 4] = x y z heading, limits8 = v_h, v_v, a_h, a_v,
+        j_h, j_v, heading speed, heading acceleration.  Returns (euclid [totS] or None, baca [totS] or None); segment s of problem p
+        at vtx_off[p] - p + s."""
+        vtx_off = np.ascontiguousarray(vtx_off, dtype=np.int32)
+        pos4 = np.ascontiguousarray(pos4, dtype=np.float64)
+        lim = np.ascontiguousarray(limits8, dtype=np.float64)
+        B = len(vtx_off) - 1
+        if lim.shape != (8,) or pos4.ndim != 2 or pos4.shape[1] != 4 or B < 1 or pos4.shape[0] != int(vtx_off[-1]):
+            raise ValueError("vtx_off [B+1] with B >= 1, pos4 [vtx_off[-1], 4] and eight limits are needed")
+        totS = max(int(vtx_off[-1]) - B, 0)
+        e = np.empty(totS) if euclidean else None
+        b = np.empty(totS) if baca else None
+        self._check(self.L.lib.tg_estimate_segment_times_batch(self.h, B, _p(vtx_off, _ip), _p(pos4), _p(lim), _p(e), _p(b)))
+        return e, b
 
     # ---- the steps either side of the path (SURVEY.md 8f) ---------------------------------------------------------------
     def preprocess_paths(self, wp_off, wp, stop_at=None, min_waypoint_distance=0.05, straightener=False, max_deviation=0.05, max_hdg_deviation=0.1):

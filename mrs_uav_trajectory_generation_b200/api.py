@@ -210,6 +210,41 @@ def sample_trajectory_start_duration(trajectory, start_time, duration, dt, full=
     return sample_trajectory_in_range(trajectory, start_time, start_time + duration, dt, full=full, ctx=ctx)
 
 
+def _vertex_positions(vertex_lists):
+    """vtx_off [B+1], pos4 [totV, 4] of lists of Vertex(4): the POSITION constraint of every vertex"""
+    vtx_off, pos = [0], []
+    for vl in vertex_lists:
+        for v in vl:
+            if v.D != D or not v.hasConstraint(derivative_order.POSITION):
+                raise ValueError("segment times are estimated from 4-dimensional vertices (x, y, z, heading) with a POSITION constraint")
+            pos.append(v.getConstraint(derivative_order.POSITION))
+        vtx_off.append(len(pos))
+    return np.array(vtx_off, dtype=np.int32), np.array(pos, dtype=np.float64).reshape(-1, D)
+
+
+def estimate_segment_times_batch(vertex_lists, limits8, ctx=None):
+    """estimateSegmentTimes (Euclidean) and estimateSegmentTimesBaca for many vertex lists in one device call (not a reference name).
+    limits8 = v_h, v_v, a_h, a_v, j_h, j_v, heading speed, heading acceleration.  Returns (euclidean, baca): one array of segment times
+    per list, a list of one vertex giving an empty one."""
+    vtx_off, pos4 = _vertex_positions(vertex_lists)
+    e, b = (ctx or default_context()).estimate_segment_times_batch(vtx_off, pos4, limits8)
+    seg_off = vtx_off - np.arange(len(vtx_off))
+    return ([e[seg_off[p]:seg_off[p + 1]] for p in range(len(vtx_off) - 1)], [b[seg_off[p]:seg_off[p + 1]] for p in range(len(vtx_off) - 1)])
+
+
+def estimate_segment_times(vertices, limits8, ctx=None):
+    """eth_trajectory_generation::estimateSegmentTimes (eth/vertex.cpp:491-565, the Euclidean estimate) of one vertex list."""
+    return estimate_segment_times_batch([vertices], limits8, ctx)[0][0]
+
+
+estimate_segment_times_euclidean = estimate_segment_times
+
+
+def estimate_segment_times_baca(vertices, limits8, ctx=None):
+    """eth_trajectory_generation::estimateSegmentTimesBaca (eth/vertex.cpp:301-485) of one vertex list."""
+    return estimate_segment_times_batch([vertices], limits8, ctx)[1][0]
+
+
 class PolynomialOptimization:
     """eth_trajectory_generation::PolynomialOptimization<N> (lin.h:60-233) for one problem or a batch.  N = 10 on 4 dimensions with
     derivative_to_optimize 2..4 (the node's shape) runs on the tuned kernels; N in {6, 8, 10, 12}, 1..4 dimensions and

@@ -855,6 +855,20 @@ int tg_scale_times_batch(tg_ctx* ctx, int B, const int* seg_off, double* coef, d
   });
 }
 
+int tg_estimate_segment_times_batch(tg_ctx* ctx, int B, const int* vtx_off, const double* pos4, const double* limits8, double* euclid,
+                                    double* baca) {
+  return tg_guard(ctx, [&]() -> int {
+    if (B < 1 || !vtx_off || !pos4 || !limits8 || (!euclid && !baca)) { ctx->err = "invalid argument"; return TG_ERR_INVALID; }
+    if (vtx_off[0] != 0) { ctx->err = "vtx_off[0] must be 0"; return TG_ERR_INVALID; }
+    for (int p = 0; p < B; ++p)
+      if (vtx_off[p + 1] <= vtx_off[p]) { ctx->err = "every vertex list needs at least one vertex"; return TG_ERR_INVALID; }
+    ctx->be.timer_start();
+    ctx->pipe.estimate_times_batch(B, vtx_off, pos4, limits8, euclid, baca);
+    ctx->last_ms = ctx->be.timer_stop();
+    return TG_OK;
+  });
+}
+
 int tg_sweep_costs(tg_ctx* ctx, int V, const uint8_t* vmask, const double* vval, int r, long long K, const double* cand, int cand_on_device,
                    double* costs, long long* best_index, double* best_cost) {
   return tg_guard(ctx, [&]() -> int {

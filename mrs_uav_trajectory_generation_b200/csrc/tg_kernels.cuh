@@ -166,6 +166,30 @@ struct BacaTotalFn {
     b.ps[p].baca_total = tot;
   }
 };
+// The same two estimates for caller-given vertex lists (tg_estimate_segment_times_batch): one thread per segment.  Segment gs
+// belongs to the last problem p with vtx_off[p] - p <= gs (found by bisection; a problem of one vertex owns no segment).
+// pos4: [totV][4] x y z heading; L = v_h, v_v, a_h, a_v, j_h, j_v, heading speed, heading acceleration.
+struct EstimateTimesFn {
+  int B;
+  const int* vtx_off;
+  const double* pos4;
+  double L[8];
+  double* euclid;  // [totS] or null
+  double* baca;    // [totS] or null
+  TG_HD void operator()(size_t gsi) const {
+    const int gs = (int)gsi;
+    int lo = 0, hi = B - 1;
+    while (lo < hi) {
+      const int mid = (lo + hi + 1) >> 1;
+      if (vtx_off[mid] - mid <= gs) lo = mid;
+      else hi = mid - 1;
+    }
+    const int v0 = vtx_off[lo], V = vtx_off[lo + 1] - v0, i = gs - (v0 - lo);
+    const double* vpos = pos4 + 4 * (size_t)v0;
+    if (euclid) euclid[gs] = segment_time_euclidean(vpos + 4 * (size_t)i, vpos + 4 * (size_t)(i + 1), L);
+    if (baca) baca[gs] = segment_time_baca(vpos, 4, i, V, L);
+  }
+};
 
 // ---- 3. per-segment records ------------------------------------------------------------------------------------------
 // base: one record per segment at times[]; Mellinger: three per segment at xeval, xeval+0.1, max(lb, xeval-corr)

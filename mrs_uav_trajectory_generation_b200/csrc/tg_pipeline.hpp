@@ -1892,6 +1892,24 @@ class Pipeline {
     if (passes) be_.d2h(passes, of.passes, sizeof(int) * B);
     if (within) be_.d2h(within, of.within, B);
   }
+  // estimateSegmentTimes / estimateSegmentTimesBaca (eth/vertex.cpp:491-565, 301-485) for B vertex lists given as positions
+  // pos4[totV][4]: euclid / baca [totS] (either null), segment s of problem p at vtx_off[p] - p + s
+  void estimate_times_batch(int B, const int* vtx_off, const double* pos4, const double* L8, double* euclid, double* baca) {
+    scratch_.reset();
+    const int totV = vtx_off[B], totS = totV - B;
+    if (totS == 0) return;
+    int* d_off = scratch_.template alloc<int>((size_t)B + 1);
+    double* d_pos = scratch_.template alloc<double>((size_t)totV * 4);
+    be_.h2d(d_off, vtx_off, sizeof(int) * ((size_t)B + 1));
+    be_.h2d(d_pos, pos4, sizeof(double) * 4 * (size_t)totV);
+    EstimateTimesFn f{B, d_off, d_pos, {}, euclid ? scratch_.template alloc<double>(totS) : nullptr,
+                      baca ? scratch_.template alloc<double>(totS) : nullptr};
+    for (int k = 0; k < 8; ++k) f.L[k] = L8[k];
+    be_.for_each((size_t)totS, f);
+    launches(1);
+    if (euclid) be_.d2h(euclid, f.euclid, sizeof(double) * totS);
+    if (baca) be_.d2h(baca, f.baca, sizeof(double) * totS);
+  }
   // PolynomialOptimizationNonLinear<N>::setupFromVertices + optimize() (Mellinger outer loop, nl_impl.h:159-234, then the time
   // scaling of scaleSegmentTimesWithViolation, 335-427) + getTrajectory for B problems given as vertices.  The evaluation runs S+1
   // solves per running problem with dense launches (a finished problem costs an early exit); the optimiser state machine is the one
